@@ -21,6 +21,10 @@ A second section (`config2`) reports BASELINE.json configs[1] (316 x 316 grid, L
 every timed phase) on each rank's own copy, as round 1 did.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scale 22] [--edges 70e6]
+                  [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (see dump_last_step); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the reference's CPU algorithm (oracle/cpu_baseline.py: the pure-Python
 fork-pool sampler, all host cores) on a bounded sample of the same workload's start nodes.  oracle/
@@ -344,6 +348,10 @@ def run_gpu(args):
     t_wall = time.perf_counter() - t_wall0
     gc.enable()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # before the sections below reuse `out`
+        dump_last_step(args.dump_outputs, torch, dist, rank, world, n, lo, hi, out, results[-1]["visits"],
+                       results[-1]["nnz"])
 
     # kernels of libgrf_b200.so per step, COUNTED: one more (untimed) step under torch's CUPTI profiler
     # (every rank runs the step -- the exchange inside it is a collective -- rank 0 alone records it)
@@ -616,6 +624,36 @@ def run_gpu(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS = 1 << 16     # rows of the product in --dump-outputs: 4 MB at t = 16 (the whole product is 268 MB)
+
+
+def dump_last_step(out_dir, torch, dist, rank, world, n, lo, hi, out, visits, nnz):
+    """What the last timed step handed its caller, gathered over the ranks and written by rank 0:
+    product_rows.npy     float32 [DUMP_ROWS, t]  rows of Phi(Phi^T V), a fixed seeded sample of the N rows
+    product_row_ids.npy  float64 [DUMP_ROWS]     which rows, ascending
+    product_colsum.npy   float64 [t]             column sums over all N rows of the product
+    walk_steps.npy       float64 [1]             walk-steps the walker executed
+    phi_nnz.npy          float64 [1]             entries of Phi (over the walk lengths)"""
+    rows = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_ROWS), replace=False))
+    mine = rows[(rows >= lo) & (rows < hi)]
+    part = (out[torch.from_numpy(mine - lo).to(out.device)].cpu().numpy(),
+            out.sum(0, dtype=torch.float64).cpu().numpy(), int(visits.item()), int(nnz))
+    parts = [part]
+    if world > 1:
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object(part, parts, dst=0)
+    if rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"product_rows": np.concatenate([p[0] for p in parts]).astype(np.float32),
+              "product_row_ids": rows.astype(np.float64),
+              "product_colsum": np.sum([p[1] for p in parts], axis=0, dtype=np.float64),
+              "walk_steps": np.array([sum(p[2] for p in parts)], dtype=np.float64),
+              "phi_nnz": np.array([sum(p[3] for p in parts)], dtype=np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def count_launches(line, world, measured):
     """Kernels of libgrf_b200.so launched per step on one rank: counted by CUPTI (torch.profiler) over one extra
     untimed step of rank 0 when that works, else from the call structure -- walker 1, row-count scan 3,
@@ -804,7 +842,13 @@ def main():
     ap.add_argument("--no-config2", action="store_true")
     ap.add_argument("--no-merged", action="store_true", help="skip the union-layout (CG steady state) product")
     ap.add_argument("--no-l3", action="store_true", help="skip the L = 3 section")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, a few MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

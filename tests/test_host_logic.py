@@ -195,3 +195,33 @@ def test_balanced_bounds_follow_the_cost_estimate():
     cost[100:] = 1.0
     b2 = sharding.balanced_bounds(graph, 2, row_cost=cost)
     assert b2[0] == 0 and b2[2] == n and 95 <= b2[1] <= 105   # half of the cost sits in the first 100 rows
+
+
+def test_bench_dump_writes_the_last_steps_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: a fixed sample of the product's rows (the same rows on every run), its column sums
+    over all rows and the two counts, as float32 / float64 .npy files of a few MB."""
+    import bench
+
+    t = 16
+    assert bench.DUMP_ROWS * (t * 4 + 8) < 64 << 20
+    monkeypatch.setattr(bench, "DUMP_ROWS", 512)
+    n = 1500
+    out = torch.randn(n, t, generator=torch.Generator().manual_seed(0))
+    # one thread: indexing a CPU tensor would start torch's worker pool, and the oracle tests fork afterwards
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        for d in ("a", "b"):
+            bench.dump_last_step(str(tmp_path / d), torch, None, 0, 1, n, 0, n, out, torch.tensor([4321]), 987)
+    finally:
+        torch.set_num_threads(threads)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["phi_nnz.npy", "product_colsum.npy", "product_row_ids.npy", "product_rows.npy", "walk_steps.npy"]
+    for name in files:
+        a, b = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert a.dtype in (np.float32, np.float64) and a.tobytes() == b.tobytes(), name
+    ids = np.load(tmp_path / "a" / "product_row_ids.npy")
+    assert ids.shape == (bench.DUMP_ROWS,) and np.all(np.diff(ids) > 0) and ids[-1] < n
+    assert np.array_equal(np.load(tmp_path / "a" / "product_rows.npy"), out.numpy()[ids.astype(np.int64)])
+    assert np.allclose(np.load(tmp_path / "a" / "product_colsum.npy"), out.double().sum(0).numpy(), rtol=1e-12)
+    assert np.load(tmp_path / "a" / "walk_steps.npy")[0] == 4321 and np.load(tmp_path / "a" / "phi_nnz.npy")[0] == 987

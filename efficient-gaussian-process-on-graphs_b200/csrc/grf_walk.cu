@@ -27,6 +27,7 @@
 // + col 4 B + val 8 B + staging write 12 B/(merged entry); three dependent
 // random 32-B sectors per step => latency / sector bound, not bandwidth bound.
 
+#include <limits.h>
 #include <stdlib.h>
 
 #include "grf_common.cuh"
@@ -525,6 +526,344 @@ static int launch_walk(const WalkParams &p, size_t smem, int threads, int grid, 
     return check_cuda(cudaGetLastError(), "walk_merge_kernel launch");
 }
 
+// ---------------- coupled walks (GRF_DRAW_COUPLE_HALT / GRF_DRAW_COUPLE_NEIGHBOURS) ----------------
+
+// exclusive max of one int per thread over the preceding threads of the group (kReverse: the following
+// ones); INT_MIN when there are none
+template <bool kBlock, bool kReverse>
+__device__ __forceinline__ int group_excl_max(int v, int *scratch) {
+    const int lane = threadIdx.x & 31;
+    int incl = v;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int n = kReverse ? __shfl_down_sync(0xffffffffu, incl, d) : __shfl_up_sync(0xffffffffu, incl, d);
+        if (kReverse ? lane + d < 32 : lane >= d) incl = max(incl, n);
+    }
+    int excl = kReverse ? __shfl_down_sync(0xffffffffu, incl, 1) : __shfl_up_sync(0xffffffffu, incl, 1);
+    if (kReverse ? lane == 31 : lane == 0) excl = INT_MIN;
+    if (!kBlock) return excl;
+    const int warp = threadIdx.x >> 5;
+    const int nwarps = blockDim.x >> 5;
+    if (kReverse ? lane == 0 : lane == 31) scratch[warp] = incl;
+    __syncthreads();
+    for (int i = 0; i < nwarps; ++i)
+        if (kReverse ? i > warp : i < warp) excl = max(excl, scratch[i]);
+    __syncthreads();
+    return excl;
+}
+
+// The W walks of a start node advance one step at a time (the kStepSync schedule of walk_merge_kernel, which
+// this generalises).  Per length l: the visits are sorted by (node, walk) -- in registers when a warp owns the
+// node (KPL keys per lane), in shared memory when a CTA does -- and parked as `keys`; every thread then owns
+// the contiguous stretch [tg * chunk, tg * chunk + chunk) of the sorted order, and that one order serves
+//   1. the merge: one entry per distinct node, loads added in walk order (the arithmetic of walk_merge_kernel);
+//   2. the halting decisions of the walks at length l (partner's word for antithetic termination);
+//   3. with repelling neighbours, a segmented rank / count of the continuing walks over the node runs:
+//      j = continuing walks before this one at its node, m = continuing walks at its node, from one add scan
+//      and two max scans (the cont-position of the last run head before and of the first run head after the
+//      thread's stretch) -- no extra shared memory, so the W limit is the one-length limit of kStepSync;
+//   4. the neighbour draws and edge gathers, which write the walker state of length l + 1.
+// Between 2 and 4 nodes[w] is free (the keys hold the nodes) and carries (cont, head cont-position, j) of
+// walk w; W < 2^15 (shared memory bounds it far below) keeps those in 15-bit fields.
+template <bool kBlock, typename KeyT, int KPL>
+__global__ void __launch_bounds__(kBlock ? 256 : 128) walk_coupled_kernel(const WalkParams p) {
+    const uint64_t keep = l2_policy_keep(), stream_pol = l2_policy_stream();
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int GS = kBlock ? (int)blockDim.x : 32;
+    const int tg = kBlock ? (int)threadIdx.x : (int)(threadIdx.x & 31);
+    const int groups_per_cta = kBlock ? 1 : (int)(blockDim.x >> 5);
+    const int group_in_cta = kBlock ? 0 : (int)(threadIdx.x >> 5);
+
+    unsigned char *base = smem_raw + (size_t)group_in_cta * p.group_bytes;
+    double *loads = reinterpret_cast<double *>(base);                                       // [W]
+    int32_t *nodes = reinterpret_cast<int32_t *>(base + p.loads_bytes);                     // [W], -1 = stopped
+    KeyT *keys = reinterpret_cast<KeyT *>(base + p.loads_bytes + p.nodes_bytes);            // [n_keys]
+    __shared__ int scan_scratch[32];
+
+    const int W = p.W, L = p.L, wbits = p.wbits;
+    const int n_keys = kBlock ? p.Wp : 32 * KPL;
+    const int chunk = n_keys / GS;
+    const int lo = tg * chunk, hi = lo + chunk;
+    const KeyT KEY_MAX = ~(KeyT)0;
+    const KeyT wmask = ((KeyT)1 << wbits) - 1;
+    const bool couple_halt = (p.draw_mode & GRF_DRAW_COUPLE_HALT) != 0;
+    const bool repel = (p.draw_mode & GRF_DRAW_COUPLE_NEIGHBOURS) != 0;
+    unsigned long long my_visits = 0;
+
+    for (int64_t row = (int64_t)blockIdx.x * groups_per_cta + group_in_cta; row < p.n_local;
+         row += (int64_t)gridDim.x * groups_per_cta) {
+        const int64_t start = p.start_lo + row;
+        for (int w = tg; w < W; w += GS) {
+            nodes[w] = (int32_t)start;
+            loads[w] = 1.0;
+        }
+        group_sync<kBlock>();
+
+        int32_t *out_col = p.stage_ent ? nullptr : p.stage_col + row * p.stride;
+        double *out_sum = p.stage_ent ? nullptr : p.stage_sum + row * p.stride;
+        GrfEntry *out_ent = p.stage_ent ? p.stage_ent + row * p.stride : nullptr;
+        auto emit = [&](int slot, int32_t node, double sum, int length) {
+            if (out_ent) {
+                GrfEntry en;
+                en.col = pack_col(node, length);
+                en.val = (float)(p.scale_mode == GRF_SCALE_MUL_RECIP ? __dmul_rn(sum, p.recip_w)
+                                                                      : __ddiv_rn(sum, p.w_as_double));
+                out_ent[slot] = en;
+            } else {
+                out_col[slot] = node;
+                out_sum[slot] = sum;
+            }
+        };
+        // walk w leaves node v (CSR row rs .. rs + deg) through neighbour index k: load update as
+        // walk_merge_kernel's phase 1 (16-byte edge records when given)
+        auto move = [&](int w, int32_t rs, int32_t deg, int32_t k) {
+            const int64_t e = (int64_t)rs + k;
+            int32_t nxt;
+            double fac;
+            if (p.edges) {
+                const GrfEdge ed = ld_stream_edge(p.edges + e, stream_pol);
+                nxt = ed.col;
+                fac = p.load_mode == GRF_LOAD_ABLATION ? __ldg(p.val + e) : ed.scaled;
+            } else {
+                nxt = __ldg(p.col_idx + e);
+                const double wv = __ldg(p.val + e);
+                fac = p.load_mode == GRF_LOAD_ABLATION ? wv : __ddiv_rn(__dmul_rn((double)deg, wv), p.one_minus_p);
+            }
+            loads[w] = p.load_mode == GRF_LOAD_CUMULATIVE ? __dmul_rn(loads[w], fac) : fac;
+            nodes[w] = nxt;
+        };
+        auto is_head = [&](int i, KeyT key) { return i == 0 || (keys[i - 1] >> wbits) != (key >> wbits); };
+
+        int off = 0;
+        for (int l = 0; l < L; ++l) {
+            // ---- the visits of length l, sorted by (node, walk) ----
+            if constexpr (!kBlock) {
+                KeyT key[KPL];
+                bool have = false;
+#pragma unroll
+                for (int r = 0; r < KPL; ++r) {
+                    const int w = r * 32 + tg;
+                    KeyT kk = KEY_MAX;
+                    if (w < W) {
+                        const int32_t nd = nodes[w];
+                        if (nd >= 0) kk = ((KeyT)(uint32_t)nd << wbits) | (KeyT)w;
+                    }
+                    key[r] = kk;
+                    have |= kk != KEY_MAX;
+                }
+                if (!__any_sync(0xffffffffu, have)) {  // every walk has stopped
+                    if (tg == 0)
+                        for (int s2 = l; s2 < L; ++s2) p.row_cnt[row * L + s2] = 0;
+                    break;
+                }
+                warp_bitonic_sort<KeyT, KPL>(key, tg);
+#pragma unroll
+                for (int r = 0; r < KPL; ++r) keys[tg * KPL + r] = key[r];
+                __syncwarp();
+            } else {
+                int have = 0;
+                for (int i = tg; i < n_keys; i += GS) {
+                    KeyT key = KEY_MAX;
+                    if (i < W) {
+                        const int32_t nd = nodes[i];
+                        if (nd >= 0) key = ((KeyT)(uint32_t)nd << wbits) | (KeyT)i;
+                    }
+                    keys[i] = key;
+                    have |= key != KEY_MAX;
+                }
+                if (!__syncthreads_or(have)) {
+                    if (tg == 0)
+                        for (int s2 = l; s2 < L; ++s2) p.row_cnt[row * L + s2] = 0;
+                    break;
+                }
+                for (uint32_t k = 2; k <= (uint32_t)n_keys; k <<= 1) {
+                    for (uint32_t j = k >> 1; j > 0; j >>= 1) {
+                        for (uint32_t c = tg; c < (uint32_t)n_keys / 2; c += GS) {
+                            const uint32_t idx = ((c & ~(j - 1)) << 1) | (c & (j - 1));
+                            const uint32_t ixj = idx | j;
+                            const KeyT a = keys[idx], b = keys[ixj];
+                            const bool up = (idx & k) == 0;
+                            if ((a > b) == up) {
+                                keys[idx] = b;
+                                keys[ixj] = a;
+                            }
+                        }
+                        __syncthreads();
+                    }
+                }
+            }
+
+            // ---- 1. merge: one entry per distinct node, loads added in walk order ----
+            int heads = 0;
+            for (int i = lo; i < hi; ++i) {
+                const KeyT key = keys[i];
+                if (key == KEY_MAX) break;
+                ++my_visits;
+                heads += is_head(i, key);
+            }
+            int total;
+            int rank = group_excl_scan<kBlock>(heads, scan_scratch, total);
+            for (int i = lo; i < hi; ++i) {
+                const KeyT key = keys[i];
+                if (key == KEY_MAX) break;
+                if (!is_head(i, key)) continue;
+                const KeyT node = key >> wbits;
+                double sum = 0.0;
+                for (int q = i; q < n_keys; ++q) {
+                    const KeyT kq = keys[q];
+                    if ((kq >> wbits) != node) break;
+                    sum = __dadd_rn(sum, loads[(int)(kq & wmask)]);
+                }
+                emit(off + rank, (int32_t)node, sum, l);
+                if (p.col_counts) atomicAdd(p.col_counts + (int64_t)node * L + l, 1);
+                ++rank;
+            }
+            if (tg == 0) p.row_cnt[row * L + l] = total;
+            off += total;
+            if (l == L - 1) break;
+            group_sync<kBlock>();  // the merge has read every load: the moves below may overwrite them
+
+            // ---- 2. halting decisions at step l ----
+            int n_cont = 0, first_head = -1, last_head = -1;  // cont-positions (within the stretch) of run heads
+            for (int i = lo; i < hi; ++i) {
+                const KeyT key = keys[i];
+                if (key == KEY_MAX) break;
+                const int w = (int)(key & wmask);
+                const int32_t v = (int32_t)(key >> wbits);
+                if (is_head(i, key)) {
+                    if (first_head < 0) first_head = n_cont;
+                    last_head = n_cont;
+                }
+                const int32_t rs = ld_keep_s32(p.row_ptr + v, keep);
+                const int32_t deg = ld_keep_s32(p.row_ptr + v + 1, keep) - rs;
+                bool cont = false;
+                if (deg > 0) {  // a dead end stops the walk without a draw
+                    const int src = (couple_halt && (w & 1)) ? w - 1 : w;  // walk 2q+1 halts on walk 2q's word
+                    const unsigned long long gid = (unsigned long long)start * (unsigned long long)W + (unsigned)src;
+                    uint32_t x[4];
+                    philox4x32_10((uint32_t)gid, (uint32_t)(gid >> 32), (uint32_t)(l >> 1), 0u, p.k0, p.k1, x);
+                    const uint32_t xh = ((l & 1) ? x[2] : x[0]) ^ (src != w ? 0x80000000u : 0u);
+                    cont = (unsigned long long)xh >= p.halt_thr;
+                    if (cont && !repel) {  // independent neighbour: the walk's own word
+                        if (src != w) {
+                            const unsigned long long own = gid + 1;
+                            philox4x32_10((uint32_t)own, (uint32_t)(own >> 32), (uint32_t)(l >> 1), 0u, p.k0, p.k1,
+                                          x);
+                        }
+                        const uint32_t xk = (l & 1) ? x[3] : x[1];
+                        move(w, rs, deg, (int32_t)__umulhi(xk, (uint32_t)deg));
+                    }
+                }
+                if (repel)
+                    nodes[w] = cont;
+                else if (!cont)
+                    nodes[w] = -1;
+                n_cont += cont;
+            }
+            if (repel) {
+                // ---- 3. segmented rank / count of the continuing walks over the node runs ----
+                int n_all;
+                const int cpos0 = group_excl_scan<kBlock>(n_cont, scan_scratch, n_all);
+                const int head_before = group_excl_max<kBlock, false>(last_head >= 0 ? cpos0 + last_head : INT_MIN,
+                                                                      scan_scratch);
+                const int neg_head_after = group_excl_max<kBlock, true>(
+                    first_head >= 0 ? -(cpos0 + first_head) : INT_MIN, scan_scratch);
+                // forward: cont-position hc of the walk's run head and j = its own cont-position - hc
+                int c = cpos0, hc = head_before;
+                for (int i = lo; i < hi; ++i) {
+                    const KeyT key = keys[i];
+                    if (key == KEY_MAX) break;
+                    const int w = (int)(key & wmask);
+                    if (is_head(i, key)) hc = c;
+                    const int cont = nodes[w];
+                    nodes[w] = (cont << 30) | (hc << 15) | (c - hc);
+                    c += cont;
+                }
+                // backward: ec = cont-position of the next run head (or the total), m = ec - hc; the moves
+                int ec = neg_head_after == INT_MIN ? n_all : -neg_head_after;
+                for (int i = hi - 1; i >= lo; --i) {
+                    const KeyT key = keys[i];
+                    if (key == KEY_MAX) continue;
+                    const int w = (int)(key & wmask);
+                    const int32_t v = (int32_t)(key >> wbits);
+                    const int packed = nodes[w];
+                    const int hcw = (packed >> 15) & 0x7fff, j = packed & 0x7fff;
+                    if (packed >> 30) {
+                        const int m = ec - hcw;
+                        const int32_t rs = ld_keep_s32(p.row_ptr + v, keep);
+                        const int32_t deg = ld_keep_s32(p.row_ptr + v + 1, keep) - rs;
+                        uint32_t x[4];
+                        philox4x32_10((uint32_t)start, (uint32_t)v, (uint32_t)l, 1u, p.k0, p.k1, x);
+                        const uint64_t cg = __umulhi(x[0], (uint32_t)deg);
+                        const uint64_t k = (cg + (uint64_t)j * (uint64_t)deg / (uint64_t)m) % (uint64_t)deg;
+                        move(w, rs, deg, (int32_t)k);
+                    } else {
+                        nodes[w] = -1;
+                    }
+                    if (is_head(i, key)) ec = hcw;
+                }
+            }
+            group_sync<kBlock>();  // the state of length l + 1 is complete
+        }
+        group_sync<kBlock>();  // every read of this row's keys and loads is done before the next row
+    }
+
+    if (p.visits != nullptr) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) my_visits += __shfl_xor_sync(0xffffffffu, my_visits, d);
+        if ((threadIdx.x & 31) == 0 && my_visits) atomicAdd(p.visits, my_visits);
+    }
+}
+
+template <bool kBlock, typename KeyT, int KPL>
+static int launch_coupled(const WalkParams &p, size_t smem, int threads, int grid, cudaStream_t stream) {
+    auto kern = walk_coupled_kernel<kBlock, KeyT, KPL>;
+    GRF_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, threads, smem, stream>>>(p);
+    return check_cuda(cudaGetLastError(), "walk_coupled_kernel launch");
+}
+
+// The coupled draws take the step-synchronous schedule: shared memory holds one length's visit records
+// (W x 12 bytes) and the sort keys.  W <= 256: a warp per start node, four per CTA; else a CTA per start node.
+static int walk_coupled(WalkParams &p, bool key32, int64_t n_nodes, cudaStream_t st) {
+    const size_t key_size = key32 ? 4 : 8;
+    const size_t kMaxSmem = 227 * 1024 - 256;
+    p.loads_bytes = (uint32_t)(((size_t)p.W * 8 + 15) & ~(size_t)15);
+    p.nodes_bytes = (uint32_t)(((size_t)p.W * 4 + 15) & ~(size_t)15);
+    p.sorted_bytes = 0;
+    if (p.W <= 256) {
+        const int kpl = p.Wp <= 32 ? 1 : p.Wp / 32;
+        const size_t gb = ((size_t)p.loads_bytes + p.nodes_bytes + (size_t)32 * kpl * key_size + 15) & ~(size_t)15;
+        p.group_bytes = (uint32_t)gb;
+        const int warps = 4;
+        const int64_t want = (p.n_local + warps - 1) / warps;
+        const int grid = (int)(want < (int64_t)kSmCount * 64 ? want : (int64_t)kSmCount * 64);
+        const size_t smem = warps * gb;
+        const int threads = warps * 32;
+#define GRF_COUPLED_CASE(K)                                                                  \
+    case K:                                                                                  \
+        return key32 ? launch_coupled<false, uint32_t, K>(p, smem, threads, grid, st)       \
+                     : launch_coupled<false, unsigned long long, K>(p, smem, threads, grid, st)
+        switch (kpl) {
+            GRF_COUPLED_CASE(1);
+            GRF_COUPLED_CASE(2);
+            GRF_COUPLED_CASE(4);
+            default:
+                GRF_COUPLED_CASE(8);
+        }
+#undef GRF_COUPLED_CASE
+    }
+    const size_t gb = ((size_t)p.loads_bytes + p.nodes_bytes + (size_t)p.Wp * key_size + 15) & ~(size_t)15;
+    if (gb > kMaxSmem)
+        return fail(GRF_ERR_UNSUPPORTED,
+                    "grf_walk: W=%d needs %zu B of shared memory per start node for one walk length (max %zu; "
+                    "%d-byte sort keys for %lld nodes)", p.W, gb, kMaxSmem, (int)key_size, (long long)n_nodes);
+    p.group_bytes = (uint32_t)gb;
+    const int grid = (int)(p.n_local < (int64_t)kSmCount * 32 ? p.n_local : (int64_t)kSmCount * 32);
+    return key32 ? launch_coupled<true, uint32_t, 0>(p, gb, 256, grid, st)
+                 : launch_coupled<true, unsigned long long, 0>(p, gb, 256, grid, st);
+}
+
 }  // namespace grf
 
 extern "C" int64_t grf_walk_stage_stride(int32_t walks_per_node, int32_t max_walk_length) {
@@ -547,7 +886,10 @@ extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t st
     GRF_REQUIRE(cfg->start_lo >= 0 && cfg->start_lo <= cfg->start_hi && cfg->start_hi <= graph->n_nodes,
                 "grf_walk: start range [%lld, %lld) outside [0, %lld)", (long long)cfg->start_lo,
                 (long long)cfg->start_hi, (long long)graph->n_nodes);
-    GRF_REQUIRE(cfg->draw_mode == GRF_DRAW_PHILOX || cfg->draw_mode == GRF_DRAW_REPLAY, "grf_walk: bad draw_mode");
+    const int32_t coupled = GRF_DRAW_COUPLE_HALT | GRF_DRAW_COUPLE_NEIGHBOURS;
+    GRF_REQUIRE((cfg->draw_mode & ~(GRF_DRAW_REPLAY | coupled)) == 0, "grf_walk: bad draw_mode");
+    GRF_REQUIRE(!(cfg->draw_mode & GRF_DRAW_REPLAY) || !(cfg->draw_mode & coupled),
+                "grf_walk: coupled draws need native Philox draws");
     GRF_REQUIRE(cfg->load_mode >= GRF_LOAD_CUMULATIVE && cfg->load_mode <= GRF_LOAD_ABLATION,
                 "grf_walk: bad load_mode");
     GRF_REQUIRE(cfg->draw_mode != GRF_DRAW_REPLAY || (cfg->trace_u && cfg->trace_k),
@@ -612,6 +954,7 @@ extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t st
     GRF_REQUIRE((uint64_t)p.W * (uint64_t)p.L < (1ull << 31), "grf_walk: W*L too large");
 
     cudaStream_t st = (cudaStream_t)stream;
+    if (cfg->draw_mode & coupled) return walk_coupled(p, key32, graph->n_nodes, st);
     // start nodes per CTA of the warp-per-node variant: as many of 4, 2, 1 as the visit records leave room for
     // (W = 200, L = 30: one group is 68 KB); none fits -> the CTA-per-node variants below
     int warps = 4;

@@ -39,14 +39,17 @@ def fast_general_grf_kernel(
     max_walk_length: int = 10,
     *,
     trace=None,
+    coupling: str = "iid",
 ) -> np.ndarray:
-    """GRF kernel estimate K ~ Phi Phi^T using importance-sampled random walks."""
+    """GRF kernel estimate K ~ Phi Phi^T using importance-sampled random walks.  ``coupling``: how the walks
+    of one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" = independent, as the reference)."""
     modulator_vector = np.asarray(modulator_vector, dtype=float)
     if modulator_vector.shape[0] != max_walk_length:
         # the reference fails inside ``feature_matrices @ modulator`` with a shape error (:38)
         raise ValueError("The length of the modulator vector must be equal to the max_walk_length.")
     laplacian = get_normalized_laplacian(adj_matrix)
     random_walk = RandomWalk(Graph(laplacian), seed=42)
-    steps = random_walk.get_step_matrices_device(walks_per_node, p_halt, max_walk_length, trace=trace)
+    steps = random_walk.get_step_matrices_device(walks_per_node, p_halt, max_walk_length, trace=trace,
+                                                   coupling=coupling)
     phi = _phi_from_steps(steps, modulator_vector)
     return (phi @ phi.T).cpu().numpy()

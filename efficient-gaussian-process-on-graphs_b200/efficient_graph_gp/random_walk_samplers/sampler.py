@@ -61,7 +61,7 @@ class RandomWalk:
         self._device = device
 
     def get_step_matrices_device(self, num_walks, p_halt, max_walk_length, ablation=False,
-                                 sequential_semantics=False, trace=None):
+                                 sequential_semantics=False, trace=None, *, coupling="iid"):
         csr = self.graph.to_csr()
         dg = DeviceGraph(csr.indptr, csr.indices, csr.data, self.graph.get_num_nodes(), self._device)
         if ablation:
@@ -72,7 +72,7 @@ class RandomWalk:
             load_mode = _lib.LOAD_CUMULATIVE
         cfg = WalkConfig(int(num_walks), float(p_halt), int(max_walk_length), seed=self.seed,
                          draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY,
-                         load_mode=load_mode, trace=trace)
+                         load_mode=load_mode, trace=trace, coupling=coupling)
         return build_step_matrices(dg, cfg, scale_mode=_lib.SCALE_DIV)  # value / num_walks, sampler.py:201
 
     def get_random_walk_matrices(
@@ -86,9 +86,11 @@ class RandomWalk:
         *,
         sequential_semantics: bool = False,
         trace=None,
+        coupling: str = "iid",
     ) -> np.ndarray:
-        """(num_nodes, num_nodes, max_walk_length) float64; [i, j, l] estimates (A^l)[i, j]."""
+        """(num_nodes, num_nodes, max_walk_length) float64; [i, j, l] estimates (A^l)[i, j].  ``coupling``:
+        how the walks of one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" = independent)."""
         del use_tqdm, n_processes
         steps = self.get_step_matrices_device(num_walks, p_halt, max_walk_length, ablation,
-                                              sequential_semantics, trace)
+                                              sequential_semantics, trace, coupling=coupling)
         return steps.to_dense_tensor()

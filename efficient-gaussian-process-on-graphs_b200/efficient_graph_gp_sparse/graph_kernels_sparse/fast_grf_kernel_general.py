@@ -23,11 +23,14 @@ def fast_general_grf_kernel(
     max_walk_length: int = 10,
     *,
     trace=None,
+    coupling: str = "iid",
 ):
-    """Sparse GRF kernel estimate K ~ Phi Phi^T on the normalized Laplacian."""
+    """Sparse GRF kernel estimate K ~ Phi Phi^T on the normalized Laplacian.  ``coupling``: how the walks of
+    one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" = independent, as the reference)."""
     # the Laplacian (graph_utils.py:5-30) is formed on the device, bit-identical to the host one
     random_walk = SparseRandomWalk.on_normalized_laplacian(adj_matrix, seed=None)
-    step_matrices = random_walk.get_random_walk_matrices(walks_per_node, p_halt, max_walk_length, trace=trace)
+    step_matrices = random_walk.get_random_walk_matrices(walks_per_node, p_halt, max_walk_length, trace=trace,
+                                                           coupling=coupling)
 
     num_nodes = adj_matrix.shape[0]
     Phi = sp.csr_matrix((num_nodes, num_nodes))

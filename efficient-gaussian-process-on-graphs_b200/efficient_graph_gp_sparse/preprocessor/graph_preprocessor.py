@@ -48,7 +48,9 @@ class GraphPreprocessor:
                  use_tqdm: bool = True,
                  cache_filename: Optional[str] = None,
                  n_processes: int = None,
-                 device=None) -> None:
+                 device=None,
+                 *,
+                 coupling: str = "iid") -> None:
         if adjacency_matrix.shape[0] != adjacency_matrix.shape[1]:
             raise ValueError("Adjacency matrix must be square.")
 
@@ -61,6 +63,7 @@ class GraphPreprocessor:
         self._cache_filename = cache_filename      # default name: hashed from the graph on first use (see below)
         self.n_processes = n_processes
         self.device = device
+        self.coupling = coupling   # grf_b200.engine.COUPLINGS: how the walks of one start node share their draws
         self._scipy = None
         self._steps_device = None
 
@@ -85,12 +88,15 @@ class GraphPreprocessor:
         self._cache_filename = value
 
     def _generate_cache_filename(self) -> str:
-        """Same key as the reference (graph_preprocessor.py:75-83), so caches are interchangeable."""
+        """Same key as the reference (graph_preprocessor.py:75-83), so caches are interchangeable; coupled
+        draws append the coupling, so that a coupled cache never answers an independent-draws request."""
         adj_hash = hashlib.md5(self.adj_matrix.data.tobytes() +
                                self.adj_matrix.indices.tobytes() +
                                self.adj_matrix.indptr.tobytes()).hexdigest()[:8]
         graph_size = self.adj_matrix.shape[0]
         params = f"{graph_size}_{self.walks_per_node}_{self.p_halt}_{self.max_walk_length}_{self.random_walk_seed}"
+        if self.coupling != "iid":
+            params += f"_{self.coupling}"
         return f"experiments_sparse/step_matrices/step_matrices_{adj_hash}_{params}.pkl"
 
     def _target_device(self) -> torch.device:
@@ -134,7 +140,8 @@ class GraphPreprocessor:
         graph = DeviceGraph.laplacian_of(self.adj_matrix, self.device)
         cfg = WalkConfig(int(self.walks_per_node), float(self.p_halt), int(self.max_walk_length),
                          seed=self.random_walk_seed or 42,
-                         draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace)
+                         draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace,
+                         coupling=self.coupling)
         self._steps_device = build_step_matrices(graph, cfg, scale_mode=_lib.SCALE_MUL_RECIP)
         self._scipy = None
         if save_to_disk:
@@ -156,7 +163,8 @@ class GraphPreprocessor:
         graph = DeviceGraph.laplacian_of(self.adj_matrix, self.device, group=group)
         cfg = WalkConfig(int(self.walks_per_node), float(self.p_halt), int(self.max_walk_length),
                          seed=self.random_walk_seed or 42,
-                         draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace)
+                         draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace,
+                         coupling=self.coupling)
         return build_phi_blocks(graph, cfg, start_lo, start_hi)
 
     @staticmethod

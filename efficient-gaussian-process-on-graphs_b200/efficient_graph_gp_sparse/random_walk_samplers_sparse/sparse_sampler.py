@@ -13,7 +13,11 @@ columns, ``M_0 = I``).  Differences, all deliberate (DESIGN.md):
   sparse_sampler.py:65) with counter (start*W + walk, step), so the result does
   not depend on how start nodes are sharded;
 * ``trace=(trace_u, trace_k)`` replays recorded draws of the reference's own
-  PCG64 streams instead -- the output is then bit-identical to the reference.
+  PCG64 streams instead -- the output is then bit-identical to the reference;
+* ``coupling=`` (keyword only, default ``"iid"``: the independent draws above)
+  couples the walks of one start node for a lower-variance estimate:
+  ``"antithetic"``, ``"repelling"`` or ``"antithetic+repelling"``
+  (``grf_b200.engine.COUPLINGS``; native draws only).
 """
 
 from typing import List, Optional
@@ -57,24 +61,24 @@ class SparseRandomWalk:
             self._graph = DeviceGraph(self.indptr, self.indices, self.data, self.num_nodes, self._device)
         return self._graph
 
-    def _config(self, num_walks, p_halt, max_walk_length, trace, trace_start=0) -> WalkConfig:
+    def _config(self, num_walks, p_halt, max_walk_length, trace, trace_start=0, coupling="iid") -> WalkConfig:
         return WalkConfig(
             walks_per_node=int(num_walks), p_halt=float(p_halt), max_walk_length=int(max_walk_length),
             seed=self.seed, draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace,
-            trace_start=int(trace_start))
+            trace_start=int(trace_start), coupling=coupling)
 
     def get_step_matrices_device(self, num_walks, p_halt, max_walk_length, start_lo=0, start_hi=None,
-                                 trace=None, trace_start=0) -> StepMatrices:
+                                 trace=None, trace_start=0, *, coupling="iid") -> StepMatrices:
         """The step matrices left in HBM (rows [start_lo, start_hi) only).  ``trace_start``: the first start
         node the replayed trace covers (a trace recorded for a row slice is indexed from there)."""
-        return build_step_matrices(self.graph, self._config(num_walks, p_halt, max_walk_length, trace, trace_start),
-                                   start_lo, start_hi, scale_mode=_lib.SCALE_MUL_RECIP)
+        cfg = self._config(num_walks, p_halt, max_walk_length, trace, trace_start, coupling)
+        return build_step_matrices(self.graph, cfg, start_lo, start_hi, scale_mode=_lib.SCALE_MUL_RECIP)
 
     def get_phi_blocks(self, num_walks, p_halt, max_walk_length, start_lo=0, start_hi=None, trace=None,
-                       trace_start=0) -> PhiBlocks:
+                       trace_start=0, *, coupling="iid") -> PhiBlocks:
         """Phi in the matvec layout, built without leaving the device."""
-        return build_phi_blocks(self.graph, self._config(num_walks, p_halt, max_walk_length, trace, trace_start),
-                                start_lo, start_hi)
+        cfg = self._config(num_walks, p_halt, max_walk_length, trace, trace_start, coupling)
+        return build_phi_blocks(self.graph, cfg, start_lo, start_hi)
 
     def get_random_walk_matrices(
         self,
@@ -85,6 +89,8 @@ class SparseRandomWalk:
         n_processes: Optional[int] = None,
         *,
         trace=None,
+        coupling: str = "iid",
     ) -> List[sp.csr_matrix]:
         del use_tqdm, n_processes
-        return self.get_step_matrices_device(num_walks, p_halt, max_walk_length, trace=trace).to_scipy()
+        return self.get_step_matrices_device(num_walks, p_halt, max_walk_length, trace=trace,
+                                             coupling=coupling).to_scipy()

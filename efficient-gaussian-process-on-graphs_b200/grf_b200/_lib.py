@@ -17,6 +17,7 @@ SO_PATH = os.environ.get("GRF_B200_SO") or os.path.join(_HERE, "libgrf_b200.so")
 
 GRF_OK, GRF_ERR_INVALID, GRF_ERR_CUDA, GRF_ERR_UNSUPPORTED = 0, -1, -2, -3
 DRAW_PHILOX, DRAW_REPLAY = 0, 1
+DRAW_COUPLE_HALT, DRAW_COUPLE_NEIGHBOURS = 2, 4   # OR-ed into draw_mode with DRAW_PHILOX
 LOAD_CUMULATIVE, LOAD_LAST_STEP, LOAD_ABLATION = 0, 1, 2
 SCALE_MUL_RECIP, SCALE_DIV = 0, 1
 ORDER_ROW_MAJOR, ORDER_STEP_MAJOR = 0, 1

@@ -100,6 +100,17 @@ def _stream(device: torch.device):
     return ctypes.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+# WalkConfig.coupling -> GRF_DRAW_COUPLE_* bits (definitions at GrfWalkCfg.seed in include/grf_b200.h):
+# "antithetic" pairs the halting draws of walks (2q, 2q+1), "repelling" spreads the walks of a start node that
+# stand on the same node over its neighbours.  Every walk keeps its marginal law: M_l stays unbiased.
+COUPLINGS = {
+    "iid": 0,
+    "antithetic": _lib.DRAW_COUPLE_HALT,
+    "repelling": _lib.DRAW_COUPLE_NEIGHBOURS,
+    "antithetic+repelling": _lib.DRAW_COUPLE_HALT | _lib.DRAW_COUPLE_NEIGHBOURS,
+}
+
+
 @dataclass
 class WalkConfig:
     """Arguments of the reference's walk loop (sparse_sampler.py:26-31) + draw source."""
@@ -112,6 +123,7 @@ class WalkConfig:
     load_mode: int = _lib.LOAD_CUMULATIVE
     trace: Optional[Tuple] = None  # (trace_u float64, trace_k int32), [(walk_id - trace_start*W)*L + step]
     trace_start: int = 0           # first start node the trace covers (a trace recorded for a row slice)
+    coupling: str = "iid"          # one of COUPLINGS: how the W walks of a start node share their draws
 
     def validate(self):
         if int(self.walks_per_node) < 1:
@@ -122,6 +134,14 @@ class WalkConfig:
             raise ValueError("p_halt must be in [0, 1]")
         if self.draw_mode == _lib.DRAW_REPLAY and self.trace is None:
             raise ValueError("replay mode needs trace=(trace_u, trace_k)")
+        if self.coupling not in COUPLINGS:
+            raise ValueError(f"coupling must be one of {sorted(COUPLINGS)}, not {self.coupling!r}")
+        if COUPLINGS[self.coupling] and (self.draw_mode != _lib.DRAW_PHILOX or self.trace is not None):
+            raise ValueError("coupled draws need native Philox draws (no replayed trace)")
+
+    def draw_flags(self) -> int:
+        """draw_mode of GrfWalkCfg: the draw source with the coupling bits OR-ed in."""
+        return int(self.draw_mode) | COUPLINGS[self.coupling]
 
 
 def _to_host_pinned(t: torch.Tensor) -> torch.Tensor:
@@ -394,7 +414,7 @@ def run_walker(graph: DeviceGraph, cfg: WalkConfig, start_lo: int = 0, start_hi:
     edges = None
     if cfg.load_mode != _lib.LOAD_ABLATION and cfg.max_walk_length > 1 and graph.nnz > 0 and cfg.p_halt < 1.0:
         edges = graph.edge_records(cfg.p_halt)
-    c = GrfWalkCfg(start_lo, start_hi, cfg.walks_per_node, cfg.max_walk_length, float(cfg.p_halt), cfg.draw_mode,
+    c = GrfWalkCfg(start_lo, start_hi, cfg.walks_per_node, cfg.max_walk_length, float(cfg.p_halt), cfg.draw_flags(),
                    cfg.load_mode, int(cfg.seed) & 0xFFFFFFFFFFFFFFFF,
                    None if tu is None else tu.data_ptr(), None if tk is None else tk.data_ptr(),
                    None if edges is None else edges.data_ptr(),

@@ -47,6 +47,9 @@ enum {
 };
 
 enum { GRF_DRAW_PHILOX = 0, GRF_DRAW_REPLAY = 1 };
+/* Coupled draws of the W walks of one start node (native Philox draws only; OR them into draw_mode).
+ * Every walk keeps its marginal law, so every M_l stays unbiased; see GrfWalkCfg.seed for the definitions. */
+enum { GRF_DRAW_COUPLE_HALT = 2, GRF_DRAW_COUPLE_NEIGHBOURS = 4 };
 /* load rule: sparse_sampler.py:54 & sampler.py:58 | sampler.py:183 | sampler.py:180-181 */
 enum { GRF_LOAD_CUMULATIVE = 0, GRF_LOAD_LAST_STEP = 1, GRF_LOAD_ABLATION = 2 };
 /* "/ num_walks": scipy csr / W == * (1/W) (sparse_sampler.py:130) | true division (sampler.py:201) */
@@ -90,11 +93,27 @@ typedef struct {
     int32_t walks_per_node;     /* W */
     int32_t max_walk_length;    /* L */
     double p_halt;
-    int32_t draw_mode;          /* GRF_DRAW_* */
+    int32_t draw_mode;          /* GRF_DRAW_PHILOX | GRF_DRAW_COUPLE_* flags, or GRF_DRAW_REPLAY alone */
     int32_t load_mode;          /* GRF_LOAD_* */
     uint64_t seed;              /* Philox key (native mode): counter (walk_lo, walk_hi, step/2, 0); words
                                  * (0,1) of the block halt / pick at the even step, (2,3) at the odd one;
-                                 * halt iff word < floor(p_halt * 2^32); neighbour = (word * deg) >> 32 */
+                                 * halt iff word < floor(p_halt * 2^32); neighbour = (word * deg) >> 32.
+                                 * A dead end (deg = 0) stops a walk without a draw.
+                                 * GRF_DRAW_COUPLE_HALT (antithetic termination): walks pair up as
+                                 *   (2q, 2q+1), 2q+1 < W (an odd W leaves the last walk unpaired); walk
+                                 *   2q+1 halts on the halting word of walk 2q (same step, taken from its
+                                 *   counter whether or not walk 2q is still alive) XOR 0x80000000.
+                                 *   Neighbour words are unchanged.
+                                 * GRF_DRAW_COUPLE_NEIGHBOURS (repelling neighbours): at step s, the
+                                 *   m walks of one start node that stand on node v, are still walking
+                                 *   and do not halt at s, taken in walk order (rank j), share the group
+                                 *   word U = word 0 of philox(counter = (start, v, s, 1)):
+                                 *   c = (U * deg(v)) >> 32, and rank j takes neighbour index
+                                 *   (c + floor(j * deg(v) / m)) mod deg(v) (64-bit integers); its own
+                                 *   neighbour word is unused.  m <= deg: m distinct neighbours; m > deg:
+                                 *   floor(m/deg) or ceil(m/deg) walks per neighbour.
+                                 * Visits of one (start, length, node) are summed in walk order into a
+                                 * double that starts at 0.0 in every mode. */
     /* replay mode: the reference's PCG64 draws, [walk_id*L + step], walk_id =
      * start*W + w; trace_u = rng.random() (NaN where none was drawn), trace_k =
      * rng.integers(deg) (-1 where none) -- sparse_sampler.py:47,51 */
@@ -189,7 +208,9 @@ int64_t grf_walk_stage_stride(int32_t walks_per_node, int32_t max_walk_length);
  * registers, and merges equal (length, node) visits of one start node in
  * shared memory -- loads added in walk order into a double, as the reference's
  * defaultdict does.  Writes stage_col / stage_sum (unscaled sums) and row_cnt;
- * *visits_out (device, may be NULL) += number of walk-steps executed. */
+ * *visits_out (device, may be NULL) += number of walk-steps executed.  With a
+ * GRF_DRAW_COUPLE_* bit in cfg->draw_mode the W walks of a start node advance
+ * one step at a time with coupled draws (same outputs, same summation). */
 int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t stage_stride, int32_t *stage_col,
              double *stage_sum, int32_t *row_cnt, unsigned long long *visits_out, void *stream);
 

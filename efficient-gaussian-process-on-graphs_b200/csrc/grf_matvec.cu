@@ -919,9 +919,11 @@ static int launch_spmm_pass(const int32_t *ptr, const GrfEntry *ent, const float
                             const int32_t *row_ids, int64_t n_tasks, int64_t row_lo, int64_t n_rows,
                             const GrfLongRows *lr, const float *X, int64_t ldx, float *Y, int64_t ldy, int32_t t_valid,
                             bool vec_ok, bool out_by_row, int64_t avg_row_len, int64_t x_rows, int32_t *sched,
-                            bool accumulate, bool stream_gather, cudaStream_t st) {
+                            bool accumulate, bool stream_gather, bool y_pad_is_scratch, cudaStream_t st) {
     // vec_ok: X rows are 16-byte aligned and padded to a multiple of 4 columns -> compute the padded
-    // column count with float4 gathers; only the t_valid real columns are stored to Y
+    // column count with float4 gathers.  y_pad_is_scratch: columns [t_valid, ldy) of Y are workspace (U),
+    // so whole padded rows may be stored; otherwise (the caller's `out`) only the t_valid real columns are
+    // written
     const bool split = lr && lr->n_long > 0 && (!row_ids || out_by_row);
     if (split) {
         GRF_REQUIRE(lr->rows && lr->chunk_ptr && lr->chunk_bounds && lr->partial && lr->ld >= t_valid,
@@ -973,12 +975,13 @@ static int launch_spmm_pass(const int32_t *ptr, const GrfEntry *ent, const float
         return GRF_OK;
     }
     const int32_t t = vec_ok ? (t_valid + 3) & ~3 : t_valid;
+    const int32_t t_store = y_pad_is_scratch && ldy >= t ? t : t_valid;
     const int32_t vec_store = (ldy % 4 == 0) && aligned16(Y);
     const Shape sh = pick_shape(t, vec_ok);
     const int grid = spmm_grid(n_tasks, sh.tpr);
     GRF_DISPATCH_SPMM(sh, stream_gather,
                       <<<grid, 256, 0, st>>>(ptr, ent, f, L, row_ids, n_tasks, row_lo, n_rows, X, ldx, Y, ldy, t,
-                                             ldy >= t ? t : t_valid, vec_store, split ? lr->threshold : 0, nullptr,
+                                             t_store, vec_store, split ? lr->threshold : 0, nullptr,
                                              out_by_row ? 1 : 0, sched, accumulate ? 1 : 0));
     GRF_CUDA_OK(cudaGetLastError());
     if (split) {
@@ -992,8 +995,8 @@ static int launch_spmm_pass(const int32_t *ptr, const GrfEntry *ent, const float
         GRF_CUDA_OK(cudaGetLastError());
         int64_t g = ((int64_t)lr->n_long * t + 255) / 256;
         if (g > (int64_t)kSmCount * 8) g = (int64_t)kSmCount * 8;
-        long_reduce_kernel<<<(int)g, 256, 0, st>>>(lr->rows, lr->chunk_ptr, lr->partial, lr->ld, Y, ldy,
-                                                   ldy >= t ? t : t_valid, lr->n_long, accumulate ? 1 : 0);
+        long_reduce_kernel<<<(int)g, 256, 0, st>>>(lr->rows, lr->chunk_ptr, lr->partial, lr->ld, Y, ldy, t_store,
+                                                   lr->n_long, accumulate ? 1 : 0);
         GRF_CUDA_OK(cudaGetLastError());
     }
     return GRF_OK;
@@ -1092,11 +1095,11 @@ extern "C" int grf_phi_matvec(const GrfPhi *phi, const float *f, const int32_t *
                              ? GRF_OK
                              : launch_spmm_pass(phi->tblk_ptr, phi->tentries, f, L, phi->tcols, phi->n_tcols, 0,
                                                 phi->n_cols, phi->long_t, src, lds, u, ldu, t, vec_ok, true, avg_len, phi->n_rows, phi->sched,
-                                                accumulate, stream_gather, st);
+                                                accumulate, stream_gather, true, st);
                 } else {
                     rc = launch_spmm_pass(phi->tblk_ptr, phi->tentries, f, L, nullptr, phi->n_cols, 0, phi->n_cols,
                                           phi->long_t, src, lds, u, ldu, t, vec_ok, false, avg_len, phi->n_rows, phi->sched,
-                                          accumulate, stream_gather, st);
+                                          accumulate, stream_gather, true, st);
                 }
                 if (rc != GRF_OK) return rc;
             }
@@ -1116,7 +1119,7 @@ extern "C" int grf_phi_matvec(const GrfPhi *phi, const float *f, const int32_t *
         if (!tiled) {
             const int rc = launch_spmm_pass(phi->blk_ptr, phi->entries, f, L, x1, n1, phi->row_lo, phi->n_rows,
                                             phi->long_fwd, u, ldu, out, ldo, t, vec_ok, false, avg_len, phi->n_cols, phi->sched,
-                                            false, stream_gather, st);
+                                            false, stream_gather, false, st);
             if (rc != GRF_OK) return rc;
         }
     }

@@ -310,7 +310,9 @@ int grf_transpose_fill(const int32_t *blk_ptr, const GrfEntry *entries, int64_t 
  * [row_lo, row_lo + n_rows) are not this GPU's and are skipped (their out rows
  * are left untouched).  V [n2][ldv], out [n1][ldo], U workspace [n_cols][ldu]
  * (= Phi[x2]^T V, this GPU's partial sum: the multi-GPU caller all-reduces it
- * between the two halves); vfull workspace [n_rows][ldu], used when x2 != NULL.
+ * between the two halves); vfull workspace [n_rows][ldu], used when x2 != NULL.  Only columns [0, t)
+ * of `out` are written; columns [t, ldu) of U and of vfull are scratch (the kernels may compute and
+ * store the padding of the column count to a multiple of 4 there; what they hold never reaches `out`).
  * When x2 selects fewer than 1/16 of the local rows (a BO training set), the first half scatters
  * from those rows of Phi with fp32 atomics instead of passing over Phi^T (cost proportional to the
  * selected rows; summation order not fixed).

@@ -32,6 +32,8 @@ EXPORTS = (
     "grf_phi_matvec", "grf_phi_fgrad", "grf_phi_row_dots", "grf_block_windows", "grf_edge_records", "grf_compact_entries", "grf_union_rank", "grf_union_fill",
     "grf_union_materialize", "grf_pairs_count", "grf_pairs_index", "grf_pairs_fill", "grf_pairs_spmm", "grf_pairs_matvec", "grf_cg_num_partials", "grf_cg_dot", "grf_cg_update", "grf_cg_direction",
     "grf_laplacian_count", "grf_laplacian_fill", "grf_shard_reach", "grf_exchange_flag_bytes", "grf_exchange_sum", "grf_exchange_sum_nvls",
+    "grf_kmat_phi_count", "grf_kmat_phi_fill", "grf_kmat_transpose_count", "grf_kmat_transpose_fill", "grf_kmat_row_sizes",
+    "grf_kmat_bin", "grf_kmat_workspace_bytes", "grf_kmat_count", "grf_kmat_fill",
 )
 
 
@@ -174,6 +176,26 @@ def lib():
     L.grf_phi_fgrad.argtypes = [POINTER(GrfPhi), vp, i64, vp, i64, vp, i64, i32, vp, vp]
     L.grf_phi_row_dots.restype = i32
     L.grf_phi_row_dots.argtypes = [POINTER(GrfPhi), vp, vp, vp, i64, vp, vp]
+    L.grf_kmat_phi_count.restype = i32
+    L.grf_kmat_phi_count.argtypes = [vp, vp, vp, i64, i32, vp, i32, i32, vp, vp]
+    L.grf_kmat_phi_fill.restype = i32
+    L.grf_kmat_phi_fill.argtypes = [vp, vp, vp, i64, i32, vp, i32, i32, vp, vp, vp, vp]
+    L.grf_kmat_transpose_count.restype = i32
+    L.grf_kmat_transpose_count.argtypes = [vp, vp, i64, i64, vp, vp]
+    L.grf_kmat_transpose_fill.restype = i32
+    L.grf_kmat_transpose_fill.argtypes = [vp, vp, vp, i64, i64, vp, vp, vp, vp, vp]
+    L.grf_kmat_row_sizes.restype = i32
+    L.grf_kmat_row_sizes.argtypes = [vp, vp, vp, i64, vp, vp]
+    L.grf_kmat_bin.restype = i32
+    L.grf_kmat_bin.argtypes = [vp, i64, vp, vp, vp]
+    L.grf_kmat_workspace_bytes.restype = i64
+    L.grf_kmat_workspace_bytes.argtypes = [i32, i32]
+    L.grf_kmat_count.restype = i32
+    L.grf_kmat_count.argtypes = [vp, vp, vp, vp, vp, vp, i64, vp, vp, POINTER(c_int64), i32, i32, vp, i64, vp, vp, vp,
+                                 vp]
+    L.grf_kmat_fill.restype = i32
+    L.grf_kmat_fill.argtypes = [vp, vp, vp, vp, vp, vp, i64, vp, vp, POINTER(c_int64), i32, i32, vp, i64, vp, vp, vp,
+                                vp, vp]
     if L.grf_abi_version() != ABI_VERSION:
         raise RuntimeError("grf_b200: ABI version mismatch between _lib.py and libgrf_b200.so")
     _lib = L

@@ -496,6 +496,15 @@ class StepMatrices:
             mats.append(m)
         return mats
 
+    def kernel_matrix(self, f, **kwargs):
+        """K = Phi_f Phi_f^T with Phi_f = sum_p f_p M_p (p < min(len(f), L)), formed on the device: a
+        ``kernel_matrix.KernelMatrix`` (device indptr / indices / data, ``.to_scipy()``) equal to the reference's
+        scipy ``Phi @ Phi.T`` (fast_grf_kernel_general.py:48-55) in every array.  Raises MemoryError, naming
+        nnz(K), when K does not fit in free device memory."""
+        from .kernel_matrix import kernel_matrix
+
+        return kernel_matrix(self, f, **kwargs)
+
     def to_dense_tensor(self) -> np.ndarray:
         """(n_rows, n_cols, L) float64 -- RandomWalk's output layout (sampler.py:196-201)."""
         return self.to_dense_device().cpu().numpy() if self.n_rows * self.n_cols * self.n_steps < (1 << 22) \

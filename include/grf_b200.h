@@ -302,6 +302,60 @@ int grf_transpose_fill(const int32_t *blk_ptr, const GrfEntry *entries, int64_t 
                        int32_t n_steps, int64_t entry_lo, int64_t nnz, void *workspace, GrfEntry *tentries,
                        void *stream);
 
+/* Sparse kernel matrix K = Phi_f Phi_f^T (csrc/grf_kernel_matrix.cu).  Replaces
+ * graph_kernels_sparse/fast_grf_kernel_general.py:48-55 (Phi = sum_p f_p M_p by scipy additions, then
+ * Phi @ Phi.T by scipy's csr_matmat) with the same float64 roundings, zero-drop and entry order, so that the
+ * three arrays equal scipy's element for element.  Shapes: Phi_f n_rows x n_cols, K n_rows x n_rows.
+ *   grf_kmat_phi_count / _fill   Phi_f from the step matrices (offsets int64[n_steps*n_rows + 1] step-major),
+ *                         using steps p < n_f only (n_f = min(len(f), L) <= 128, f float64: device, or host
+ *                         with f_on_host = 1): acc = 0.0, acc = acc + f_p * m over the steps that store the
+ *                         entry in ascending p (no FMA; stored zeros of M_p take part), stored iff acc != 0
+ *                         (NaN is kept).  count: phi_cnt[n_rows]; caller scans (grf_scan_counts(n_rows, 1),
+ *                         int64) -> phi_ptr; fill writes sorted int32 columns and float64 values
+ *   grf_kmat_transpose_count / _fill   Phi_f^T as CSR over the n_cols columns: a COUNTING transpose with an
+ *                         atomic cursor per column (cursor: int64[n_cols] scratch), so the ORDER OF THE ROWS
+ *                         INSIDE A COLUMN IS UNSPECIFIED -- the product only needs the k order, and within one
+ *                         k every row j occurs once.  count zeroes and fills tcnt[n_cols]; caller scans
+ *                         (int64) -> tptr [n_cols + 1]
+ *   grf_kmat_row_sizes    size[i] = min(products of row i, n_rows): an upper bound on the j row i touches
+ *   grf_kmat_bin          rows [3][n_rows]: the rows of each bin (order not deterministic, results are);
+ *                         stats int64[4] = {rows of bin 0, 1, 2, largest size in bin 2}.  Bins: size <= 256
+ *                         warp per row, shared-memory hash; <= 2048 CTA per row, shared-memory hash; larger
+ *                         CTA per row with its hash in `workspace` (grf_kmat_workspace_bytes(max_size,
+ *                         global_ctas) bytes, global_ctas CTAs).  Every table holds next_pow2(2 * size) slots
+ *                         for the row's size; a row that touches more j than its size sets *overflow
+ *   grf_kmat_count        sizes from grf_kmat_row_sizes: touched[i] = distinct j (scipy's csr_matmat_maxnnz
+ *                         per row), stored[i] = j with sum != 0.  The count COMPUTES THE SUMS (zero-drop
+ *                         makes the stored count value-dependent); caller scans stored -> kptr (int64)
+ *   grf_kmat_fill         sizes = touched (re-binned): writes row i at kptr[i] in scipy's order, DESCENDING by
+ *                         (first k that touched j, j), i.e. not sorted by column
+ * bin_rows: HOST int64[3] (stats[0..3) read back); max_size: stats[3].  *overflow (device int32) is zeroed by
+ * count / fill and set to 1 if any row outgrew its table or (fill) disagrees with kptr. */
+int grf_kmat_phi_count(const int64_t *offsets_step_major, const int32_t *col, const double *val, int64_t n_rows,
+                       int32_t n_steps, const double *f, int32_t n_f, int32_t f_on_host, int32_t *phi_cnt,
+                       void *stream);
+int grf_kmat_phi_fill(const int64_t *offsets_step_major, const int32_t *col, const double *val, int64_t n_rows,
+                      int32_t n_steps, const double *f, int32_t n_f, int32_t f_on_host, const int64_t *phi_ptr,
+                      int32_t *phi_col, double *phi_val, void *stream);
+int grf_kmat_transpose_count(const int64_t *phi_ptr, const int32_t *phi_col, int64_t n_rows, int64_t n_cols,
+                             int32_t *tcnt, void *stream);
+int grf_kmat_transpose_fill(const int64_t *phi_ptr, const int32_t *phi_col, const double *phi_val, int64_t n_rows,
+                            int64_t n_cols, const int64_t *tptr, int64_t *cursor, int32_t *trow, double *tval,
+                            void *stream);
+int grf_kmat_row_sizes(const int64_t *phi_ptr, const int32_t *phi_col, const int64_t *tptr, int64_t n_rows,
+                       int32_t *size, void *stream);
+int grf_kmat_bin(const int32_t *size, int64_t n_rows, int32_t *rows, int64_t *stats, void *stream);
+int64_t grf_kmat_workspace_bytes(int32_t max_size, int32_t global_ctas);
+int grf_kmat_count(const int64_t *phi_ptr, const int32_t *phi_col, const double *phi_val, const int64_t *tptr,
+                   const int32_t *trow, const double *tval, int64_t n_rows, const int32_t *size, const int32_t *rows,
+                   const int64_t *bin_rows, int32_t max_size, int32_t global_ctas, void *workspace,
+                   int64_t workspace_bytes, int32_t *touched, int32_t *stored, int32_t *overflow, void *stream);
+int grf_kmat_fill(const int64_t *phi_ptr, const int32_t *phi_col, const double *phi_val, const int64_t *tptr,
+                  const int32_t *trow, const double *tval, int64_t n_rows, const int32_t *size, const int32_t *rows,
+                  const int64_t *bin_rows, int32_t max_size, int32_t global_ctas, void *workspace,
+                  int64_t workspace_bytes, const int64_t *kptr, int32_t *kcol, double *kval, int32_t *overflow,
+                  void *stream);
+
 /* Replaces the 2L SparseLinearOperator._matmul calls (sparse_lo.py:16-18), the
  * ConstantMul/Sum operators (sparse_grf_kernel.py:59-61) and the row selection
  * (sparse_grf_kernel.py:32-41) of one kernel matvec

@@ -44,6 +44,19 @@ class SparseGraphGP(ExactGP):
             out = K_test_train._matmul(alpha)[:, 0]
         return (out, info) if return_info else out
 
+    def posterior_variance(self, x_test, include_noise=False):
+        """Exact posterior variance k(x*, x*) - k(x*, X) (K(X, X) + sigma^2 I)^-1 k(X, x*) at every test node
+        (float32 device tensor), with sigma^2 added when ``include_noise``.  No sampling: a float64 Cholesky factor
+        on the columns the training rows touch, then one CUDA pass over the test rows (grf_b200/posterior.py)."""
+        from grf_b200.posterior import ExactPosterior
+
+        blocks = self.covar_module.phi_blocks
+        f = self.covar_module.modulator_vector.detach()
+        train_indices = self.x_train.long().flatten()
+        test_indices = torch.as_tensor(x_test).long().flatten()
+        post = ExactPosterior(blocks, f, train_indices, float(self.likelihood.noise.item()))
+        return post.variance(test_indices, include_noise=include_noise)
+
     def predict(self, x_test, n_samples=64, cg_tolerance=None, max_cg_iterations=1000, return_info=False):
         """Posterior samples at ``x_test`` by pathwise conditioning (sparse_grf_model.py:21-45):
         f_test_prior + K_test,train (K_train,train + sigma^2 I)^-1 (y - f_train_prior - eps)."""

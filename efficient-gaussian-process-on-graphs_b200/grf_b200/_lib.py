@@ -33,7 +33,7 @@ EXPORTS = (
     "grf_union_materialize", "grf_pairs_count", "grf_pairs_index", "grf_pairs_fill", "grf_pairs_spmm", "grf_pairs_matvec", "grf_cg_num_partials", "grf_cg_dot", "grf_cg_update", "grf_cg_direction",
     "grf_laplacian_count", "grf_laplacian_fill", "grf_shard_reach", "grf_exchange_flag_bytes", "grf_exchange_sum", "grf_exchange_sum_nvls",
     "grf_kmat_phi_count", "grf_kmat_phi_fill", "grf_kmat_transpose_count", "grf_kmat_transpose_fill", "grf_kmat_row_sizes",
-    "grf_kmat_bin", "grf_kmat_workspace_bytes", "grf_kmat_count", "grf_kmat_fill",
+    "grf_kmat_bin", "grf_kmat_workspace_bytes", "grf_kmat_count", "grf_kmat_fill", "grf_phi_row_quadform",
 )
 
 
@@ -176,6 +176,8 @@ def lib():
     L.grf_phi_fgrad.argtypes = [POINTER(GrfPhi), vp, i64, vp, i64, vp, i64, i32, vp, vp]
     L.grf_phi_row_dots.restype = i32
     L.grf_phi_row_dots.argtypes = [POINTER(GrfPhi), vp, vp, vp, i64, vp, vp]
+    L.grf_phi_row_quadform.restype = i32
+    L.grf_phi_row_quadform.argtypes = [POINTER(GrfPhi), vp, vp, i64, vp, vp, i64, i32, vp, vp, vp]
     L.grf_kmat_phi_count.restype = i32
     L.grf_kmat_phi_count.argtypes = [vp, vp, vp, i64, i32, vp, i32, i32, vp, vp]
     L.grf_kmat_phi_fill.restype = i32

@@ -1094,6 +1094,32 @@ class PhiBlocks:
         check(_lib.lib().grf_phi_row_dots(ctypes.byref(phi), _ptr(f), _ptr(a), _ptr(b), n, _ptr(dots), _stream(dev)))
         return dots
 
+    def row_quadform(self, f, x, col_slot, C):
+        """(q, d), float32 [n] each: q[i] = sum_c (sum_{e in row x[i], col_slot[col e] >= 0} w_e C[col_slot[col e], c])^2
+        and d[i] = sum_e w_e^2, w_e = f[length e] * e.val (``grf_phi_row_quadform``).  C: float32 [m, r] with unit
+        column stride (a column slice of a wider buffer is fine: its row stride is the leading dimension).  x = None:
+        every local row.  See grf_b200/posterior.py for the posterior variance built on it."""
+        dev = self.device
+        f = self._f(f)
+        xi = self._ids(x, dev)
+        n = self.n_rows if xi is None else xi.numel()
+        col_slot = torch.as_tensor(col_slot, device=dev).to(torch.int32).contiguous()
+        if col_slot.numel() != self.n_cols:
+            raise ValueError(f"row_quadform: col_slot has {col_slot.numel()} entries, Phi has {self.n_cols} columns")
+        if C.dim() != 2 or C.dtype != torch.float32 or C.device != dev or (C.shape[1] > 1 and C.stride(1) != 1):
+            raise ValueError("row_quadform: C must be a 2-D float32 tensor on Phi's device with unit column stride")
+        r = int(C.shape[1])
+        ldc = max(r, int(C.stride(0))) if C.shape[0] > 1 else r
+        q = torch.empty(n, dtype=torch.float32, device=dev)
+        d = torch.empty(n, dtype=torch.float32, device=dev)
+        if n == 0:
+            return q, d
+        keep = C if C.numel() else torch.zeros(1, dtype=torch.float32, device=dev)   # no row of C is read then
+        phi = self.c_struct()
+        check(_lib.lib().grf_phi_row_quadform(ctypes.byref(phi), _ptr(f), _ptr(xi), n, _ptr(col_slot), _ptr(keep),
+                                              ldc, r, _ptr(q), _ptr(d), _stream(dev)))
+        return q, d
+
     def _f(self, f) -> torch.Tensor:
         f = torch.as_tensor(f, device=self.device).detach().to(torch.float32).contiguous()
         if f.numel() != self.n_steps:

@@ -451,6 +451,18 @@ int grf_phi_fgrad(const GrfPhi *phi, const int32_t *x, int64_t n, const float *l
 int grf_phi_row_dots(const GrfPhi *phi, const float *f, const int32_t *x1, const int32_t *x2, int64_t n,
                      float *dots, void *stream);
 
+/* Exact GP posterior variance at test rows (csrc/grf_posterior.cu; no reference counterpart: its users estimate
+ * the variance from SparseGraphGP.predict samples).  With w_e = f[length(e)] * e.val:
+ *   q[i] = sum_{c < r} ( sum_{e in row x[i], col_slot[col(e)] >= 0} w_e * C[col_slot[col(e)] * ldc + c] )^2
+ *   d[i] = sum_{e in row x[i]} w_e^2                                   (d may be NULL)
+ * col_slot int32[n_cols]: the row of C that holds column c of Phi_f, or -1; C [m][ldc] float32 (columns
+ * [r, ldc) are never read into a result).  On the merged Phi_f with C = G L^-T of the training rows, d - q is
+ * the posterior variance (grf_b200/posterior.py).  x: global row ids (NULL = every local row, n = n_rows); ids
+ * outside [row_lo, row_lo + n_rows) give q = d = +0.  Only q[0, n) and d[0, n) are written; the summation order
+ * is fixed (no atomics), so repeated calls agree bit for bit. */
+int grf_phi_row_quadform(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n, const int32_t *col_slot,
+                         const float *C, int64_t ldc, int32_t r, float *q, float *d, void *stream);
+
 /* The one exchange of the path (SURVEY.md 8e; no reference counterpart: its matvec runs on one device):
  * U <- sum over the GPUs of the partials U_g = Phi_g[x2]^T V_g between the two halves of a product, as one
  * kernel per rank over NVLink peer memory.  peer_u[g] / peer_flags[g] (HOST arrays of `world` DEVICE pointers)

@@ -59,6 +59,7 @@ struct WalkParams {
     GrfEntry *stage_ent;   // optional: finished Phi entries instead of (stage_col, stage_sum)
     int32_t scale_mode;
     double recip_w, w_as_double;
+    const GrfAliasEdge *alias;  // weighted draws (grf_walk_weighted): the rows' alias tables
 };
 
 // L2 eviction hints (createpolicy + ld.global.L2::cache_hint).  On a graph that does not fit L2 (config 4:
@@ -88,6 +89,23 @@ __device__ __forceinline__ GrfEdge ld_stream_edge(const GrfEdge *ptr, uint64_t p
     GrfEdge e;
     e.scaled = __hiloint2double(raw.y, raw.x);
     e.col = raw.z;
+    e.pad = 0;
+    return e;
+}
+// weighted draws: bucket j of the row's alias table (one 32-byte sector) and the entry the draw takes --
+// its own if frac < thr, else its alias
+__device__ __forceinline__ GrfEdge ld_stream_alias_pick(const GrfAliasEdge *ptr, uint32_t frac, uint64_t pol) {
+    int4 a, b;
+    asm("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.s32 {%0, %1, %2, %3}, [%4], %5;"
+        : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w)
+        : "l"(ptr), "l"(pol));
+    asm("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.s32 {%0, %1, %2, %3}, [%4], %5;"
+        : "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w)
+        : "l"(reinterpret_cast<const char *>(ptr) + 16), "l"(pol));
+    const bool own = frac < (uint32_t)b.z;
+    GrfEdge e;
+    e.scaled = own ? __hiloint2double(a.y, a.x) : __hiloint2double(a.w, a.z);
+    e.col = own ? b.x : b.y;
     e.pad = 0;
     return e;
 }
@@ -144,7 +162,9 @@ __device__ __forceinline__ int group_excl_scan(int v, int *scratch, int &total) 
 // merged and written out before the next step, so shared memory holds ONE length's visit records (W x 12 bytes)
 // instead of all L-1 of them -- the fallback for W x L beyond 227 KB (the reference's wind experiment runs
 // W = 8192, L = 5, its ablation notebook W = 10000, L = 10).  Same draws, same arithmetic, same output.
-template <bool kBlock, typename KeyT, int KPL, bool kFast, bool kWide, bool kStepSync>
+// kWeighted (grf_walk_weighted): the neighbour is drawn from the row's alias table (p.alias) and the load takes
+// that record's factor; a factor of 0.0 (a row of explicit zeros) stops the walk.  Nothing else differs.
+template <bool kBlock, typename KeyT, int KPL, bool kFast, bool kWide, bool kStepSync, bool kWeighted>
 __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINBLOCKS) walk_merge_kernel(const WalkParams p) {
     static_assert(!kStepSync || (kBlock && !kFast && !kWide), "step-synchronous walks: generic CTA variant only");
     constexpr int kIlp = !kWide ? 1 : (kBlock ? 4 : (KPL < 4 ? KPL : 4));
@@ -217,9 +237,11 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
                     }
                 }
                 int64_t e[kIlp];
+                uint32_t frac[kIlp];  // weighted draws: low word of (word * deg), against the bucket's threshold
 #pragma unroll
                 for (int r = 0; r < kIlp; ++r) {
                     e[r] = 0;
+                    frac[r] = 0u;
                     if (!alive[r]) continue;
                     if (deg[r] == 0) {  // dead end: stop without drawing (sparse_sampler.py:47)
                         alive[r] = false;
@@ -228,7 +250,7 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
                     const unsigned long long walk_id =
                         (unsigned long long)start * (unsigned long long)W + (unsigned)(w0 + r * GS);
                     int32_t k;
-                    if (!kFast && p.draw_mode == GRF_DRAW_REPLAY) {
+                    if (!kFast && !kWeighted && p.draw_mode == GRF_DRAW_REPLAY) {
                         const long long ti = ((long long)walk_id - p.trace_base) * L + step;
                         if (__ldg(p.trace_u + ti) < p.p_halt) {
                             alive[r] = false;
@@ -255,6 +277,7 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
                             continue;
                         }
                         k = (int32_t)__umulhi(xk, (uint32_t)deg[r]);
+                        if constexpr (kWeighted) frac[r] = xk * (uint32_t)deg[r];
                     }
                     e[r] = (int64_t)rs[r] + k;
                 }
@@ -268,7 +291,11 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
                     nxt[r] = 0;
                     fac[r] = 0.0;
                     if (!alive[r]) continue;
-                    if (kFast || p.edges) {
+                    if constexpr (kWeighted) {
+                        const GrfEdge ed = ld_stream_alias_pick(p.alias + e[r], frac[r], stream_pol);
+                        nxt[r] = ed.col;
+                        fac[r] = ed.scaled;
+                    } else if (kFast || p.edges) {
                         const GrfEdge ed = ld_stream_edge(p.edges + e[r], stream_pol);
                         nxt[r] = ed.col;
                         fac[r] = ed.scaled;
@@ -285,7 +312,12 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
 #pragma unroll
                 for (int r = 0; r < kIlp; ++r) {
                     if (!alive[r]) continue;
-                    load[r] = (kFast || p.load_mode == GRF_LOAD_CUMULATIVE) ? __dmul_rn(load[r], fac[r]) : fac[r];
+                    if (kWeighted && fac[r] == 0.0) {  // a row of explicit zeros (S = 0): a dead end
+                        alive[r] = false;
+                        continue;
+                    }
+                    load[r] = (kFast || kWeighted || p.load_mode == GRF_LOAD_CUMULATIVE) ? __dmul_rn(load[r], fac[r])
+                                                                                         : fac[r];
                     cur[r] = nxt[r];
                     const int w = w0 + r * GS;
                     nodes[step * W + w] = cur[r];  // the visit at length step + 1
@@ -339,7 +371,8 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
                     }
                     const unsigned long long walk_id = (unsigned long long)start * (unsigned long long)W + (unsigned)w;
                     int32_t k;
-                    if (p.draw_mode == GRF_DRAW_REPLAY) {
+                    uint32_t frac = 0u;
+                    if (!kWeighted && p.draw_mode == GRF_DRAW_REPLAY) {
                         const long long ti = ((long long)walk_id - p.trace_base) * L + si;
                         if (__ldg(p.trace_u + ti) < p.p_halt) {
                             nodes[w] = -1;
@@ -356,8 +389,20 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
                             continue;
                         }
                         k = (int32_t)__umulhi(xk, (uint32_t)deg);
+                        if constexpr (kWeighted) frac = xk * (uint32_t)deg;
                     }
                     const int64_t e = (int64_t)rs + k;
+                    if constexpr (kWeighted) {
+                        const GrfEdge ed = ld_stream_alias_pick(p.alias + e, frac, stream_pol);
+                        if (ed.scaled == 0.0) {  // a row of explicit zeros: a dead end
+                            nodes[w] = -1;
+                            continue;
+                        }
+                        nodes[w] = ed.col;
+                        loads[w] = __dmul_rn(loads[w], ed.scaled);
+                        ++my_visits;
+                        continue;
+                    }
                     const double wv = __ldg(p.val + e);
                     const double fac = p.load_mode == GRF_LOAD_ABLATION
                                            ? wv
@@ -518,9 +563,10 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128, kBlock ? 1 : GRF_WALK_MINB
     }
 }
 
-template <bool kBlock, typename KeyT, int KPL, bool kFast = false, bool kWide = false, bool kStepSync = false>
+template <bool kBlock, typename KeyT, int KPL, bool kFast = false, bool kWide = false, bool kStepSync = false,
+          bool kWeighted = false>
 static int launch_walk(const WalkParams &p, size_t smem, int threads, int grid, cudaStream_t stream) {
-    auto kern = walk_merge_kernel<kBlock, KeyT, KPL, kFast, kWide, kStepSync>;
+    auto kern = walk_merge_kernel<kBlock, KeyT, KPL, kFast, kWide, kStepSync, kWeighted>;
     GRF_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, threads, smem, stream>>>(p);
     return check_cuda(cudaGetLastError(), "walk_merge_kernel launch");
@@ -565,8 +611,11 @@ __device__ __forceinline__ int group_excl_max(int v, int *scratch) {
 //   4. the neighbour draws and edge gathers, which write the walker state of length l + 1.
 // Between 2 and 4 nodes[w] is free (the keys hold the nodes) and carries (cont, head cont-position, j) of
 // walk w; W < 2^15 (shared memory bounds it far below) keeps those in 15-bit fields.
-template <bool kBlock, typename KeyT, int KPL>
-__global__ void __launch_bounds__(kBlock ? 256 : 128) walk_coupled_kernel(const WalkParams p) {
+// kWeighted: antithetic termination with weight-proportional neighbours (p.alias); repelling neighbours are not
+// combined with it.  Its minimum of 4 CTAs per SM only steers ptxas's register target (without it the warp form with
+// 2 keys per lane and 64-bit keys spilled 4 bytes); the existing instantiations keep no minimum.
+template <bool kBlock, typename KeyT, int KPL, bool kWeighted>
+__global__ void __launch_bounds__(kBlock ? 256 : 128, kWeighted ? 4 : 0) walk_coupled_kernel(const WalkParams p) {
     const uint64_t keep = l2_policy_keep(), stream_pol = l2_policy_stream();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int GS = kBlock ? (int)blockDim.x : 32;
@@ -587,7 +636,7 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128) walk_coupled_kernel(const 
     const KeyT KEY_MAX = ~(KeyT)0;
     const KeyT wmask = ((KeyT)1 << wbits) - 1;
     const bool couple_halt = (p.draw_mode & GRF_DRAW_COUPLE_HALT) != 0;
-    const bool repel = (p.draw_mode & GRF_DRAW_COUPLE_NEIGHBOURS) != 0;
+    const bool repel = !kWeighted && (p.draw_mode & GRF_DRAW_COUPLE_NEIGHBOURS) != 0;
     unsigned long long my_visits = 0;
 
     for (int64_t row = (int64_t)blockIdx.x * groups_per_cta + group_in_cta; row < p.n_local;
@@ -751,7 +800,18 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128) walk_coupled_kernel(const 
                                           x);
                         }
                         const uint32_t xk = (l & 1) ? x[3] : x[1];
-                        move(w, rs, deg, (int32_t)__umulhi(xk, (uint32_t)deg));
+                        if constexpr (kWeighted) {  // the bucket of the uniform index, its entry or its alias
+                            const GrfEdge ed = ld_stream_alias_pick(
+                                p.alias + rs + (int32_t)__umulhi(xk, (uint32_t)deg), xk * (uint32_t)deg, stream_pol);
+                            if (ed.scaled == 0.0) {  // a row of explicit zeros: a dead end
+                                cont = false;
+                            } else {
+                                loads[w] = __dmul_rn(loads[w], ed.scaled);
+                                nodes[w] = ed.col;
+                            }
+                        } else {
+                            move(w, rs, deg, (int32_t)__umulhi(xk, (uint32_t)deg));
+                        }
                     }
                 }
                 if (repel)
@@ -815,9 +875,9 @@ __global__ void __launch_bounds__(kBlock ? 256 : 128) walk_coupled_kernel(const 
     }
 }
 
-template <bool kBlock, typename KeyT, int KPL>
+template <bool kBlock, typename KeyT, int KPL, bool kWeighted = false>
 static int launch_coupled(const WalkParams &p, size_t smem, int threads, int grid, cudaStream_t stream) {
-    auto kern = walk_coupled_kernel<kBlock, KeyT, KPL>;
+    auto kern = walk_coupled_kernel<kBlock, KeyT, KPL, kWeighted>;
     GRF_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<grid, threads, smem, stream>>>(p);
     return check_cuda(cudaGetLastError(), "walk_coupled_kernel launch");
@@ -825,7 +885,8 @@ static int launch_coupled(const WalkParams &p, size_t smem, int threads, int gri
 
 // The coupled draws take the step-synchronous schedule: shared memory holds one length's visit records
 // (W x 12 bytes) and the sort keys.  W <= 256: a warp per start node, four per CTA; else a CTA per start node.
-static int walk_coupled(WalkParams &p, bool key32, int64_t n_nodes, cudaStream_t st) {
+template <bool kWeighted>
+static int walk_coupled(WalkParams &p, bool key32, int64_t n_nodes, cudaStream_t st, const char *fn) {
     const size_t key_size = key32 ? 4 : 8;
     const size_t kMaxSmem = 227 * 1024 - 256;
     p.loads_bytes = (uint32_t)(((size_t)p.W * 8 + 15) & ~(size_t)15);
@@ -840,10 +901,10 @@ static int walk_coupled(WalkParams &p, bool key32, int64_t n_nodes, cudaStream_t
         const int grid = (int)(want < (int64_t)kSmCount * 64 ? want : (int64_t)kSmCount * 64);
         const size_t smem = warps * gb;
         const int threads = warps * 32;
-#define GRF_COUPLED_CASE(K)                                                                  \
-    case K:                                                                                  \
-        return key32 ? launch_coupled<false, uint32_t, K>(p, smem, threads, grid, st)       \
-                     : launch_coupled<false, unsigned long long, K>(p, smem, threads, grid, st)
+#define GRF_COUPLED_CASE(K)                                                                             \
+    case K:                                                                                             \
+        return key32 ? launch_coupled<false, uint32_t, K, kWeighted>(p, smem, threads, grid, st)       \
+                     : launch_coupled<false, unsigned long long, K, kWeighted>(p, smem, threads, grid, st)
         switch (kpl) {
             GRF_COUPLED_CASE(1);
             GRF_COUPLED_CASE(2);
@@ -856,57 +917,64 @@ static int walk_coupled(WalkParams &p, bool key32, int64_t n_nodes, cudaStream_t
     const size_t gb = ((size_t)p.loads_bytes + p.nodes_bytes + (size_t)p.Wp * key_size + 15) & ~(size_t)15;
     if (gb > kMaxSmem)
         return fail(GRF_ERR_UNSUPPORTED,
-                    "grf_walk: W=%d needs %zu B of shared memory per start node for one walk length (max %zu; "
-                    "%d-byte sort keys for %lld nodes)", p.W, gb, kMaxSmem, (int)key_size, (long long)n_nodes);
+                    "%s: W=%d needs %zu B of shared memory per start node for one walk length (max %zu; "
+                    "%d-byte sort keys for %lld nodes)", fn, p.W, gb, kMaxSmem, (int)key_size, (long long)n_nodes);
     p.group_bytes = (uint32_t)gb;
     const int grid = (int)(p.n_local < (int64_t)kSmCount * 32 ? p.n_local : (int64_t)kSmCount * 32);
-    return key32 ? launch_coupled<true, uint32_t, 0>(p, gb, 256, grid, st)
-                 : launch_coupled<true, unsigned long long, 0>(p, gb, 256, grid, st);
+    return key32 ? launch_coupled<true, uint32_t, 0, kWeighted>(p, gb, 256, grid, st)
+                 : launch_coupled<true, unsigned long long, 0, kWeighted>(p, gb, 256, grid, st);
 }
 
-}  // namespace grf
-
-extern "C" int64_t grf_walk_stage_stride(int32_t walks_per_node, int32_t max_walk_length) {
-    if (walks_per_node < 1 || max_walk_length < 1) return 0;
-    return 1 + (int64_t)(max_walk_length - 1) * (int64_t)walks_per_node;
+// the warp-per-node forms of one key type and sort width: fast (+ wide) or generic; weighted draws always take
+// the fast forms (Philox draws, cumulative load, one record gather per step)
+template <bool kWeighted, typename KeyT, int K>
+static int launch_warp_forms(const WalkParams &p, bool fast, bool wide, size_t smem, int threads, int grid,
+                             cudaStream_t st) {
+    if (fast && wide) return launch_walk<false, KeyT, K, true, true, false, kWeighted>(p, smem, threads, grid, st);
+    if (fast) return launch_walk<false, KeyT, K, true, false, false, kWeighted>(p, smem, threads, grid, st);
+    if constexpr (kWeighted)
+        return fail(GRF_ERR_INVALID, "grf_walk_weighted: no generic form");
+    else
+        return launch_walk<false, KeyT, K>(p, smem, threads, grid, st);
 }
 
-extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t stage_stride, int32_t *stage_col,
-                        double *stage_sum, int32_t *row_cnt, unsigned long long *visits_out, void *stream) {
-    GRF_ON_STREAM_DEVICE(stream, row_cnt);
-    using namespace grf;
-    GRF_REQUIRE(graph && cfg, "grf_walk: null graph/cfg");
-    GRF_REQUIRE(graph->n_nodes >= 0 && graph->n_nodes < (1ll << 31), "grf_walk: n_nodes %lld out of int32 range",
+// Validation and WalkParams of grf_walk and grf_walk_weighted.  *launch = false: nothing to do (no start node).
+static int walk_prepare(const char *fn, const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t stage_stride, int32_t *stage_col,
+                        double *stage_sum, int32_t *row_cnt, unsigned long long *visits_out, WalkParams &p,
+                        bool &launch) {
+    launch = false;
+    GRF_REQUIRE(graph && cfg, "%s: null graph/cfg", fn);
+    GRF_REQUIRE(graph->n_nodes >= 0 && graph->n_nodes < (1ll << 31), "%s: n_nodes %lld out of int32 range", fn,
                 (long long)graph->n_nodes);
-    GRF_REQUIRE(graph->nnz >= 0 && graph->nnz < (1ll << 31), "grf_walk: nnz %lld out of int32 range",
+    GRF_REQUIRE(graph->nnz >= 0 && graph->nnz < (1ll << 31), "%s: nnz %lld out of int32 range", fn,
                 (long long)graph->nnz);
-    GRF_REQUIRE(cfg->walks_per_node >= 1, "grf_walk: walks_per_node must be >= 1");
-    GRF_REQUIRE(cfg->max_walk_length >= 1, "grf_walk: max_walk_length must be >= 1");
-    GRF_REQUIRE(cfg->p_halt >= 0.0 && cfg->p_halt <= 1.0, "grf_walk: p_halt must be in [0, 1]");
+    GRF_REQUIRE(cfg->walks_per_node >= 1, "%s: walks_per_node must be >= 1", fn);
+    GRF_REQUIRE(cfg->max_walk_length >= 1, "%s: max_walk_length must be >= 1", fn);
+    GRF_REQUIRE(cfg->p_halt >= 0.0 && cfg->p_halt <= 1.0, "%s: p_halt must be in [0, 1]", fn);
     GRF_REQUIRE(cfg->start_lo >= 0 && cfg->start_lo <= cfg->start_hi && cfg->start_hi <= graph->n_nodes,
-                "grf_walk: start range [%lld, %lld) outside [0, %lld)", (long long)cfg->start_lo,
+                "%s: start range [%lld, %lld) outside [0, %lld)", fn, (long long)cfg->start_lo,
                 (long long)cfg->start_hi, (long long)graph->n_nodes);
     const int32_t coupled = GRF_DRAW_COUPLE_HALT | GRF_DRAW_COUPLE_NEIGHBOURS;
-    GRF_REQUIRE((cfg->draw_mode & ~(GRF_DRAW_REPLAY | coupled)) == 0, "grf_walk: bad draw_mode");
+    GRF_REQUIRE((cfg->draw_mode & ~(GRF_DRAW_REPLAY | coupled)) == 0, "%s: bad draw_mode", fn);
     GRF_REQUIRE(!(cfg->draw_mode & GRF_DRAW_REPLAY) || !(cfg->draw_mode & coupled),
-                "grf_walk: coupled draws need native Philox draws");
+                "%s: coupled draws need native Philox draws", fn);
     GRF_REQUIRE(cfg->load_mode >= GRF_LOAD_CUMULATIVE && cfg->load_mode <= GRF_LOAD_ABLATION,
-                "grf_walk: bad load_mode");
+                "%s: bad load_mode", fn);
     GRF_REQUIRE(cfg->draw_mode != GRF_DRAW_REPLAY || (cfg->trace_u && cfg->trace_k),
-                "grf_walk: replay mode needs trace_u and trace_k");
+                "%s: replay mode needs trace_u and trace_k", fn);
     GRF_REQUIRE(stage_stride >= grf_walk_stage_stride(cfg->walks_per_node, cfg->max_walk_length),
-                "grf_walk: stage_stride too small");
+                "%s: stage_stride too small", fn);
     const int64_t n_local = cfg->start_hi - cfg->start_lo;
     if (n_local == 0) return GRF_OK;
-    GRF_REQUIRE(graph->row_ptr && row_cnt && (cfg->stage_entries || (stage_col && stage_sum)), "grf_walk: null buffer");
-    GRF_REQUIRE(cfg->scale_mode == GRF_SCALE_MUL_RECIP || cfg->scale_mode == GRF_SCALE_DIV, "grf_walk: bad scale_mode");
-    GRF_REQUIRE(graph->nnz == 0 || (graph->col_idx && graph->val), "grf_walk: null edge arrays");
+    GRF_REQUIRE(graph->row_ptr && row_cnt && (cfg->stage_entries || (stage_col && stage_sum)), "%s: null buffer", fn);
+    GRF_REQUIRE(cfg->scale_mode == GRF_SCALE_MUL_RECIP || cfg->scale_mode == GRF_SCALE_DIV, "%s: bad scale_mode", fn);
+    GRF_REQUIRE(graph->nnz == 0 || (graph->col_idx && graph->val), "%s: null edge arrays", fn);
 
-    WalkParams p;
     p.row_ptr = graph->row_ptr;
     p.col_idx = graph->col_idx;
     p.val = graph->val;
     p.edges = cfg->edges;
+    p.alias = nullptr;
     p.trace_base = cfg->trace_walk_base;
     p.stage_ent = cfg->stage_entries;
     p.scale_mode = cfg->scale_mode;
@@ -935,7 +1003,17 @@ extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t st
     p.row_cnt = row_cnt;
     p.visits = visits_out;
     p.col_counts = cfg->col_counts;
+    GRF_REQUIRE((uint64_t)p.W * (uint64_t)p.L < (1ull << 31), "%s: W*L too large", fn);
+    launch = true;
+    return GRF_OK;
+}
 
+// Every launch shape of the walker: coupled draws -> walk_coupled; W <= 256 and the visit records of all lengths
+// fit -> warp per start node (4, 2 or 1 per CTA); else a CTA per start node, all lengths or one at a time.
+template <bool kWeighted>
+static int walk_launch(WalkParams &p, const GrfGraph *graph, cudaStream_t st, const char *fn) {
+    const int64_t n_local = p.n_local;
+    const int32_t coupled = GRF_DRAW_COUPLE_HALT | GRF_DRAW_COUPLE_NEIGHBOURS;
     const int node_bits = bit_width((uint64_t)(graph->n_nodes > 0 ? graph->n_nodes - 1 : 0));
     const bool key32 = node_bits + p.wbits <= 31;
     const size_t key_size = key32 ? 4 : 8;
@@ -951,10 +1029,8 @@ extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t st
     const size_t gb = ((size_t)p.loads_bytes + p.nodes_bytes + p.sorted_bytes + key_area + 15) & ~(size_t)15;
     p.group_bytes = (uint32_t)gb;
     const size_t kMaxSmem = 227 * 1024 - 256;
-    GRF_REQUIRE((uint64_t)p.W * (uint64_t)p.L < (1ull << 31), "grf_walk: W*L too large");
 
-    cudaStream_t st = (cudaStream_t)stream;
-    if (cfg->draw_mode & coupled) return walk_coupled(p, key32, graph->n_nodes, st);
+    if (p.draw_mode & coupled) return walk_coupled<kWeighted>(p, key32, graph->n_nodes, st, fn);
     // start nodes per CTA of the warp-per-node variant: as many of 4, 2, 1 as the visit records leave room for
     // (W = 200, L = 30: one group is 68 KB); none fits -> the CTA-per-node variants below
     int warps = 4;
@@ -964,20 +1040,16 @@ extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t st
         const int grid = (int)(want < (int64_t)kSmCount * 64 ? want : (int64_t)kSmCount * 64);
         const size_t smem = warps * gb;
         const int threads = warps * 32;
-        const bool fast = p.draw_mode == GRF_DRAW_PHILOX && p.load_mode == GRF_LOAD_CUMULATIVE && p.edges;
+        const bool fast =
+            kWeighted || (p.draw_mode == GRF_DRAW_PHILOX && p.load_mode == GRF_LOAD_CUMULATIVE && p.edges);
         // the edge records of this graph do not fit L2 (126 MB, shared with staging writes): latency-bound regime
         const char *ilp_env = getenv("GRF_B200_WALK_WIDE");
-        const bool wide = ilp_env ? ilp_env[0] == '1' : graph->nnz * (int64_t)sizeof(GrfEdge) > (48ll << 20);
-#define GRF_WALK_CASE(K)                                                                                    \
-    case K:                                                                                                 \
-        if (fast && wide)                                                                                   \
-            return key32 ? launch_walk<false, uint32_t, K, true, true>(p, smem, threads, grid, st)         \
-                         : launch_walk<false, unsigned long long, K, true, true>(p, smem, threads, grid, st); \
-        if (fast)                                                                                           \
-            return key32 ? launch_walk<false, uint32_t, K, true>(p, smem, threads, grid, st)               \
-                         : launch_walk<false, unsigned long long, K, true>(p, smem, threads, grid, st);     \
-        return key32 ? launch_walk<false, uint32_t, K>(p, smem, threads, grid, st)                         \
-                     : launch_walk<false, unsigned long long, K>(p, smem, threads, grid, st)
+        const int64_t rec_bytes = kWeighted ? (int64_t)sizeof(GrfAliasEdge) : (int64_t)sizeof(GrfEdge);
+        const bool wide = ilp_env ? ilp_env[0] == '1' : graph->nnz * rec_bytes > (48ll << 20);
+#define GRF_WALK_CASE(K)                                                                                 \
+    case K:                                                                                              \
+        return key32 ? launch_warp_forms<kWeighted, uint32_t, K>(p, fast, wide, smem, threads, grid, st) \
+                     : launch_warp_forms<kWeighted, unsigned long long, K>(p, fast, wide, smem, threads, grid, st)
         switch (kpl) {
             GRF_WALK_CASE(1);
             GRF_WALK_CASE(2);
@@ -995,8 +1067,8 @@ extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t st
     if (gb_cta <= kMaxSmem) {
         p.sorted_bytes = 0;
         p.group_bytes = (uint32_t)gb_cta;
-        return key32 ? launch_walk<true, uint32_t, 0, false, true>(p, gb_cta, 256, grid, st)
-                     : launch_walk<true, unsigned long long, 0, false, true>(p, gb_cta, 256, grid, st);
+        return key32 ? launch_walk<true, uint32_t, 0, false, true, false, kWeighted>(p, gb_cta, 256, grid, st)
+                     : launch_walk<true, unsigned long long, 0, false, true, false, kWeighted>(p, gb_cta, 256, grid, st);
     }
     // all lengths do not fit: one length at a time (W x 12 bytes of records + the sort keys)
     p.loads_bytes = (uint32_t)(((size_t)p.W * 8 + 15) & ~(size_t)15);
@@ -1005,12 +1077,53 @@ extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t st
     const size_t gb_ss = ((size_t)p.loads_bytes + p.nodes_bytes + cta_keys + 15) & ~(size_t)15;
     if (gb_ss > kMaxSmem)
         return fail(GRF_ERR_UNSUPPORTED,
-                    "grf_walk: W=%d needs %zu B of shared memory per start node for one walk length (max %zu; "
-                    "%d-byte sort keys for %lld nodes)", p.W, gb_ss, kMaxSmem, (int)key_size,
+                    "%s: W=%d needs %zu B of shared memory per start node for one walk length (max %zu; "
+                    "%d-byte sort keys for %lld nodes)", fn, p.W, gb_ss, kMaxSmem, (int)key_size,
                     (long long)graph->n_nodes);
     p.group_bytes = (uint32_t)gb_ss;
-    return key32 ? launch_walk<true, uint32_t, 0, false, false, true>(p, gb_ss, 256, grid, st)
-                 : launch_walk<true, unsigned long long, 0, false, false, true>(p, gb_ss, 256, grid, st);
+    return key32 ? launch_walk<true, uint32_t, 0, false, false, true, kWeighted>(p, gb_ss, 256, grid, st)
+                 : launch_walk<true, unsigned long long, 0, false, false, true, kWeighted>(p, gb_ss, 256, grid, st);
+}
+
+}  // namespace grf
+
+extern "C" int64_t grf_walk_stage_stride(int32_t walks_per_node, int32_t max_walk_length) {
+    if (walks_per_node < 1 || max_walk_length < 1) return 0;
+    return 1 + (int64_t)(max_walk_length - 1) * (int64_t)walks_per_node;
+}
+
+extern "C" int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t stage_stride, int32_t *stage_col,
+                        double *stage_sum, int32_t *row_cnt, unsigned long long *visits_out, void *stream) {
+    GRF_ON_STREAM_DEVICE(stream, row_cnt);
+    using namespace grf;
+    WalkParams p;
+    bool launch;
+    const int rc =
+        walk_prepare("grf_walk", graph, cfg, stage_stride, stage_col, stage_sum, row_cnt, visits_out, p, launch);
+    if (rc != GRF_OK || !launch) return rc;
+    return walk_launch<false>(p, graph, (cudaStream_t)stream, "grf_walk");
+}
+
+extern "C" int grf_walk_weighted(const GrfGraph *graph, const GrfWalkCfg *cfg, const GrfAliasEdge *alias,
+                                 int64_t stage_stride, int32_t *stage_col, double *stage_sum, int32_t *row_cnt,
+                                 unsigned long long *visits_out, void *stream) {
+    GRF_ON_STREAM_DEVICE(stream, row_cnt);
+    using namespace grf;
+    GRF_REQUIRE(cfg, "grf_walk_weighted: null cfg");
+    GRF_REQUIRE(cfg->draw_mode == GRF_DRAW_PHILOX || cfg->draw_mode == (GRF_DRAW_PHILOX | GRF_DRAW_COUPLE_HALT),
+                "grf_walk_weighted: draw_mode must be GRF_DRAW_PHILOX, optionally | GRF_DRAW_COUPLE_HALT "
+                "(no replay, no repelling neighbours)");
+    GRF_REQUIRE(cfg->load_mode == GRF_LOAD_CUMULATIVE, "grf_walk_weighted: load_mode must be GRF_LOAD_CUMULATIVE");
+    GRF_REQUIRE(cfg->edges == nullptr, "grf_walk_weighted: cfg->edges must be NULL (the alias records replace them)");
+    WalkParams p;
+    bool launch;
+    const int rc = walk_prepare("grf_walk_weighted", graph, cfg, stage_stride, stage_col, stage_sum, row_cnt,
+                                visits_out, p, launch);
+    if (rc != GRF_OK || !launch) return rc;
+    const bool steps = p.L > 1 && p.halt_thr < (1ull << 32) && graph->nnz > 0;
+    GRF_REQUIRE(alias || !steps, "grf_walk_weighted: null alias records");
+    p.alias = alias;
+    return walk_launch<true>(p, graph, (cudaStream_t)stream, "grf_walk_weighted");
 }
 
 namespace grf {

@@ -40,9 +40,12 @@ def fast_general_grf_kernel(
     *,
     trace=None,
     coupling: str = "iid",
+    neighbour_sampling: str = "uniform",
 ) -> np.ndarray:
     """GRF kernel estimate K ~ Phi Phi^T using importance-sampled random walks.  ``coupling``: how the walks
-    of one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" = independent, as the reference)."""
+    of one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" = independent, as the reference).
+    ``neighbour_sampling``: "uniform" (as the reference) or "weighted" (neighbour k with probability |w_k| / sum |w|:
+    bounded importance weights on the normalized Laplacian)."""
     modulator_vector = np.asarray(modulator_vector, dtype=float)
     if modulator_vector.shape[0] != max_walk_length:
         # the reference fails inside ``feature_matrices @ modulator`` with a shape error (:38)
@@ -50,6 +53,6 @@ def fast_general_grf_kernel(
     laplacian = get_normalized_laplacian(adj_matrix)
     random_walk = RandomWalk(Graph(laplacian), seed=42)
     steps = random_walk.get_step_matrices_device(walks_per_node, p_halt, max_walk_length, trace=trace,
-                                                   coupling=coupling)
+                                                   coupling=coupling, neighbour_sampling=neighbour_sampling)
     phi = _phi_from_steps(steps, modulator_vector)
     return (phi @ phi.T).cpu().numpy()

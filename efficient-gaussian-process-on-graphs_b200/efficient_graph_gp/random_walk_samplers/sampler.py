@@ -61,7 +61,8 @@ class RandomWalk:
         self._device = device
 
     def get_step_matrices_device(self, num_walks, p_halt, max_walk_length, ablation=False,
-                                 sequential_semantics=False, trace=None, *, coupling="iid"):
+                                 sequential_semantics=False, trace=None, *, coupling="iid",
+                                 neighbour_sampling="uniform"):
         csr = self.graph.to_csr()
         dg = DeviceGraph(csr.indptr, csr.indices, csr.data, self.graph.get_num_nodes(), self._device)
         if ablation:
@@ -72,7 +73,8 @@ class RandomWalk:
             load_mode = _lib.LOAD_CUMULATIVE
         cfg = WalkConfig(int(num_walks), float(p_halt), int(max_walk_length), seed=self.seed,
                          draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY,
-                         load_mode=load_mode, trace=trace, coupling=coupling)
+                         load_mode=load_mode, trace=trace, coupling=coupling,
+                         neighbour_sampling=neighbour_sampling)
         return build_step_matrices(dg, cfg, scale_mode=_lib.SCALE_DIV)  # value / num_walks, sampler.py:201
 
     def get_random_walk_matrices(
@@ -87,10 +89,14 @@ class RandomWalk:
         sequential_semantics: bool = False,
         trace=None,
         coupling: str = "iid",
+        neighbour_sampling: str = "uniform",
     ) -> np.ndarray:
         """(num_nodes, num_nodes, max_walk_length) float64; [i, j, l] estimates (A^l)[i, j].  ``coupling``:
-        how the walks of one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" = independent)."""
+        how the walks of one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" = independent).
+        ``neighbour_sampling``: "uniform" (the reference's rule) or "weighted" (neighbour k with probability
+        |w_k| / sum |w|; ``grf_b200.engine.NEIGHBOUR_SAMPLINGS``)."""
         del use_tqdm, n_processes
         steps = self.get_step_matrices_device(num_walks, p_halt, max_walk_length, ablation,
-                                              sequential_semantics, trace, coupling=coupling)
+                                              sequential_semantics, trace, coupling=coupling,
+                                              neighbour_sampling=neighbour_sampling)
         return steps.to_dense_tensor()

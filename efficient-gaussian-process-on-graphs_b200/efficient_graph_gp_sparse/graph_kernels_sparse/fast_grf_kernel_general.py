@@ -24,13 +24,15 @@ def fast_general_grf_kernel(
     *,
     trace=None,
     coupling: str = "iid",
+    neighbour_sampling: str = "uniform",
 ):
     """Sparse GRF kernel estimate K ~ Phi Phi^T on the normalized Laplacian, as a scipy csr_matrix.
     ``modulator_vector``: f_p for p < min(len, max_walk_length), real scalars that widen to float64.
     ``coupling``: how the walks of one start node share their draws (``grf_b200.engine.COUPLINGS``; "iid" =
-    independent, as the reference).  Raises MemoryError, naming nnz(K), when K does not fit on the device."""
+    independent, as the reference).  ``neighbour_sampling``: "uniform" (as the reference) or "weighted" (neighbour k
+    with probability |w_k| / sum |w|: bounded importance weights on the normalized Laplacian).  Raises MemoryError, naming nnz(K), when K does not fit on the device."""
     # the Laplacian (graph_utils.py:5-30) is formed on the device, bit-identical to the host one
     random_walk = SparseRandomWalk.on_normalized_laplacian(adj_matrix, seed=None)
     step_matrices = random_walk.get_step_matrices_device(walks_per_node, p_halt, max_walk_length, trace=trace,
-                                                          coupling=coupling)
+                                                          coupling=coupling, neighbour_sampling=neighbour_sampling)
     return step_matrices.kernel_matrix(modulator_vector).to_scipy()

@@ -50,7 +50,8 @@ class GraphPreprocessor:
                  n_processes: int = None,
                  device=None,
                  *,
-                 coupling: str = "iid") -> None:
+                 coupling: str = "iid",
+                 neighbour_sampling: str = "uniform") -> None:
         if adjacency_matrix.shape[0] != adjacency_matrix.shape[1]:
             raise ValueError("Adjacency matrix must be square.")
 
@@ -64,6 +65,7 @@ class GraphPreprocessor:
         self.n_processes = n_processes
         self.device = device
         self.coupling = coupling   # grf_b200.engine.COUPLINGS: how the walks of one start node share their draws
+        self.neighbour_sampling = neighbour_sampling   # grf_b200.engine.NEIGHBOUR_SAMPLINGS: how a walk moves on
         self._scipy = None
         self._steps_device = None
 
@@ -89,7 +91,8 @@ class GraphPreprocessor:
 
     def _generate_cache_filename(self) -> str:
         """Same key as the reference (graph_preprocessor.py:75-83), so caches are interchangeable; coupled
-        draws append the coupling, so that a coupled cache never answers an independent-draws request."""
+        draws append the coupling and weighted neighbour draws append "_weighted", so that such a cache never answers a
+        request for the reference's draws."""
         adj_hash = hashlib.md5(self.adj_matrix.data.tobytes() +
                                self.adj_matrix.indices.tobytes() +
                                self.adj_matrix.indptr.tobytes()).hexdigest()[:8]
@@ -97,6 +100,8 @@ class GraphPreprocessor:
         params = f"{graph_size}_{self.walks_per_node}_{self.p_halt}_{self.max_walk_length}_{self.random_walk_seed}"
         if self.coupling != "iid":
             params += f"_{self.coupling}"
+        if self.neighbour_sampling != "uniform":
+            params += f"_{self.neighbour_sampling}"
         return f"experiments_sparse/step_matrices/step_matrices_{adj_hash}_{params}.pkl"
 
     def _target_device(self) -> torch.device:
@@ -141,7 +146,7 @@ class GraphPreprocessor:
         cfg = WalkConfig(int(self.walks_per_node), float(self.p_halt), int(self.max_walk_length),
                          seed=self.random_walk_seed or 42,
                          draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace,
-                         coupling=self.coupling)
+                         coupling=self.coupling, neighbour_sampling=self.neighbour_sampling)
         self._steps_device = build_step_matrices(graph, cfg, scale_mode=_lib.SCALE_MUL_RECIP)
         self._scipy = None
         if save_to_disk:
@@ -164,7 +169,7 @@ class GraphPreprocessor:
         cfg = WalkConfig(int(self.walks_per_node), float(self.p_halt), int(self.max_walk_length),
                          seed=self.random_walk_seed or 42,
                          draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace,
-                         coupling=self.coupling)
+                         coupling=self.coupling, neighbour_sampling=self.neighbour_sampling)
         return build_phi_blocks(graph, cfg, start_lo, start_hi)
 
     @staticmethod

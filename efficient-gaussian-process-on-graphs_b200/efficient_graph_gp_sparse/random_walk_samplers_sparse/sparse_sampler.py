@@ -17,7 +17,12 @@ columns, ``M_0 = I``).  Differences, all deliberate (DESIGN.md):
 * ``coupling=`` (keyword only, default ``"iid"``: the independent draws above)
   couples the walks of one start node for a lower-variance estimate:
   ``"antithetic"``, ``"repelling"`` or ``"antithetic+repelling"``
-  (``grf_b200.engine.COUPLINGS``; native draws only).
+  (``grf_b200.engine.COUPLINGS``; native draws only);
+* ``neighbour_sampling=`` (keyword only, default ``"uniform"``: the reference's
+  rule) with ``"weighted"`` picks neighbour k with probability |w_k| / sum |w|
+  and multiplies the load by sign(w_k) * sum |w| / (1 - p_halt): still
+  unbiased, and far less variance on graphs with hubs (native draws only, not
+  with repelling neighbours).
 """
 
 from typing import List, Optional
@@ -61,23 +66,25 @@ class SparseRandomWalk:
             self._graph = DeviceGraph(self.indptr, self.indices, self.data, self.num_nodes, self._device)
         return self._graph
 
-    def _config(self, num_walks, p_halt, max_walk_length, trace, trace_start=0, coupling="iid") -> WalkConfig:
+    def _config(self, num_walks, p_halt, max_walk_length, trace, trace_start=0, coupling="iid",
+                neighbour_sampling="uniform") -> WalkConfig:
         return WalkConfig(
             walks_per_node=int(num_walks), p_halt=float(p_halt), max_walk_length=int(max_walk_length),
             seed=self.seed, draw_mode=_lib.DRAW_PHILOX if trace is None else _lib.DRAW_REPLAY, trace=trace,
-            trace_start=int(trace_start), coupling=coupling)
+            trace_start=int(trace_start), coupling=coupling, neighbour_sampling=neighbour_sampling)
 
     def get_step_matrices_device(self, num_walks, p_halt, max_walk_length, start_lo=0, start_hi=None,
-                                 trace=None, trace_start=0, *, coupling="iid") -> StepMatrices:
+                                 trace=None, trace_start=0, *, coupling="iid",
+                                 neighbour_sampling="uniform") -> StepMatrices:
         """The step matrices left in HBM (rows [start_lo, start_hi) only).  ``trace_start``: the first start
         node the replayed trace covers (a trace recorded for a row slice is indexed from there)."""
-        cfg = self._config(num_walks, p_halt, max_walk_length, trace, trace_start, coupling)
+        cfg = self._config(num_walks, p_halt, max_walk_length, trace, trace_start, coupling, neighbour_sampling)
         return build_step_matrices(self.graph, cfg, start_lo, start_hi, scale_mode=_lib.SCALE_MUL_RECIP)
 
     def get_phi_blocks(self, num_walks, p_halt, max_walk_length, start_lo=0, start_hi=None, trace=None,
-                       trace_start=0, *, coupling="iid") -> PhiBlocks:
+                       trace_start=0, *, coupling="iid", neighbour_sampling="uniform") -> PhiBlocks:
         """Phi in the matvec layout, built without leaving the device."""
-        cfg = self._config(num_walks, p_halt, max_walk_length, trace, trace_start, coupling)
+        cfg = self._config(num_walks, p_halt, max_walk_length, trace, trace_start, coupling, neighbour_sampling)
         return build_phi_blocks(self.graph, cfg, start_lo, start_hi)
 
     def get_random_walk_matrices(
@@ -90,7 +97,8 @@ class SparseRandomWalk:
         *,
         trace=None,
         coupling: str = "iid",
+        neighbour_sampling: str = "uniform",
     ) -> List[sp.csr_matrix]:
         del use_tqdm, n_processes
         return self.get_step_matrices_device(num_walks, p_halt, max_walk_length, trace=trace,
-                                             coupling=coupling).to_scipy()
+                                             coupling=coupling, neighbour_sampling=neighbour_sampling).to_scipy()

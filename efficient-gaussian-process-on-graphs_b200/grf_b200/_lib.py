@@ -34,6 +34,7 @@ EXPORTS = (
     "grf_laplacian_count", "grf_laplacian_fill", "grf_shard_reach", "grf_exchange_flag_bytes", "grf_exchange_sum", "grf_exchange_sum_nvls",
     "grf_kmat_phi_count", "grf_kmat_phi_fill", "grf_kmat_transpose_count", "grf_kmat_transpose_fill", "grf_kmat_row_sizes",
     "grf_kmat_bin", "grf_kmat_workspace_bytes", "grf_kmat_count", "grf_kmat_fill", "grf_phi_row_quadform",
+    "grf_alias_records", "grf_walk_weighted",
 )
 
 
@@ -162,6 +163,10 @@ def lib():
     L.grf_laplacian_fill.argtypes = [POINTER(GrfGraph), vp, vp, vp, vp, vp, vp]
     L.grf_edge_records.restype = i32
     L.grf_edge_records.argtypes = [POINTER(GrfGraph), c_double, vp, vp]
+    L.grf_alias_records.restype = i32
+    L.grf_alias_records.argtypes = [POINTER(GrfGraph), c_double, vp, vp]
+    L.grf_walk_weighted.restype = i32
+    L.grf_walk_weighted.argtypes = [POINTER(GrfGraph), POINTER(GrfWalkCfg), vp, i64, vp, vp, vp, vp, vp]
     L.grf_compact_entries.restype = i32
     L.grf_compact_entries.argtypes = [vp, vp, i64, i32, i64, vp, vp]
     L.grf_exchange_flag_bytes.restype = i64

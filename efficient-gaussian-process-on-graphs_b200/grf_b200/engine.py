@@ -110,6 +110,12 @@ COUPLINGS = {
     "antithetic+repelling": _lib.DRAW_COUPLE_HALT | _lib.DRAW_COUPLE_NEIGHBOURS,
 }
 
+# WalkConfig.neighbour_sampling: "uniform" picks a neighbour uniformly and multiplies the load by
+# deg * w / (1 - p) (the reference's rule); "weighted" picks neighbour k with probability |w_k| / S, S = sum |w|
+# over the row, and multiplies by sign(w_k) * S / (1 - p) -- unbiased, with a per-step factor bounded by
+# S / (1 - p) (definitions at GrfAliasEdge in include/grf_b200.h).
+NEIGHBOUR_SAMPLINGS = ("uniform", "weighted")
+
 
 @dataclass
 class WalkConfig:
@@ -124,6 +130,7 @@ class WalkConfig:
     trace: Optional[Tuple] = None  # (trace_u float64, trace_k int32), [(walk_id - trace_start*W)*L + step]
     trace_start: int = 0           # first start node the trace covers (a trace recorded for a row slice)
     coupling: str = "iid"          # one of COUPLINGS: how the W walks of a start node share their draws
+    neighbour_sampling: str = "uniform"   # one of NEIGHBOUR_SAMPLINGS: how a walk picks its next node
 
     def validate(self):
         if int(self.walks_per_node) < 1:
@@ -138,6 +145,16 @@ class WalkConfig:
             raise ValueError(f"coupling must be one of {sorted(COUPLINGS)}, not {self.coupling!r}")
         if COUPLINGS[self.coupling] and (self.draw_mode != _lib.DRAW_PHILOX or self.trace is not None):
             raise ValueError("coupled draws need native Philox draws (no replayed trace)")
+        if self.neighbour_sampling not in NEIGHBOUR_SAMPLINGS:
+            raise ValueError(f"neighbour_sampling must be one of {NEIGHBOUR_SAMPLINGS}, "
+                             f"not {self.neighbour_sampling!r}")
+        if self.neighbour_sampling == "weighted":
+            if self.draw_mode != _lib.DRAW_PHILOX or self.trace is not None:
+                raise ValueError("weighted neighbour sampling needs native Philox draws (no replayed trace)")
+            if COUPLINGS[self.coupling] & _lib.DRAW_COUPLE_NEIGHBOURS:
+                raise ValueError("weighted neighbour sampling does not combine with repelling neighbours")
+            if self.load_mode != _lib.LOAD_CUMULATIVE:
+                raise ValueError("weighted neighbour sampling needs the cumulative load rule")
 
     def draw_flags(self) -> int:
         """draw_mode of GrfWalkCfg: the draw source with the coupling bits OR-ed in."""
@@ -343,7 +360,24 @@ class DeviceGraph:
             out = torch.empty((max(1, self.nnz), 2), dtype=torch.float64, device=self.device)
             g = self.c_struct()
             check(_lib.lib().grf_edge_records(ctypes.byref(g), key, _ptr(out), _stream(self.device)))
-            self._scaled = {key: out}
+            # one p_halt at a time per kind of record: drop other edge records, keep the alias tables
+            self._scaled = {k: v for k, v in self._scaled.items() if isinstance(k, tuple)}
+            self._scaled[key] = out
+        return self._scaled[key]
+
+    def alias_records(self, p_halt: float) -> torch.Tensor:
+        """Alias-table buckets of every row for weight-proportional neighbour draws, 32 bytes each (cached per
+        p_halt, like ``edge_records``).  Non-finite weights raise ValueError."""
+        key = ("alias", float(p_halt))
+        if key not in self._scaled:
+            if self.nnz and not bool(torch.isfinite(self.val).all()):
+                raise ValueError("weighted neighbour sampling needs finite weights")
+            out = torch.empty((max(1, self.nnz), 4), dtype=torch.float64, device=self.device)
+            g = self.c_struct()
+            check(_lib.lib().grf_alias_records(ctypes.byref(g), key[1], _ptr(out), _stream(self.device)))
+            # one p_halt at a time per kind of record: drop other alias tables, keep the edge records
+            self._scaled = {k: v for k, v in self._scaled.items() if not isinstance(k, tuple)}
+            self._scaled[key] = out
         return self._scaled[key]
 
 
@@ -411,8 +445,11 @@ def run_walker(graph: DeviceGraph, cfg: WalkConfig, start_lo: int = 0, start_hi:
             raise ValueError("trace arrays must cover the walks of start nodes trace_start .. start_hi - 1 "
                              "((start_hi - trace_start) * W * L entries)")
     g = graph.c_struct()
-    edges = None
-    if cfg.load_mode != _lib.LOAD_ABLATION and cfg.max_walk_length > 1 and graph.nnz > 0 and cfg.p_halt < 1.0:
+    edges = alias = None
+    steps = cfg.max_walk_length > 1 and graph.nnz > 0 and cfg.p_halt < 1.0
+    if cfg.neighbour_sampling == "weighted":
+        alias = graph.alias_records(cfg.p_halt) if steps and n_rows > 0 else None
+    elif cfg.load_mode != _lib.LOAD_ABLATION and steps:
         edges = graph.edge_records(cfg.p_halt)
     c = GrfWalkCfg(start_lo, start_hi, cfg.walks_per_node, cfg.max_walk_length, float(cfg.p_halt), cfg.draw_flags(),
                    cfg.load_mode, int(cfg.seed) & 0xFFFFFFFFFFFFFFFF,
@@ -421,8 +458,12 @@ def run_walker(graph: DeviceGraph, cfg: WalkConfig, start_lo: int = 0, start_hi:
                    None if col_counts is None else col_counts.data_ptr(), trace_base,
                    None if stage_ent is None else stage_ent.data_ptr(),
                    _lib.SCALE_MUL_RECIP if entries_scale_mode is None else int(entries_scale_mode))
-    check(L.grf_walk(ctypes.byref(g), ctypes.byref(c), stride, _ptr(stage_col), _ptr(stage_sum), _ptr(row_cnt),
-                     _ptr(visits), _stream(dev)))
+    if cfg.neighbour_sampling == "weighted":
+        check(L.grf_walk_weighted(ctypes.byref(g), ctypes.byref(c), _ptr(alias), stride, _ptr(stage_col),
+                                  _ptr(stage_sum), _ptr(row_cnt), _ptr(visits), _stream(dev)))
+    else:
+        check(L.grf_walk(ctypes.byref(g), ctypes.byref(c), stride, _ptr(stage_col), _ptr(stage_sum), _ptr(row_cnt),
+                         _ptr(visits), _stream(dev)))
     return Staging(stage_col, stage_sum, row_cnt, stride, n_rows, start_lo, visits, col_counts, stage_ent)
 
 

@@ -141,10 +141,12 @@ def pilot_row_cost(graph, cfg, pilot_walks: int = 25, walk_share: float = 0.38) 
     region fills three times the entries of one in the tail, and everything after the walker (compaction,
     transposition, both halves of the product) scales with entries, not with walks.  Cost = ``walk_share`` x the
     node's share of the walks + the rest x its share of the pilot entries (config 4, one GPU: walker 17.9 ms of
-    47 ms).  Same draws on every rank, so every rank computes the same bounds."""
+    47 ms).  Same draws on every rank, so every rank computes the same bounds.  The pilot samples neighbours as
+    ``cfg`` does: weighted draws reach other rows than uniform ones, so the balance follows the Phi that is built."""
     from . import engine
 
-    pilot = engine.WalkConfig(int(pilot_walks), cfg.p_halt, cfg.max_walk_length, seed=cfg.seed)
+    pilot = engine.WalkConfig(int(pilot_walks), cfg.p_halt, cfg.max_walk_length, seed=cfg.seed,
+                              neighbour_sampling=getattr(cfg, "neighbour_sampling", "uniform"))
     phi = engine.build_phi_blocks(graph, pilot, transpose=False)
     L = phi.n_steps
     ptr = phi.blk_ptr

@@ -86,6 +86,39 @@ typedef struct {
     int32_t pad;
 } GrfEdge;
 
+/* Weight-proportional neighbour draws (grf_walk_weighted): one bucket of a row's alias table, 32 bytes = one
+ * sector.  Bucket k of a row holds its own entry (col, scaled) and its alias (col_alias, scaled_alias);
+ * scaled = sign(w) * S / (1 - p_halt) of that entry, the load factor of a step through it.
+ *
+ * Definition, for row i with d entries, weights w_k and a_k = |w_k| (k = 0 .. d-1, CSR order):
+ *   S       float64: s_l = sum of a_k over k = l, l + 32, l + 64, ... in that order from 0.0 (l = 0 .. 31),
+ *           then for h = 16, 8, 4, 2, 1: s_l = s_l + s_{l+h} (l < h); S = s_0.
+ *   masses  m_k = (uint64)floor((a_k * D) / S), D = d * 2^32, float64 multiply then divide, no contraction.
+ *           The deficit d * 2^32 - sum m_k (int64, may be negative) is added to the largest m_k (lowest index
+ *           among ties).  Rows whose |w| are all equal get m_k = 2^32 exactly.
+ *   table   T = 2^32.  Light items (m < T) and heavy items (m > T) are each taken in index order (Vose's
+ *           method, sweeping form of Huebschle-Schneider & Sanders 2019): h = first heavy, r = m_h; loop:
+ *             r > T:  the next light item k gets thr_k = m_k, alias_k = h; r -= T - m_k
+ *             r < T:  bucket h gets thr_h = r, alias_h = h' = the next heavy item; r = m_h' - (T - r); h = h'
+ *             r = T:  bucket h is full; h = the next heavy item (none: done), r = m_h.
+ *           A full bucket (m_k = T, or a heavy item left at exactly T) has thr = 0xffffffff and aliases
+ *           itself.  Everything after the masses is integer arithmetic: one exact table per row.
+ *   S = 0   (only explicit zeros): every bucket is full with scaled = 0.0, the walk stops there (a dead end).
+ *   draw    with the neighbour word x of the Philox schedule of GrfWalkCfg.seed (same counter, same word):
+ *           P = (uint64)x * d, j = P >> 32 (the uniform draw's index), frac = (uint32)P; the walk takes
+ *           bucket j's entry if frac < thr_j, else its alias.  Entry k is taken with probability m_k / 2^32 / d,
+ *           |w_k| / S up to d / 2^32; w = 0 is never taken.  load = load * scaled of the entry taken.
+ * On a row whose weights are all +-1 every bucket is full and the draw is the uniform one; the factor
+ * sign(w) * (d / (1 - p)) equals (d * w) / (1 - p): the weighted walk is then bit-identical to grf_walk. */
+typedef struct {
+    double scaled;
+    double scaled_alias;
+    int32_t col;
+    int32_t col_alias;
+    uint32_t thr;
+    int32_t pad;
+} GrfAliasEdge;
+
 /* Arguments of _worker_walks (sparse_sampler.py:26-31) plus the shard and the
  * draw source. */
 typedef struct {
@@ -213,6 +246,20 @@ int64_t grf_walk_stage_stride(int32_t walks_per_node, int32_t max_walk_length);
  * one step at a time with coupled draws (same outputs, same summation). */
 int grf_walk(const GrfGraph *graph, const GrfWalkCfg *cfg, int64_t stage_stride, int32_t *stage_col,
              double *stage_sum, int32_t *row_cnt, unsigned long long *visits_out, void *stream);
+
+/* Weight-proportional neighbour draws (no reference counterpart; definitions at GrfAliasEdge): the alias
+ * tables of every row for this p_halt (csrc/grf_alias.cu), once per graph and p_halt as grf_edge_records.
+ * The weights must be finite (the caller checks). */
+int grf_alias_records(const GrfGraph *graph, double p_halt, GrfAliasEdge *out /* [nnz] */, void *stream);
+
+/* grf_walk with neighbour k of a row taken with probability |w_k| / S and the load multiplied by
+ * sign(w_k) * S / (1 - p_halt): an unbiased M_l whose per-step factor is bounded by S / (1 - p) (on the
+ * normalized Laplacian S <= 1 + sqrt(deg)).  Same outputs as grf_walk.  cfg->draw_mode: GRF_DRAW_PHILOX,
+ * optionally | GRF_DRAW_COUPLE_HALT; cfg->load_mode: GRF_LOAD_CUMULATIVE; cfg->edges: NULL; `alias` from
+ * grf_alias_records for cfg->p_halt (may be NULL only when no step can be taken: L = 1, p_halt = 1 or nnz = 0). */
+int grf_walk_weighted(const GrfGraph *graph, const GrfWalkCfg *cfg, const GrfAliasEdge *alias,
+                      int64_t stage_stride, int32_t *stage_col, double *stage_sum, int32_t *row_cnt,
+                      unsigned long long *visits_out, void *stream);
 
 /* Exclusive prefix sum of row_cnt[n_rows][L] in row-major or step-major order;
  * offsets has n_rows*L + 1 elements (last = total).  out_is_i64 selects

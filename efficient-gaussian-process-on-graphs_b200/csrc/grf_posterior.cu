@@ -172,6 +172,257 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_quadform_kernel(
     }
 }
 
+// ---- row projection: out[i, c] = sum_{e in row x[i], slot >= 0} w_e B[slot(e), c] -------------------------------
+// The posterior mean (r = 1), samples (r up to 64) and covariance (r = n) are this product.  Three warp shapes,
+// chosen by r (profiles/prof_row_project_shapes.py compares them with a build that takes the panels for every r):
+//   r <= 4   row_project_narrow_kernel: lanes own entries.  In the panel form one lane of 32 would gather B for
+//            every touched entry of the row in a serial chain of dependent loads (power-law hub rows hold 10^4 and
+//            more); here every lane gathers its own entries, four rounds of loads in flight at a time.
+//   <= 64    row_project_mid_kernel: entry groups x column quads, so the gather chain of a row is split over the
+//            groups instead of running in the few lanes whose columns are < r.
+//   r > 64   row_project_kernel: the panels of row_quadform_kernel (128 columns, a float4 of column sums per
+//            lane), stored instead of squared (16-byte stores when out and ldo allow it); long rows re-stream per
+//            panel in the same order.
+// Each fixes its summation order and uses no atomics, so repeated calls agree bit for bit.
+
+// columns [c, min(c + 4, r)) of s into the output row o
+__device__ __forceinline__ void pj_store(float *__restrict__ o, int32_t c, int32_t r, const float4 &s, bool vec) {
+    if (c >= r) return;
+    if (vec && c + 4 <= r) {
+        *reinterpret_cast<float4 *>(o + c) = s;
+        return;
+    }
+    o[c] = s.x;
+    if (c + 1 < r) o[c + 1] = s.y;
+    if (c + 2 < r) o[c + 2] = s.z;
+    if (c + 3 < r) o[c + 3] = s.w;
+}
+
+// r <= 4: lane l adds w * B[slot, 0 .. 3] for its entries l, l + 32, l + 64, ... in that order, with the loads of
+// kNarrowRounds rounds issued before their sums; the warp then adds the lanes with a fixed xor tree (every lane ends
+// with the same bits) and lane c stores column c.  With VEC a 16-byte load reads B[slot, 0 .. 3] (ldb % 4 == 0, so
+// those columns lie inside the row); otherwise columns past r - 1 load column r - 1 again, and are never stored.
+constexpr int kNarrowRounds = 4;
+
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_project_narrow_kernel(
+    const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
+    const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows, const int32_t *__restrict__ col_slot,
+    const float *__restrict__ B, int64_t ldb, int32_t r, float *__restrict__ out, int64_t ldo) {
+    __shared__ float fs[kMaxSteps];
+    if (threadIdx.x < kMaxSteps) fs[threadIdx.x] = threadIdx.x < L ? __ldg(f + threadIdx.x) : 0.f;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int2 *ent2 = reinterpret_cast<const int2 *>(ent);
+    const int o1 = min(1, r - 1), o2 = min(2, r - 1), o3 = min(3, r - 1);
+    for (int64_t i = warp0; i < n; i += n_warps) {
+        const int64_t a = (x ? (int64_t)__ldg(x + i) : i + row_lo) - row_lo;
+        float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (a >= 0 && a < n_rows) {   // rows outside this shard stay +0
+            const int32_t b = __ldg(ptr + a * L), e = __ldg(ptr + (a + 1) * L);
+            for (int32_t k0 = b + lane; k0 < e; k0 += 32 * kNarrowRounds) {
+                int2 en[kNarrowRounds];
+                int32_t slot[kNarrowRounds];
+                float4 v[kNarrowRounds];
+#pragma unroll
+                for (int u = 0; u < kNarrowRounds; ++u)
+                    en[u] = k0 + 32 * u < e ? __ldg(ent2 + k0 + 32 * u) : make_int2(0, 0);
+#pragma unroll
+                for (int u = 0; u < kNarrowRounds; ++u)
+                    slot[u] = k0 + 32 * u < e ? __ldg(col_slot + entry_col(en[u].x)) : -1;
+#pragma unroll
+                for (int u = 0; u < kNarrowRounds; ++u) {
+                    v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (slot[u] >= 0) {
+                        const float *row = B + (int64_t)slot[u] * ldb;
+                        if (VEC) {
+                            v[u] = __ldg(reinterpret_cast<const float4 *>(row));
+                        } else {
+                            v[u].x = __ldg(row);
+                            v[u].y = __ldg(row + o1);
+                            v[u].z = __ldg(row + o2);
+                            v[u].w = __ldg(row + o3);
+                        }
+                    }
+                }
+#pragma unroll
+                for (int u = 0; u < kNarrowRounds; ++u) {
+                    if (slot[u] >= 0) {
+                        const float w = fs[entry_step(en[u].x)] * __int_as_float(en[u].y);
+                        s.x = fmaf(w, v[u].x, s.x);
+                        s.y = fmaf(w, v[u].y, s.y);
+                        s.z = fmaf(w, v[u].z, s.z);
+                        s.w = fmaf(w, v[u].w, s.w);
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            s.x += __shfl_xor_sync(0xffffffffu, s.x, o);
+            s.y += __shfl_xor_sync(0xffffffffu, s.y, o);
+            s.z += __shfl_xor_sync(0xffffffffu, s.z, o);
+            s.w += __shfl_xor_sync(0xffffffffu, s.w, o);
+        }
+        if (lane < r) out[i * ldo + lane] = lane == 0 ? s.x : lane == 1 ? s.y : lane == 2 ? s.z : s.w;
+    }
+}
+
+// s += w * B[slot, c .. c + 3]: a 16-byte load, or scalar loads of columns < r (columns past r - 1 load column
+// r - 1 again, whose sums pj_store drops)
+template <bool VEC>
+__device__ __forceinline__ void pj_fma(const float *__restrict__ B, int64_t ldb, int32_t slot, float w, int32_t c,
+                                       int32_t r, float4 &s) {
+    const float *row = B + (int64_t)slot * ldb + c;
+    if (VEC) {
+        const float4 v = __ldg(reinterpret_cast<const float4 *>(row));
+        s.x = fmaf(w, v.x, s.x);
+        s.y = fmaf(w, v.y, s.y);
+        s.z = fmaf(w, v.z, s.z);
+        s.w = fmaf(w, v.w, s.w);
+    } else {
+        const int o1 = min(1, r - 1 - c), o2 = min(2, r - 1 - c), o3 = min(3, r - 1 - c);
+        s.x = fmaf(w, __ldg(row), s.x);
+        s.y = fmaf(w, __ldg(row + o1), s.y);
+        s.z = fmaf(w, __ldg(row + o2), s.z);
+        s.w = fmaf(w, __ldg(row + o3), s.w);
+    }
+}
+
+// 4 < r <= 64: group g of the 32 / Q entry groups adds the buffered pairs g, g + 32 / Q, ... (Q column quads,
+// Q = 1 << qlog); four pairs' loads in flight at a time
+template <bool VEC>
+__device__ __forceinline__ void pj_gather_groups(const QfPair *buf, int cnt, int grp, int step,
+                                                 const float *__restrict__ B, int64_t ldb, int32_t c, int32_t r,
+                                                 float4 &s) {
+    if (c >= r) return;
+    int j = grp;
+    for (; j + 3 * step < cnt; j += 4 * step) {
+        QfPair p[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) p[u] = buf[j + u * step];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) pj_fma<VEC>(B, ldb, p[u].slot, p[u].w, c, r, s);
+    }
+    for (; j < cnt; j += step) {
+        const QfPair p = buf[j];
+        pj_fma<VEC>(B, ldb, p.slot, p.w, c, r, s);
+    }
+}
+
+// 4 < r <= 64: the warp is 32 / Q entry groups x Q column quads (Q the next power of two >= r / 4).  The touched
+// pairs are compacted as in row_quadform_kernel, each group gathers its share, the groups are added with a fixed
+// xor tree and group 0 stores.  Rows with more touched entries than the buffer re-stream in buffer loads.
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_project_mid_kernel(
+    const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
+    const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows, const int32_t *__restrict__ col_slot,
+    const float *__restrict__ B, int64_t ldb, int32_t r, float *__restrict__ out, int64_t ldo, int32_t qlog,
+    bool vec_out) {
+    __shared__ float fs[kMaxSteps];
+    __shared__ QfPair sbuf[kQfWarps][kQfCap];
+    if (threadIdx.x < kMaxSteps) fs[threadIdx.x] = threadIdx.x < L ? __ldg(f + threadIdx.x) : 0.f;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int grp = lane >> qlog, step = 32 >> qlog;
+    const int32_t c = 4 * (lane & ((1 << qlog) - 1));
+    QfPair *buf = sbuf[threadIdx.x >> 5];
+    const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int2 *ent2 = reinterpret_cast<const int2 *>(ent);
+    double unused = 0.0;
+    for (int64_t i = warp0; i < n; i += n_warps) {
+        const int64_t a = (x ? (int64_t)__ldg(x + i) : i + row_lo) - row_lo;
+        float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (a >= 0 && a < n_rows) {   // rows outside this shard stay +0
+            const int32_t b = __ldg(ptr + a * L), e = __ldg(ptr + (a + 1) * L);
+            int cnt = 0;
+            for (int32_t k0 = b; k0 < e; k0 += 32)
+                cnt += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, cnt, lane, unused);
+            __syncwarp();
+            if (cnt <= kQfCap) {
+                pj_gather_groups<VEC>(buf, cnt, grp, step, B, ldb, c, r, s);
+            } else {
+                int part = 0;
+                for (int32_t k0 = b; k0 < e; k0 += 32) {
+                    if (part + 32 > kQfCap) {
+                        __syncwarp();
+                        pj_gather_groups<VEC>(buf, part, grp, step, B, ldb, c, r, s);
+                        __syncwarp();
+                        part = 0;
+                    }
+                    part += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, part, lane, unused);
+                }
+                __syncwarp();
+                pj_gather_groups<VEC>(buf, part, grp, step, B, ldb, c, r, s);
+            }
+            __syncwarp();   // the buffer is reused by the next row
+        }
+        for (int o = 16; o >= (1 << qlog); o >>= 1) {
+            s.x += __shfl_xor_sync(0xffffffffu, s.x, o);
+            s.y += __shfl_xor_sync(0xffffffffu, s.y, o);
+            s.z += __shfl_xor_sync(0xffffffffu, s.z, o);
+            s.w += __shfl_xor_sync(0xffffffffu, s.w, o);
+        }
+        if (grp == 0) pj_store(out + i * ldo, c, r, s, vec_out);
+    }
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_project_kernel(
+    const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
+    const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows, const int32_t *__restrict__ col_slot,
+    const float *__restrict__ B, int64_t ldb, int32_t r, float *__restrict__ out, int64_t ldo, bool vec_out) {
+    __shared__ float fs[kMaxSteps];
+    __shared__ QfPair sbuf[kQfWarps][kQfCap];
+    if (threadIdx.x < kMaxSteps) fs[threadIdx.x] = threadIdx.x < L ? __ldg(f + threadIdx.x) : 0.f;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    QfPair *buf = sbuf[threadIdx.x >> 5];
+    const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int2 *ent2 = reinterpret_cast<const int2 *>(ent);
+    double unused = 0.0;
+    for (int64_t i = warp0; i < n; i += n_warps) {
+        const int64_t a = (x ? (int64_t)__ldg(x + i) : i + row_lo) - row_lo;
+        int32_t b = 0, e = 0;                 // rows outside this shard: no entries, a row of +0
+        if (a >= 0 && a < n_rows) {
+            b = __ldg(ptr + a * L);
+            e = __ldg(ptr + (a + 1) * L);
+        }
+        int cnt = 0;
+        for (int32_t k0 = b; k0 < e; k0 += 32)
+            cnt += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, cnt, lane, unused);
+        __syncwarp();
+        float *o = out + i * ldo;
+        for (int32_t c0 = 0; c0 < r; c0 += kQfPanel) {
+            const int32_t c = c0 + 4 * lane;
+            float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (cnt <= kQfCap) {
+                qf_gather<VEC>(buf, cnt, B, ldb, c, r, s);
+            } else {
+                int part = 0;
+                for (int32_t k0 = b; k0 < e; k0 += 32) {
+                    if (part + 32 > kQfCap) {
+                        __syncwarp();
+                        qf_gather<VEC>(buf, part, B, ldb, c, r, s);
+                        __syncwarp();
+                        part = 0;
+                    }
+                    part += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, part, lane, unused);
+                }
+                __syncwarp();
+                qf_gather<VEC>(buf, part, B, ldb, c, r, s);
+                __syncwarp();
+            }
+            pj_store(o, c, r, s, vec_out);
+        }
+        __syncwarp();   // the buffer is reused by the next row
+    }
+}
+
 }  // namespace
 }  // namespace grf
 
@@ -200,4 +451,52 @@ extern "C" int grf_phi_row_quadform(const GrfPhi *phi, const float *f, const int
                                                                      x, n, phi->row_lo, phi->n_rows, col_slot, C,
                                                                      ldc, r, q, d);
     return check_cuda(cudaGetLastError(), "row_quadform_kernel launch");
+}
+
+extern "C" int grf_phi_row_project(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n,
+                                   const int32_t *col_slot, const float *B, int64_t ldb, int32_t r, float *out,
+                                   int64_t ldo, void *stream) {
+    GRF_ON_STREAM_DEVICE(stream, out);
+    GRF_REQUIRE(phi && f && col_slot && B && out, "grf_phi_row_project: null argument");
+    GRF_REQUIRE(n >= 0 && r >= 0 && ldb >= r && ldo >= r, "grf_phi_row_project: bad n / r / ldb / ldo");
+    GRF_REQUIRE(phi->n_steps >= 1 && phi->n_steps <= kMaxSteps, "grf_phi_row_project: n_steps out of range");
+    GRF_REQUIRE(x || n == phi->n_rows, "grf_phi_row_project: n must equal n_rows when x is NULL");
+    GRF_REQUIRE(phi->blk_ptr, "grf_phi_row_project: Phi blocks missing");
+    if (n == 0 || r == 0) return GRF_OK;
+    const bool vin = ldb % 4 == 0 && ((uintptr_t)B & 15u) == 0;
+    const bool vout = ldo % 4 == 0 && ((uintptr_t)out & 15u) == 0;
+    int64_t g = (n + kQfWarps - 1) / kQfWarps;
+    if (g > (int64_t)kSmCount * 16) g = (int64_t)kSmCount * 16;
+    const dim3 grid((unsigned)g), block(kQfWarps * 32);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int32_t *ptr = phi->blk_ptr;
+    const GrfEntry *ent = phi->entries;
+    const int32_t L = phi->n_steps;
+    if (r <= 4) {
+        if (vin)
+            row_project_narrow_kernel<true><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
+                                                                    col_slot, B, ldb, r, out, ldo);
+        else
+            row_project_narrow_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
+                                                                     col_slot, B, ldb, r, out, ldo);
+        return check_cuda(cudaGetLastError(), "row_project_narrow_kernel launch");
+    }
+    if (r <= 64) {
+        int qlog = 1;                         // quads: the next power of two >= ceil(r / 4), 2 .. 16
+        while ((4 << qlog) < r) ++qlog;
+        if (vin)
+            row_project_mid_kernel<true><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
+                                                                 col_slot, B, ldb, r, out, ldo, qlog, vout);
+        else
+            row_project_mid_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
+                                                                  col_slot, B, ldb, r, out, ldo, qlog, vout);
+        return check_cuda(cudaGetLastError(), "row_project_mid_kernel launch");
+    }
+    if (vin)
+        row_project_kernel<true><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows, col_slot, B,
+                                                         ldb, r, out, ldo, vout);
+    else
+        row_project_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows, col_slot, B,
+                                                          ldb, r, out, ldo, vout);
+    return check_cuda(cudaGetLastError(), "row_project_kernel launch");
 }

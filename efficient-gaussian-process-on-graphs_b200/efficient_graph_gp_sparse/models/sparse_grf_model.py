@@ -57,6 +57,30 @@ class SparseGraphGP(ExactGP):
         post = ExactPosterior(blocks, f, train_indices, float(self.likelihood.noise.item()))
         return post.variance(test_indices, include_noise=include_noise)
 
+    def posterior_covariance(self, x_test, include_noise=False):
+        """Exact joint posterior covariance K** - K*X (K(X, X) + sigma^2 I)^-1 KX* between the test nodes (float64
+        device tensor [q, q], exactly symmetric), with sigma^2 I added when ``include_noise``
+        (grf_b200/posterior.py)."""
+        from grf_b200.posterior import ExactPosterior
+
+        blocks = self.covar_module.phi_blocks
+        f = self.covar_module.modulator_vector.detach()
+        train_indices = self.x_train.long().flatten()
+        test_indices = torch.as_tensor(x_test).long().flatten()
+        post = ExactPosterior(blocks, f, train_indices, float(self.likelihood.noise.item()))
+        return post.covariance(test_indices, include_noise=include_noise)
+
+    def exact_posterior(self):
+        """The exact posterior (grf_b200.posterior.ExactPosterior) for the current modulator, noise, x_train and
+        y_train: factor once per refit, then ``mean``, ``variance``, ``covariance`` and ``sample`` at any test
+        nodes without a further solve."""
+        from grf_b200.posterior import ExactPosterior
+
+        blocks = self.covar_module.phi_blocks
+        f = self.covar_module.modulator_vector.detach()
+        return ExactPosterior(blocks, f, self.x_train.long().flatten(), float(self.likelihood.noise.item()),
+                              y_train=self.y_train.flatten())
+
     def predict(self, x_test, n_samples=64, cg_tolerance=None, max_cg_iterations=1000, return_info=False):
         """Posterior samples at ``x_test`` by pathwise conditioning (sparse_grf_model.py:21-45):
         f_test_prior + K_test,train (K_train,train + sigma^2 I)^-1 (y - f_train_prior - eps)."""

@@ -1161,6 +1161,42 @@ class PhiBlocks:
                                               ldc, r, _ptr(q), _ptr(d), _stream(dev)))
         return q, d
 
+    def row_project(self, f, x, col_slot, B, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """out[i, c] = sum_{e in row x[i], col_slot[col e] >= 0} w_e B[col_slot[col e], c], w_e = f[length e] * e.val
+        (``grf_phi_row_project``), float32 [n, r].  B: float32 [m, r] (a column slice of a wider buffer is read in
+        place; any other layout is copied); ValueError when col_slot names a row past m.  ``out``: a float32 [n, r]
+        tensor with unit column stride and rows at least r floats apart to write into.  x = None:
+        every local row.  See grf_b200/posterior.py for the posterior mean, covariance and samples built on it."""
+        dev = self.device
+        f = self._f(f)
+        xi = self._ids(x, dev)
+        n = self.n_rows if xi is None else xi.numel()
+        col_slot = torch.as_tensor(col_slot, device=dev).to(torch.int32).contiguous()
+        if col_slot.numel() != self.n_cols:
+            raise ValueError(f"row_project: col_slot has {col_slot.numel()} entries, Phi has {self.n_cols} columns")
+        if B.dim() != 2 or B.dtype != torch.float32 or B.device != dev:
+            raise ValueError("row_project: B must be a 2-D float32 tensor on Phi's device")
+        r = int(B.shape[1])
+        if (r > 1 and B.stride(1) != 1) or (B.shape[0] > 1 and B.stride(0) < r):
+            B = B.contiguous()          # the kernel reads rows of r floats ldb apart
+        ldb = int(B.stride(0)) if B.shape[0] > 1 else r
+        if out is None:
+            out = torch.empty((n, r), dtype=torch.float32, device=dev)
+        elif (out.shape != (n, r) or out.dtype != torch.float32 or out.device != dev
+              or (r > 1 and out.stride(1) != 1) or (n > 1 and out.stride(0) < r)):
+            raise ValueError(f"row_project: out must be a float32 [{n}, {r}] tensor on Phi's device with unit column "
+                             f"stride and rows at least {r} floats apart")
+        if n == 0 or r == 0:
+            return out
+        if col_slot.numel() and int(col_slot.max()) >= B.shape[0]:
+            raise ValueError(f"row_project: col_slot names row {int(col_slot.max())} of B, which has {B.shape[0]} rows")
+        ldo = int(out.stride(0)) if n > 1 else r
+        keep = B if B.numel() else torch.zeros(1, dtype=torch.float32, device=dev)   # no row of B is read then
+        phi = self.c_struct()
+        check(_lib.lib().grf_phi_row_project(ctypes.byref(phi), _ptr(f), _ptr(xi), n, _ptr(col_slot), _ptr(keep),
+                                             ldb, r, _ptr(out), ldo, _stream(dev)))
+        return out
+
     def _f(self, f) -> torch.Tensor:
         f = torch.as_tensor(f, device=self.device).detach().to(torch.float32).contiguous()
         if f.numel() != self.n_steps:

@@ -510,6 +510,17 @@ int grf_phi_row_dots(const GrfPhi *phi, const float *f, const int32_t *x1, const
 int grf_phi_row_quadform(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n, const int32_t *col_slot,
                          const float *C, int64_t ldc, int32_t r, float *q, float *d, void *stream);
 
+/* Row projection onto the training column set (csrc/grf_posterior.cu): with w_e = f[length(e)] * e.val,
+ *   out[i * ldo + c] = sum_{e in row x[i], col_slot[col(e)] >= 0} w_e * B[col_slot[col(e)] * ldb + c]    (c < r)
+ * col_slot as for grf_phi_row_quadform; B [m][ldb] float32.  With the slot map and factor of
+ * grf_b200/posterior.py this is the exact posterior mean (B = G K^-1 y, r = 1), the cross term of the joint
+ * covariance (B = C = G L^-T, r = n) and the correction of pathwise samples (B = G K^-1 V, r = samples).
+ * x: global row ids (NULL = every local row, n = n_rows); ids outside [row_lo, row_lo + n_rows) give a row of +0.
+ * Only columns [0, r) of out are written, and columns [r, ldb) of B never reach a result.  The summation order
+ * is fixed (no atomics), so repeated calls agree bit for bit.  Per-length and merged blocks, L <= 32. */
+int grf_phi_row_project(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n, const int32_t *col_slot,
+                        const float *B, int64_t ldb, int32_t r, float *out, int64_t ldo, void *stream);
+
 /* The one exchange of the path (SURVEY.md 8e; no reference counterpart: its matvec runs on one device):
  * U <- sum over the GPUs of the partials U_g = Phi_g[x2]^T V_g between the two halves of a product, as one
  * kernel per rank over NVLink peer memory.  peer_u[g] / peer_flags[g] (HOST arrays of `world` DEVICE pointers)

@@ -81,6 +81,15 @@ class SparseGraphGP(ExactGP):
         return ExactPosterior(blocks, f, self.x_train.long().flatten(), float(self.likelihood.noise.item()),
                               y_train=self.y_train.flatten())
 
+    def exact_mll(self):
+        """The exact -mll/n and its closed-form gradients (grf_b200.mll.ExactMLL) for x_train and y_train: the
+        per-length Gram of the training rows is built once, then ``loss(f, noise)`` / ``backward(kernel,
+        likelihood)`` cost dense n x n float64 work per evaluation.  A drop-in for ``neg_mll_backward`` in a refit
+        loop, deterministic, so L-BFGS can run on it."""
+        from grf_b200.mll import ExactMLL
+
+        return ExactMLL(self.covar_module.phi_blocks, self.x_train.long().flatten(), self.y_train.flatten())
+
     def predict(self, x_test, n_samples=64, cg_tolerance=None, max_cg_iterations=1000, return_info=False):
         """Posterior samples at ``x_test`` by pathwise conditioning (sparse_grf_model.py:21-45):
         f_test_prior + K_test,train (K_train,train + sigma^2 I)^-1 (y - f_train_prior - eps)."""

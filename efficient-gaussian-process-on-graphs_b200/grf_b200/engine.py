@@ -43,6 +43,9 @@ _LAZY_ENTRY_BYTES = 1 << 30  # up to this bound the Phi entries are allocated by
 # blocks the first half of the config-4 product went from 7.4 to 12.8 ms (every block re-reads the 21 M segment
 # pointers and read-modify-writes all of U, and most columns hold ~1 entry per block).  Hence one block up to 2^22 rows.
 T_BLOCK_ROWS = 1 << 22
+# training_gram: a column reached by more than this many (training row, length) entries is a hub column; its
+# products go to the dense float64 H H^T instead of the light kernel (choice measured in DESIGN.md, section 3)
+GRAM_HEAVY_THRESHOLD = 4096
 
 
 def _device(device=None) -> torch.device:
@@ -84,6 +87,17 @@ def _keep_until_done(buf: torch.Tensor, event: torch.cuda.Event) -> None:
     not see: hold a reference until the copy's event has completed, whoever drops the owner first."""
     _pending_host[:] = [(b, e) for b, e in _pending_host if not e.query()]
     _pending_host.append((buf, event))
+
+
+def _free_bytes(dev: torch.device) -> int:
+    free, _ = torch.cuda.mem_get_info(dev)
+    return int(free) + int(torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev))
+
+
+def training_gram_bytes(n: int, L: int, h: int) -> int:
+    """Bytes of PhiBlocks.training_gram's E (float64 [L n, L n]) and of the dense H (float64 [L n, h]) of its h hub
+    columns."""
+    return 8 * (n * L) ** 2 + 8 * n * L * h
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -1196,6 +1210,92 @@ class PhiBlocks:
         check(_lib.lib().grf_phi_row_project(ctypes.byref(phi), _ptr(f), _ptr(xi), n, _ptr(col_slot), _ptr(keep),
                                              ldb, r, _ptr(out), ldo, _stream(dev)))
         return out
+
+    def training_gram(self, x, mem_limit: Optional[int] = None) -> torch.Tensor:
+        """E[l, i, l', j] = <M_l[x_i], M_l'[x_j]>, float64 [L, n, L, n]: the per-length Gram of the training rows, so
+        that K(f) = sum_{l, l'} f_l f_l' E[l, :, l', :] for every modulator f (grf_b200/mll.py fits f and sigma^2 on
+        it).  Products are exact in float64 and the sums have a fixed order: repeated calls agree bit for bit, and
+        the (L n) x (L n) view is exactly symmetric.  Repeated ids are allowed.  ValueError on a row shard,
+        IndexError for ids outside Phi, MemoryError (naming the bytes) before E or the hub columns' dense H are
+        allocated when they do not fit in ``mem_limit`` bytes (default: the free device memory)."""
+        return self._training_gram(x, mem_limit)[0]
+
+    def _training_gram(self, x, mem_limit: Optional[int] = None, events: Optional[dict] = None):
+        """training_gram, plus its sizes (dict: n, L, nnz_train, m, h, p_light, threshold); ``events`` receives CUDA
+        events "gather", "light", "heavy" and "symmetrise" at the stage ends."""
+        if self.is_shard:
+            raise ValueError("training_gram needs the whole Phi; a row shard holds only some of the training rows")
+        dev = self.device
+        xi = self._ids(x, dev)
+        self.check_ids(xi)
+        n, L = int(xi.numel()), self.n_steps
+        N = n * L
+        T = GRAM_HEAVY_THRESHOLD
+
+        def mark(name):
+            if events is not None:
+                events[name] = torch.cuda.Event(enable_timing=True)
+                events[name].record(torch.cuda.current_stream(dev))
+
+        with torch.cuda.device(dev):
+            i64 = torch.int64
+            ptr = self.blk_ptr.to(i64)
+            xl = xi.to(i64)
+            start = ptr[xl * L]
+            lens = ptr[(xl + 1) * L] - start
+            total = int(lens.sum().item()) if n else 0
+            i = torch.repeat_interleave(torch.arange(n, device=dev), lens, output_size=total)
+            first = torch.cumsum(lens, 0) - lens
+            idx = start[i] + torch.arange(total, device=dev) - first[i]
+            word = self.entries[idx, 0].to(i64) & 0xFFFFFFFF
+            val = self.entries[idx, 1].view(torch.float32)
+            row = (word >> _lib.ENTRY_STEP_SHIFT) * n + i                  # E row l n + i of every entry
+            cols, slot = torch.unique(word & ((1 << _lib.ENTRY_STEP_SHIFT) - 1), return_inverse=True)
+            del word, idx, first, i, start, lens
+            m = int(cols.numel())
+            t = torch.bincount(slot, minlength=m)                          # t_s
+            heavy_slot = t > T
+            h = int(heavy_slot.sum().item()) if m else 0
+            need = training_gram_bytes(n, L, h)
+            budget = _free_bytes(dev) if mem_limit is None else int(mem_limit)
+            if need > budget:
+                raise MemoryError(f"training_gram: E of {n} training rows x {L} lengths and H of {h} hub columns "
+                                  f"need {need} bytes, {budget} bytes of device memory are free")
+            stats = dict(n=n, L=L, nnz_train=total, m=m, h=h, threshold=T,
+                         p_light=int((t[~heavy_slot] ** 2).sum().item()) if m else 0)
+            heavy = heavy_slot[slot]
+            light = ~heavy
+            rl, sl, vl = row[light], slot[light], val[light].view(torch.int32)
+            by_row = torch.argsort(rl * max(m, 1) + sl)                    # (row, slot) is unique
+            row_ent = torch.stack([sl[by_row].to(torch.int32), vl[by_row]], 1).contiguous()
+            by_slot = torch.argsort(sl * max(N, 1) + rl)
+            slot_ent = torch.stack([rl[by_slot].to(torch.int32), vl[by_slot]], 1).contiguous()
+            del by_row, by_slot
+            row_ptr = torch.zeros(N + 1, dtype=torch.int32, device=dev)
+            row_ptr[1:] = torch.cumsum(torch.bincount(rl, minlength=N), 0)
+            slot_ptr = torch.zeros(m + 1, dtype=torch.int32, device=dev)
+            slot_ptr[1:] = torch.cumsum(torch.bincount(sl, minlength=m), 0)
+            work = torch.zeros(N, dtype=i64, device=dev).index_add_(0, rl, t[sl])   # integer: order-free
+            order = torch.argsort(work, descending=True, stable=True).to(torch.int32)
+            del work, rl, sl, vl
+            mark("gather")
+            E = torch.zeros((N, N), dtype=torch.float64, device=dev)
+            lib = _lib.lib()
+            if row_ent.numel():
+                check(lib.grf_gram_light(_ptr(order), N, _ptr(row_ptr), _ptr(row_ent), _ptr(slot_ptr),
+                                         _ptr(slot_ent), m, _ptr(E), N, _stream(dev)))
+            del row_ent, slot_ent, row_ptr, slot_ptr, order
+            mark("light")
+            if h:
+                hcol = torch.cumsum(heavy_slot, 0) - 1
+                H = torch.zeros((N, h), dtype=torch.float64, device=dev)
+                H[row[heavy], hcol[slot[heavy]]] = val[heavy].to(torch.float64)   # one entry per (row, slot)
+                E.addmm_(H, H.T)                                            # E + H H^T, after the light sums
+                del H, hcol
+            mark("heavy")
+            check(lib.grf_gram_mirror(_ptr(E), N, N, _stream(dev)))
+            mark("symmetrise")
+        return E.view(L, n, L, n), stats
 
     def _f(self, f) -> torch.Tensor:
         f = torch.as_tensor(f, device=self.device).detach().to(torch.float32).contiguous()

@@ -17,7 +17,7 @@ import torch
 
 from . import _lib
 from ._lib import check
-from .engine import _ptr, _stream, scan_counts
+from .engine import _free_bytes, _ptr, _stream, scan_counts
 
 _INT32_MAX = np.iinfo(np.int32).max
 MAX_STEPS = 128        # modulator values merged per row of Phi_f (min(len(f), L))
@@ -82,11 +82,6 @@ class KernelMatrix:
         torch.cuda.current_stream(self.data.device).synchronize()
         col = col_h.numpy() if idx == np.int32 else col_h.numpy().astype(np.int64)
         return sp.csr_matrix((val_h.numpy(), col, ip_h.numpy()), shape=(self.n, self.n))
-
-
-def _free_bytes(dev: torch.device) -> int:
-    free, _ = torch.cuda.mem_get_info(dev)
-    return int(free) + int(torch.cuda.memory_reserved(dev) - torch.cuda.memory_allocated(dev))
 
 
 def _bins(size: torch.Tensor, n: int, dev) -> tuple:

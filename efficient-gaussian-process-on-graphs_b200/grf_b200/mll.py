@@ -18,9 +18,12 @@ gpytorch is not installed in this image, so parity is against a float64 dense ev
 
 from __future__ import annotations
 
-from typing import Optional
+import math
+from typing import Dict, Optional
 
 import torch
+
+from .engine import PhiBlocks, _free_bytes
 
 
 def lanczos_logdet(matmul, probes: torch.Tensor, iterations: int = 1) -> float:
@@ -108,3 +111,142 @@ def neg_mll_backward(kernel, likelihood, x_train: torch.Tensor, y_train: torch.T
     noise.backward(torch.as_tensor([-dL_ds2 / n], dtype=noise.dtype, device=noise.device).reshape(noise.shape))
     return {"loss": loss, "datafit": datafit, "cg_iterations": info["iterations"],
             "grad_modulator": (-dL_df / n).cpu(), "grad_noise": -dL_ds2 / n}
+
+
+class _ExactLoss(torch.autograd.Function):
+    """-mll/n as a function of (f, sigma^2); the backward is the closed form of ExactMLL._evaluate, not autograd
+    through the Cholesky factor."""
+
+    @staticmethod
+    def forward(ctx, f, noise, mll):
+        out = mll._evaluate(f.detach(), noise.detach())
+        ctx.grads = [(g, t.shape, t.dtype, t.device) for g, t in ((out["grad_f"], f), (out["grad_noise"], noise))]
+        return out["loss"]
+
+    @staticmethod
+    def backward(ctx, g):
+        (gf, *f_meta), (gn, *n_meta) = ctx.grads
+
+        def like(v, shape, dtype, device):
+            return (g.to(v.device) * v).to(device=device, dtype=dtype).reshape(shape)
+
+        return like(gf, *f_meta), like(gn, *n_meta), None
+
+
+class ExactMLL:
+    """Exact negative log-marginal likelihood -mll/n of the GRF GP and its closed-form gradients in the modulator f
+    and the noise sigma^2, for fitting them on BO-sized training sets (hundreds to a few thousand nodes).
+
+    The constructor builds the per-length Gram E = PhiBlocks.training_gram(x) once (float64 [L, n, L, n]; E does
+    not depend on f or sigma^2).  Every evaluation is then dense float64 n x n work, with no pass over Phi:
+
+        K = sum_{l, b} f_l f_b E[l, :, b, :] + sigma^2 I = L_K L_K^T,       alpha = K^-1 y,   W = alpha alpha^T - K^-1
+        -mll/n = (1/2 y^T alpha + sum log diag L_K + n/2 log 2 pi) / n
+        d mll / d f_l = sum_b f_b <W, E[l, :, b, :]>_F,                      d mll / d sigma^2 = (alpha^T alpha - tr K^-1) / 2
+
+    ``loss(f, noise)`` is differentiable in both (``loss.backward()`` reaches the raw parameters behind them), and
+    ``backward(kernel, likelihood)`` is the drop-in for ``neg_mll_backward``.  Evaluations are deterministic: the
+    same (f, sigma^2) gives the same bits, so L-BFGS line searches and early stopping on the loss work.
+
+    ``y_train`` is held in float64; ValueError for non-finite values, a length other than len(x_train), an empty
+    training set or a row shard; IndexError for ids outside Phi.  ``mem_limit``: bytes E, the hub columns' dense H
+    and the n x n work arrays may take instead of the free device memory (MemoryError, naming the bytes, before they
+    are allocated).  ``events``: CUDA events at the stage boundaries ("start", then training_gram's "gather",
+    "light", "heavy", "symmetrise"; every evaluation "eval_start", "kernel", "cholesky", "solve", "grad")."""
+
+    def __init__(self, blocks: PhiBlocks, x_train, y_train, mem_limit: Optional[int] = None,
+                 events: Optional[Dict[str, torch.cuda.Event]] = None):
+        if blocks.is_shard:
+            raise ValueError("ExactMLL needs the whole Phi; a row shard holds only some of the training rows")
+        dev = blocks.device
+        self.blocks, self.events, self.device = blocks, events, dev
+        x = PhiBlocks._ids(x_train, dev)
+        blocks.check_ids(x)
+        n, L = int(x.numel()), blocks.n_steps
+        if n == 0:
+            raise ValueError("ExactMLL: the training set is empty")
+        y = torch.as_tensor(y_train, device=dev).detach().flatten().to(torch.float64)
+        if y.numel() != n:
+            raise ValueError(f"ExactMLL: y_train has {y.numel()} values for {n} training ids")
+        if not bool(torch.isfinite(y).all()):
+            raise ValueError("ExactMLL: y_train holds non-finite values")
+        self.n, self.L, self.x, self.y = n, L, x, y
+        work = exact_mll_work_bytes(n, L)
+        budget = _free_bytes(dev) if mem_limit is None else int(mem_limit)
+        if work > budget:
+            raise MemoryError(f"ExactMLL: the n x n work arrays of {n} training rows and {L} lengths need {work} "
+                              f"bytes, {budget} bytes of device memory are free")
+        with torch.cuda.device(dev):
+            self._mark("start")
+            self.E, self.gram_stats = blocks._training_gram(x, budget - work, events)
+        self.last = None
+
+    def _mark(self, name: str) -> None:
+        if self.events is not None:
+            self.events[name] = torch.cuda.Event(enable_timing=True)
+            self.events[name].record(torch.cuda.current_stream(self.device))
+
+    def _evaluate(self, f: torch.Tensor, noise: torch.Tensor) -> dict:
+        n, L, dev = self.n, self.L, self.device
+        fv = f.to(device=dev, dtype=torch.float64).flatten()
+        if fv.numel() != L:
+            raise ValueError(f"ExactMLL: the modulator has {fv.numel()} entries, Phi has {L} walk lengths")
+        s2 = float(noise)
+        if not s2 > 0.0 or s2 == float("inf"):
+            raise ValueError(f"ExactMLL: the noise variance must be positive and finite, got {s2}")
+        fh = fv.tolist()
+        with torch.cuda.device(dev):
+            self._mark("eval_start")
+            eb = torch.zeros((L, n, n), dtype=torch.float64, device=dev)    # eb[l] = sum_b f_b E[l, :, b, :]
+            for b in range(L):
+                eb.add_(self.E[:, :, b, :], alpha=fh[b])
+            k = torch.zeros((n, n), dtype=torch.float64, device=dev)
+            for l in range(L):
+                k.add_(eb[l], alpha=fh[l])
+            k.diagonal().add_(s2)
+            self._mark("kernel")
+            chol, info = torch.linalg.cholesky_ex(k)
+            del k
+            self._mark("cholesky")
+            if int(info.item()) > 0:
+                raise ValueError(f"ExactMLL: K = sum f_l f_b E_lb + sigma^2 I is not positive definite in float64 "
+                                 f"(sigma^2 = {s2}, n = {n}, leading minor {int(info.item())})")
+            alpha = torch.cholesky_solve(self.y[:, None], chol)[:, 0]
+            w = torch.cholesky_inverse(chol)
+            self._mark("solve")
+            tr_inv = w.diagonal().sum()
+            w.neg_().add_(torch.outer(alpha, alpha))                         # W = alpha alpha^T - K^-1
+            g_f = eb.reshape(L, n * n) @ w.reshape(n * n)                    # d mll / d f
+            del w, eb
+            g_s2 = 0.5 * (alpha @ alpha - tr_inv)
+            datafit = 0.5 * (self.y @ alpha)
+            logdet = 2.0 * torch.log(chol.diagonal()).sum()
+            loss = (datafit + 0.5 * logdet + 0.5 * n * math.log(2.0 * math.pi)) / n
+            self._mark("grad")
+        self.last = {"loss": loss, "datafit": datafit, "logdet": logdet, "grad_f": -g_f / n, "grad_noise": -g_s2 / n}
+        return self.last
+
+    def loss(self, f, noise) -> torch.Tensor:
+        """-mll/n at the modulator f (length L) and noise variance sigma^2 (> 0), a float64 scalar on Phi's device,
+        differentiable in ``f`` and ``noise`` when they are tensors that require grad.  ValueError for a modulator
+        of the wrong length, sigma^2 <= 0 or non-finite, or a K that is not positive definite in float64."""
+        f = f if torch.is_tensor(f) else torch.as_tensor(f, dtype=torch.float64)
+        noise = noise if torch.is_tensor(noise) else torch.as_tensor(noise, dtype=torch.float64)
+        return _ExactLoss.apply(f, noise, self)
+
+    def backward(self, kernel, likelihood) -> dict:
+        """Accumulate d(-mll/n)/dtheta into ``.grad`` of the kernel's and the likelihood's parameters (through
+        ``kernel.modulator_vector`` and ``likelihood.noise``), as ``neg_mll_backward`` does, exactly.  Returns its
+        keys (``loss``, ``datafit``, ``cg_iterations`` = 0, ``grad_modulator``, ``grad_noise``) and ``logdet``."""
+        loss = self.loss(kernel.modulator_vector, likelihood.noise)
+        loss.backward()
+        out = self.last
+        return {"loss": loss.item(), "datafit": float(out["datafit"]), "cg_iterations": 0,
+                "grad_modulator": out["grad_f"].cpu(), "grad_noise": float(out["grad_noise"]),
+                "logdet": float(out["logdet"])}
+
+
+def exact_mll_work_bytes(n: int, L: int) -> int:
+    """Bytes of one ExactMLL evaluation's float64 work arrays: sum_b f_b E[:, :, b, :] (L n^2), K, its factor and
+    K^-1 (or W) and alpha alpha^T (4 n^2)."""
+    return 8 * n * n * (L + 4)

@@ -521,6 +521,23 @@ int grf_phi_row_quadform(const GrfPhi *phi, const float *f, const int32_t *x, in
 int grf_phi_row_project(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n, const int32_t *col_slot,
                         const float *B, int64_t ldb, int32_t r, float *out, int64_t ldo, void *stream);
 
+/* Per-length Gram of the training rows, light part (csrc/grf_gram.cu; no reference counterpart: the reference
+ * estimates the marginal likelihood by CG and probes).  With A[R, c] = M_l[x_i, c] for the E row R = l * n + i,
+ * E = A A^T is float64 [n_rows][lde], n_rows = L * n.  The columns the training rows touch are numbered as slots
+ * 0 .. n_slots - 1 by the caller (grf_b200/engine.py, PhiBlocks.training_gram):
+ *   row_ptr  int32[n_rows + 1], row_ent: the entries of row R as {slot, val}, ascending slot
+ *   slot_ptr int32[n_slots + 1], slot_ent: the entries of slot s as {R', val}, each R' at most once
+ *   order    int32[n_rows], the order in which the rows are handed to the warps (NULL = ascending R)
+ * For every R and every C >= R this adds sum over the slots s shared by R and C of val(R, s) * val(C, s) into
+ * E[R * lde + C], the slots in ascending order, each product exact in float64; no other element is touched (the
+ * caller zero-fills E, adds the hub slots' dense part and mirrors).  Fixed order, no atomics: repeated calls agree
+ * bit for bit. */
+int grf_gram_light(const int32_t *order, int64_t n_rows, const int32_t *row_ptr, const GrfEntry *row_ent,
+                   const int32_t *slot_ptr, const GrfEntry *slot_ent, int64_t n_slots, double *E, int64_t lde,
+                   void *stream);
+/* E[C * lde + R] = E[R * lde + C] for every R < C < n_rows (float64): the upper triangle mirrored, exactly. */
+int grf_gram_mirror(double *E, int64_t n_rows, int64_t lde, void *stream);
+
 /* The one exchange of the path (SURVEY.md 8e; no reference counterpart: its matvec runs on one device):
  * U <- sum over the GPUs of the partials U_g = Phi_g[x2]^T V_g between the two halves of a product, as one
  * kernel per rank over NVLink peer memory.  peer_u[g] / peer_flags[g] (HOST arrays of `world` DEVICE pointers)

@@ -204,6 +204,49 @@ __device__ __forceinline__ void pj_store(float *__restrict__ o, int32_t c, int32
 // those columns lie inside the row); otherwise columns past r - 1 load column r - 1 again, and are never stored.
 constexpr int kNarrowRounds = 4;
 
+// the lane's share of the narrow sums over the entries [b, e) of one row (o1 .. o3 as in the kernel)
+template <bool VEC>
+__device__ __forceinline__ void pj_narrow_row(const int2 *__restrict__ ent2, int32_t b, int32_t e, const float *fs,
+                                              const int32_t *__restrict__ col_slot, const float *__restrict__ B,
+                                              int64_t ldb, int lane, int o1, int o2, int o3, float4 &s) {
+    for (int32_t k0 = b + lane; k0 < e; k0 += 32 * kNarrowRounds) {
+        int2 en[kNarrowRounds];
+        int32_t slot[kNarrowRounds];
+        float4 v[kNarrowRounds];
+#pragma unroll
+        for (int u = 0; u < kNarrowRounds; ++u)
+            en[u] = k0 + 32 * u < e ? __ldg(ent2 + k0 + 32 * u) : make_int2(0, 0);
+#pragma unroll
+        for (int u = 0; u < kNarrowRounds; ++u)
+            slot[u] = k0 + 32 * u < e ? __ldg(col_slot + entry_col(en[u].x)) : -1;
+#pragma unroll
+        for (int u = 0; u < kNarrowRounds; ++u) {
+            v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (slot[u] >= 0) {
+                const float *row = B + (int64_t)slot[u] * ldb;
+                if (VEC) {
+                    v[u] = __ldg(reinterpret_cast<const float4 *>(row));
+                } else {
+                    v[u].x = __ldg(row);
+                    v[u].y = __ldg(row + o1);
+                    v[u].z = __ldg(row + o2);
+                    v[u].w = __ldg(row + o3);
+                }
+            }
+        }
+#pragma unroll
+        for (int u = 0; u < kNarrowRounds; ++u) {
+            if (slot[u] >= 0) {
+                const float w = fs[entry_step(en[u].x)] * __int_as_float(en[u].y);
+                s.x = fmaf(w, v[u].x, s.x);
+                s.y = fmaf(w, v[u].y, s.y);
+                s.z = fmaf(w, v[u].z, s.z);
+                s.w = fmaf(w, v[u].w, s.w);
+            }
+        }
+    }
+}
+
 template <bool VEC>
 __global__ void __launch_bounds__(kQfWarps * 32) row_project_narrow_kernel(
     const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
@@ -222,42 +265,7 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_project_narrow_kernel(
         float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
         if (a >= 0 && a < n_rows) {   // rows outside this shard stay +0
             const int32_t b = __ldg(ptr + a * L), e = __ldg(ptr + (a + 1) * L);
-            for (int32_t k0 = b + lane; k0 < e; k0 += 32 * kNarrowRounds) {
-                int2 en[kNarrowRounds];
-                int32_t slot[kNarrowRounds];
-                float4 v[kNarrowRounds];
-#pragma unroll
-                for (int u = 0; u < kNarrowRounds; ++u)
-                    en[u] = k0 + 32 * u < e ? __ldg(ent2 + k0 + 32 * u) : make_int2(0, 0);
-#pragma unroll
-                for (int u = 0; u < kNarrowRounds; ++u)
-                    slot[u] = k0 + 32 * u < e ? __ldg(col_slot + entry_col(en[u].x)) : -1;
-#pragma unroll
-                for (int u = 0; u < kNarrowRounds; ++u) {
-                    v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (slot[u] >= 0) {
-                        const float *row = B + (int64_t)slot[u] * ldb;
-                        if (VEC) {
-                            v[u] = __ldg(reinterpret_cast<const float4 *>(row));
-                        } else {
-                            v[u].x = __ldg(row);
-                            v[u].y = __ldg(row + o1);
-                            v[u].z = __ldg(row + o2);
-                            v[u].w = __ldg(row + o3);
-                        }
-                    }
-                }
-#pragma unroll
-                for (int u = 0; u < kNarrowRounds; ++u) {
-                    if (slot[u] >= 0) {
-                        const float w = fs[entry_step(en[u].x)] * __int_as_float(en[u].y);
-                        s.x = fmaf(w, v[u].x, s.x);
-                        s.y = fmaf(w, v[u].y, s.y);
-                        s.z = fmaf(w, v[u].z, s.z);
-                        s.w = fmaf(w, v[u].w, s.w);
-                    }
-                }
-            }
+            pj_narrow_row<VEC>(ent2, b, e, fs, col_slot, B, ldb, lane, o1, o2, o3, s);
         }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
@@ -312,6 +320,36 @@ __device__ __forceinline__ void pj_gather_groups(const QfPair *buf, int cnt, int
     }
 }
 
+// the group's share of the mid sums over the entries [b, e) of one row: compaction, then the gathers (re-streamed
+// in buffer loads when the row has more touched entries than the buffer)
+template <bool VEC>
+__device__ __forceinline__ void pj_mid_row(const int2 *__restrict__ ent2, int32_t b, int32_t e, const float *fs,
+                                           const int32_t *__restrict__ col_slot, QfPair *buf, int grp, int step,
+                                           const float *__restrict__ B, int64_t ldb, int32_t c, int32_t r, int lane,
+                                           double &unused, float4 &s) {
+    int cnt = 0;
+    for (int32_t k0 = b; k0 < e; k0 += 32)
+        cnt += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, cnt, lane, unused);
+    __syncwarp();
+    if (cnt <= kQfCap) {
+        pj_gather_groups<VEC>(buf, cnt, grp, step, B, ldb, c, r, s);
+    } else {
+        int part = 0;
+        for (int32_t k0 = b; k0 < e; k0 += 32) {
+            if (part + 32 > kQfCap) {
+                __syncwarp();
+                pj_gather_groups<VEC>(buf, part, grp, step, B, ldb, c, r, s);
+                __syncwarp();
+                part = 0;
+            }
+            part += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, part, lane, unused);
+        }
+        __syncwarp();
+        pj_gather_groups<VEC>(buf, part, grp, step, B, ldb, c, r, s);
+    }
+    __syncwarp();   // the buffer is reused by the next row
+}
+
 // 4 < r <= 64: the warp is 32 / Q entry groups x Q column quads (Q the next power of two >= r / 4).  The touched
 // pairs are compacted as in row_quadform_kernel, each group gathers its share, the groups are added with a fixed
 // xor tree and group 0 stores.  Rows with more touched entries than the buffer re-stream in buffer loads.
@@ -338,27 +376,7 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_project_mid_kernel(
         float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
         if (a >= 0 && a < n_rows) {   // rows outside this shard stay +0
             const int32_t b = __ldg(ptr + a * L), e = __ldg(ptr + (a + 1) * L);
-            int cnt = 0;
-            for (int32_t k0 = b; k0 < e; k0 += 32)
-                cnt += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, cnt, lane, unused);
-            __syncwarp();
-            if (cnt <= kQfCap) {
-                pj_gather_groups<VEC>(buf, cnt, grp, step, B, ldb, c, r, s);
-            } else {
-                int part = 0;
-                for (int32_t k0 = b; k0 < e; k0 += 32) {
-                    if (part + 32 > kQfCap) {
-                        __syncwarp();
-                        pj_gather_groups<VEC>(buf, part, grp, step, B, ldb, c, r, s);
-                        __syncwarp();
-                        part = 0;
-                    }
-                    part += qf_compact<false>(ent2, k0, e, fs, col_slot, buf, part, lane, unused);
-                }
-                __syncwarp();
-                pj_gather_groups<VEC>(buf, part, grp, step, B, ldb, c, r, s);
-            }
-            __syncwarp();   // the buffer is reused by the next row
+            pj_mid_row<VEC>(ent2, b, e, fs, col_slot, buf, grp, step, B, ldb, c, r, lane, unused, s);
         }
         for (int o = 16; o >= (1 << qlog); o >>= 1) {
             s.x += __shfl_xor_sync(0xffffffffu, s.x, o);
@@ -420,6 +438,127 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_project_kernel(
             pj_store(o, c, r, s, vec_out);
         }
         __syncwarp();   // the buffer is reused by the next row
+    }
+}
+
+// ---- rank-k conditioning of the variance (and mean) at fixed candidate rows ---------------------------------------
+// After the posterior gains b training rows, C gains b columns and a changes (grf_b200/posterior.py, condition_on);
+// the variance at a candidate only drops by the squares of its projection onto the new columns.  With k = r +
+// with_mean columns of B = [C_new | a]:
+//     p_c(i) = sum_{e in row x[i], slot >= 0} w_e B[slot(e), c],   q[i] += sum_{c < r} p_c(i)^2   (float64, c = 0, 1, ..),
+//     var[i] = max((float)(d[i] - q[i]), +0) (NaN stays NaN),       mean[i] = p_r(i).
+// The sums p are those of the projection shapes (narrow for k <= 4, mid for k <= 64), in the same order; lane 0
+// then adds the squares to q in column order, so repeated calls agree bit for bit.  Ids outside the shard have
+// p = 0: q is left as it is, var is still written.
+
+// lane 0: q += s_c^2 for the columns c .. c + 3 below r, and the mean from column r when it is one of them
+__device__ __forceinline__ void rc_add(double &qv, float &mv, const float4 &s, int32_t c, int32_t r) {
+    const float v[4] = {s.x, s.y, s.z, s.w};
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+        if (c + u < r) qv += (double)v[u] * (double)v[u];
+        else if (c + u == r) mv = v[u];
+    }
+}
+
+__device__ __forceinline__ float rc_var(float d, double q) {
+    const float v = (float)((double)d - q);
+    return v > 0.f || v != v ? v : 0.f;   // clamped at +0; NaN propagates as in torch.clamp_min
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_condition_narrow_kernel(
+    const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
+    const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows, const int32_t *__restrict__ col_slot,
+    const float *__restrict__ B, int64_t ldb, int32_t k, int32_t r, double *__restrict__ q,
+    const float *__restrict__ d, float *__restrict__ var, float *__restrict__ mean) {
+    __shared__ float fs[kMaxSteps];
+    if (threadIdx.x < kMaxSteps) fs[threadIdx.x] = threadIdx.x < L ? __ldg(f + threadIdx.x) : 0.f;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int2 *ent2 = reinterpret_cast<const int2 *>(ent);
+    const int o1 = min(1, k - 1), o2 = min(2, k - 1), o3 = min(3, k - 1);
+    for (int64_t i = warp0; i < n; i += n_warps) {
+        const int64_t a = (x ? (int64_t)__ldg(x + i) : i + row_lo) - row_lo;
+        const bool inside = a >= 0 && a < n_rows;
+        float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (inside) {
+            const int32_t b = __ldg(ptr + a * L), e = __ldg(ptr + (a + 1) * L);
+            pj_narrow_row<VEC>(ent2, b, e, fs, col_slot, B, ldb, lane, o1, o2, o3, s);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            s.x += __shfl_xor_sync(0xffffffffu, s.x, o);
+            s.y += __shfl_xor_sync(0xffffffffu, s.y, o);
+            s.z += __shfl_xor_sync(0xffffffffu, s.z, o);
+            s.w += __shfl_xor_sync(0xffffffffu, s.w, o);
+        }
+        if (lane == 0) {
+            double qv = q[i];
+            float mv = 0.f;
+            if (inside) {
+                rc_add(qv, mv, s, 0, r);
+                q[i] = qv;
+            }
+            var[i] = rc_var(__ldg(d + i), qv);
+            if (mean) mean[i] = mv;
+        }
+    }
+}
+
+// 4 < k <= 64: the groups x quads of row_project_mid_kernel; after the group tree, lane 0 collects the quads of
+// group 0 in column order
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_condition_mid_kernel(
+    const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
+    const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows, const int32_t *__restrict__ col_slot,
+    const float *__restrict__ B, int64_t ldb, int32_t k, int32_t r, double *__restrict__ q,
+    const float *__restrict__ d, float *__restrict__ var, float *__restrict__ mean, int32_t qlog) {
+    __shared__ float fs[kMaxSteps];
+    __shared__ QfPair sbuf[kQfWarps][kQfCap];
+    if (threadIdx.x < kMaxSteps) fs[threadIdx.x] = threadIdx.x < L ? __ldg(f + threadIdx.x) : 0.f;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int grp = lane >> qlog, step = 32 >> qlog;
+    const int32_t c = 4 * (lane & ((1 << qlog) - 1));
+    const int nq = (k + 3) / 4;
+    QfPair *buf = sbuf[threadIdx.x >> 5];
+    const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int2 *ent2 = reinterpret_cast<const int2 *>(ent);
+    double unused = 0.0;
+    for (int64_t i = warp0; i < n; i += n_warps) {
+        const int64_t a = (x ? (int64_t)__ldg(x + i) : i + row_lo) - row_lo;
+        const bool inside = a >= 0 && a < n_rows;
+        float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (inside) {
+            const int32_t b = __ldg(ptr + a * L), e = __ldg(ptr + (a + 1) * L);
+            pj_mid_row<VEC>(ent2, b, e, fs, col_slot, buf, grp, step, B, ldb, c, k, lane, unused, s);
+        }
+        for (int o = 16; o >= (1 << qlog); o >>= 1) {
+            s.x += __shfl_xor_sync(0xffffffffu, s.x, o);
+            s.y += __shfl_xor_sync(0xffffffffu, s.y, o);
+            s.z += __shfl_xor_sync(0xffffffffu, s.z, o);
+            s.w += __shfl_xor_sync(0xffffffffu, s.w, o);
+        }
+        double qv = lane == 0 ? q[i] : 0.0;
+        float mv = 0.f;
+#pragma unroll 1
+        for (int j = 0; j < nq; ++j) {   // quad j of group 0 sits in lane j
+            float4 t;
+            t.x = __shfl_sync(0xffffffffu, s.x, j);
+            t.y = __shfl_sync(0xffffffffu, s.y, j);
+            t.z = __shfl_sync(0xffffffffu, s.z, j);
+            t.w = __shfl_sync(0xffffffffu, s.w, j);
+            if (inside) rc_add(qv, mv, t, 4 * j, r);
+        }
+        if (lane == 0) {
+            if (inside) q[i] = qv;
+            var[i] = rc_var(__ldg(d + i), qv);
+            if (mean) mean[i] = mv;
+        }
     }
 }
 
@@ -499,4 +638,49 @@ extern "C" int grf_phi_row_project(const GrfPhi *phi, const float *f, const int3
         row_project_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows, col_slot, B,
                                                           ldb, r, out, ldo, vout);
     return check_cuda(cudaGetLastError(), "row_project_kernel launch");
+}
+
+extern "C" int grf_phi_row_condition(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n,
+                                     const int32_t *col_slot, const float *B, int64_t ldb, int32_t r,
+                                     int32_t with_mean, double *q, const float *d, float *var, float *mean,
+                                     void *stream) {
+    GRF_ON_STREAM_DEVICE(stream, var);
+    GRF_REQUIRE(phi && f && col_slot && B && q && d && var && (mean || !with_mean),
+                "grf_phi_row_condition: null argument");
+    GRF_REQUIRE(with_mean == 0 || with_mean == 1, "grf_phi_row_condition: with_mean must be 0 or 1");
+    const int64_t k = (int64_t)r + with_mean;
+    GRF_REQUIRE(n >= 0 && r >= 0 && k >= 1 && k <= 64 && ldb >= k,
+                "grf_phi_row_condition: bad n / r / ldb (needs 1 <= r + with_mean <= 64 and ldb >= r + with_mean)");
+    GRF_REQUIRE(phi->n_steps >= 1 && phi->n_steps <= kMaxSteps, "grf_phi_row_condition: n_steps out of range");
+    GRF_REQUIRE(x || n == phi->n_rows, "grf_phi_row_condition: n must equal n_rows when x is NULL");
+    GRF_REQUIRE(phi->blk_ptr, "grf_phi_row_condition: Phi blocks missing");
+    if (n == 0) return GRF_OK;
+    const bool vin = ldb % 4 == 0 && ((uintptr_t)B & 15u) == 0;
+    int64_t g = (n + kQfWarps - 1) / kQfWarps;
+    if (g > (int64_t)kSmCount * 16) g = (int64_t)kSmCount * 16;
+    const dim3 grid((unsigned)g), block(kQfWarps * 32);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int32_t *ptr = phi->blk_ptr;
+    const GrfEntry *ent = phi->entries;
+    const int32_t L = phi->n_steps, kk = (int32_t)k;
+    float *mo = with_mean ? mean : nullptr;
+    if (k <= 4) {
+        if (vin)
+            row_condition_narrow_kernel<true><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
+                                                                      col_slot, B, ldb, kk, r, q, d, var, mo);
+        else
+            row_condition_narrow_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo,
+                                                                       phi->n_rows, col_slot, B, ldb, kk, r, q, d,
+                                                                       var, mo);
+        return check_cuda(cudaGetLastError(), "row_condition_narrow_kernel launch");
+    }
+    int qlog = 1;                             // quads: the next power of two >= ceil(k / 4), 2 .. 16
+    while ((4 << qlog) < k) ++qlog;
+    if (vin)
+        row_condition_mid_kernel<true><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
+                                                               col_slot, B, ldb, kk, r, q, d, var, mo, qlog);
+    else
+        row_condition_mid_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
+                                                                col_slot, B, ldb, kk, r, q, d, var, mo, qlog);
+    return check_cuda(cudaGetLastError(), "row_condition_mid_kernel launch");
 }

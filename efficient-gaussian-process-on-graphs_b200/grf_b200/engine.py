@@ -1211,6 +1211,46 @@ class PhiBlocks:
                                              ldb, r, _ptr(out), ldo, _stream(dev)))
         return out
 
+    def row_condition(self, f, x, col_slot, B, r: int, with_mean: bool, q, d, var, mean=None) -> None:
+        """In place, with p = the projection of ``row_project`` onto columns [0, r + with_mean) of B:
+        q[i] += sum_{c < r} p[i, c]^2 (float64), var[i] = max(d[i] - q[i], 0) (float32; NaN stays NaN) and, with
+        ``with_mean``, mean[i] = p[i, r] (``grf_phi_row_condition``).  q: float64 [n], d, var and mean: float32 [n],
+        contiguous, on Phi's device.  B: float32 [m, >= r + with_mean] (a column slice of a wider buffer is read in
+        place; any other layout is copied); ValueError when col_slot names a row past m, or for 1 <= r + with_mean
+        <= 64 not holding.  x = None: every local row.  See grf_b200/posterior.py, PosteriorMarginals."""
+        dev = self.device
+        f = self._f(f)
+        xi = self._ids(x, dev)
+        n = self.n_rows if xi is None else xi.numel()
+        r, wm = int(r), int(bool(with_mean))
+        k = r + wm
+        if not 1 <= k <= 64 or r < 0:
+            raise ValueError(f"row_condition: r + with_mean must be in [1, 64], got r = {r}, with_mean = {wm}")
+        col_slot = torch.as_tensor(col_slot, device=dev).to(torch.int32).contiguous()
+        if col_slot.numel() != self.n_cols:
+            raise ValueError(f"row_condition: col_slot has {col_slot.numel()} entries, Phi has {self.n_cols} columns")
+        if B.dim() != 2 or B.dtype != torch.float32 or B.device != dev or B.shape[1] < k:
+            raise ValueError(f"row_condition: B must be a 2-D float32 tensor on Phi's device with at least {k} "
+                             "columns")
+        if (k > 1 and B.stride(1) != 1) or (B.shape[0] > 1 and B.stride(0) < k):
+            B = B[:, :k].contiguous()      # the kernel reads rows of k floats ldb apart
+        ldb = int(B.stride(0)) if B.shape[0] > 1 else int(B.shape[1])
+        for name, t, dt in (("q", q, torch.float64), ("d", d, torch.float32), ("var", var, torch.float32)) + \
+                (("mean", mean, torch.float32),) * wm:
+            if (t is None or t.dtype != dt or t.device != dev or t.numel() != n or t.dim() != 1
+                    or (n > 1 and t.stride(0) != 1)):
+                raise ValueError(f"row_condition: {name} must be a contiguous {dt} [{n}] tensor on Phi's device")
+        if n == 0:
+            return
+        if col_slot.numel() and int(col_slot.max()) >= B.shape[0]:
+            raise ValueError(f"row_condition: col_slot names row {int(col_slot.max())} of B, which has "
+                             f"{B.shape[0]} rows")
+        keep = B if B.numel() else torch.zeros(k, dtype=torch.float32, device=dev)   # no row of B is read then
+        phi = self.c_struct()
+        check(_lib.lib().grf_phi_row_condition(ctypes.byref(phi), _ptr(f), _ptr(xi), n, _ptr(col_slot), _ptr(keep),
+                                               ldb, r, wm, _ptr(q), _ptr(d), _ptr(var),
+                                               _ptr(mean) if wm else None, _stream(dev)))
+
     def training_gram(self, x, mem_limit: Optional[int] = None) -> torch.Tensor:
         """E[l, i, l', j] = <M_l[x_i], M_l'[x_j]>, float64 [L, n, L, n]: the per-length Gram of the training rows, so
         that K(f) = sum_{l, l'} f_l f_l' E[l, :, l', :] for every modulator f (grf_b200/mll.py fits f and sigma^2 on

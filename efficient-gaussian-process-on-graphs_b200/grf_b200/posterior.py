@@ -27,6 +27,11 @@ of the posterior is the projection S* B = [s_i . B[:, c]] for a dense B (``grf_p
 
 the samples being pathwise conditioning (``SparseGraphGP.predict``) with an exact solve: eps ~ N(0, I_N) and
 E ~ N(0, I_n) per sample, L^-1 V a float64 triangular solve and B a float32 GEMM.
+
+Between refits of f and sigma^2 a BO loop only appends observations: ``condition_on`` extends L and C by block
+Cholesky (C keeps its old columns and gains b), and ``PosteriorMarginals`` keeps the mean and variance at a fixed
+candidate set current with one pass over the candidate rows per update (``grf_phi_row_condition``: q grows by the
+squares of the projections onto the new columns of C, the mean is the projection onto the new a).
 """
 
 from __future__ import annotations
@@ -39,6 +44,22 @@ from .engine import PhiBlocks
 from .kernel_matrix import _free_bytes
 
 
+def _condition_chunk(n: int, m: int) -> int:
+    """Rows of C_old converted to float64 at a time by condition_on: 256 MiB of them."""
+    return max(1, min(m, (1 << 28) // (8 * max(n, 1))))
+
+
+def condition_bytes(n: int, b: int, m: int, nnz_old: int) -> int:
+    """Device bytes ExactPosterior.condition_on allocates to append b rows to n rows (nnz_old entries of Phi_f)
+    that touch m columns afterwards: the new C (float32, ldc = round_up(n + b, 4)) and L (float64), G_new^T (float64
+    [b, m]), one float64 row chunk of C_old and its product, and the K_21 products (two float64 [entries, b]
+    buffers over at most the nnz_old old entries)."""
+    nb = n + b
+    ldc = (nb + 3) // 4 * 4
+    chunk = _condition_chunk(n, m)
+    return 4 * m * ldc + 8 * nb * nb + 8 * b * m + 8 * chunk * (n + 2 * b) + 16 * nnz_old * b
+
+
 class ExactPosterior:
     """The training-side cache (slots, L, C and, with ``y_train``, a = G K^-1 y) of the exact posterior, built once
     per (Phi, f, x, sigma^2, y).
@@ -47,7 +68,9 @@ class ExactPosterior:
     MemoryError (naming the bytes) is raised before they are allocated when they do not fit.  ``events``: CUDA
     events recorded at the stage boundaries ("start", "merge", "slots", "G", "gram", "cholesky", "solve";
     ``variance`` adds "quadform_start" and "quadform"; every projection, of ``mean``, ``covariance`` and ``sample``,
-    "project_start" and "project"; ``sample`` also "sample_start", "prior", "triangular" and "gemm")."""
+    "project_start" and "project"; ``sample`` also "sample_start", "prior", "triangular" and "gemm";
+    ``condition_on`` "condition_start", "cross", "factor", "append" and "weights"; a PosteriorMarginals refresh
+    "refresh_start" and "refresh")."""
 
     def __init__(self, blocks: PhiBlocks, f, x_train, noise, mem_limit: Optional[int] = None,
                  events: Optional[Dict[str, torch.cuda.Event]] = None, *, y_train=None):
@@ -73,18 +96,9 @@ class ExactPosterior:
             self._mark("start")
             self.phi_f = blocks.merged(f)                 # Phi_f: one length, one entry per (row, col)
             self._mark("merge")
-            ptr = self.phi_f.blk_ptr.to(torch.int64)
-            ent = self.phi_f.entries
-            xl = x.to(torch.int64)
-            start = ptr[xl]
-            lens = ptr[xl + 1] - start
-            total = int(lens.sum().item()) if n else 0
+            j, cols, vals = self._gather(x)
+            total = int(j.numel())
             self.nnz_train = total
-            j = torch.repeat_interleave(torch.arange(n, device=dev), lens, output_size=total)
-            first = torch.cumsum(lens, 0) - lens
-            idx = start[j] + torch.arange(total, device=dev) - first[j]
-            cols = ent[idx, 0].to(torch.int64)           # length 0: the packed word is the column
-            vals = ent[idx, 1].view(torch.float32)
             cols_s = torch.unique(cols)                  # S, ascending
             m = int(cols_s.numel())
             self.m = m
@@ -101,7 +115,7 @@ class ExactPosterior:
             gt = torch.zeros((n, m), dtype=torch.float64, device=dev)           # G^T
             if total:
                 gt[j, self.slot[cols].to(torch.int64)] = vals.to(torch.float64)
-            del j, first, idx, cols, vals
+            del j, cols, vals
             self._mark("G")
             k = gt @ gt.T
             k.diagonal().add_(noise)
@@ -124,6 +138,24 @@ class ExactPosterior:
             self.C[:, :n] = ct.T
             del ct
             self._mark("solve")
+        self.version = 0
+
+    def _gather(self, x):
+        """(row index j, column, value) of every entry of the rows x of the merged Phi_f, row by row in entry
+        order: int64, int64 and float32 device tensors."""
+        dev = self.device
+        ptr = self.phi_f.blk_ptr.to(torch.int64)
+        ent = self.phi_f.entries
+        xl = x.to(torch.int64)
+        start = ptr[xl]
+        lens = ptr[xl + 1] - start
+        total = int(lens.sum().item()) if xl.numel() else 0
+        j = torch.repeat_interleave(torch.arange(xl.numel(), device=dev), lens, output_size=total)
+        first = torch.cumsum(lens, 0) - lens
+        idx = start[j] + torch.arange(total, device=dev) - first[j]
+        cols = ent[idx, 0].to(torch.int64)           # length 0: the packed word is the column
+        vals = ent[idx, 1].view(torch.float32)
+        return j, cols, vals
 
     def _mark(self, name: str) -> None:
         if self.events is not None:
@@ -255,3 +287,186 @@ class ExactPosterior:
             if include_noise:
                 fs = fs + sigma * torch.randn((q, s), generator=generator, device=dev)
         return fs.T.contiguous()
+
+    def condition_on(self, x_new, y_new=None) -> "ExactPosterior":
+        """Append b training rows in place (f and sigma^2 stay): afterwards every method answers as a posterior
+        constructed on x + x_new (and y + y_new) does, within float32 round-off.  Returns self.
+
+        With K_21 = G_new^T G and K_22 = G_new^T G_new (float64 sums of the exact products of the gathered entries):
+            L_21 = (L_11^-1 K_21^T)^T,   L_22 = chol(K_22 + sigma^2 I - L_21 L_21^T),
+            C    = [C_old | C_new],      C_new = (G_new - C_old L_21^T) L_22^-T     (float64 in row chunks, stored
+                                                                                     as float32; ldc = round_up(n + b, 4))
+        and, with y, a = G K^-1 y from the new factor (float64).  Columns of the new rows outside S get the slots
+        m, m + 1, .. in ascending column order, so after a call the slots are no longer ascending over S (the
+        kernels do not care).  C and L are reallocated at their new size.
+
+        ``y_new`` is required exactly when the posterior has y (``y_new = mean(x_new)`` gives the "hallucinated"
+        conditioning of batch UCB selection).  Ids may repeat or be in x already.  An empty x_new is a no-op; each
+        call that adds rows increments ``version``.  IndexError for ids outside Phi; ValueError for a y_new of the
+        wrong length, or when the extended K is not positive definite in float64 (the posterior is then left as it
+        was); MemoryError (naming the bytes) before anything is allocated.  Events: "condition_start", "cross",
+        "factor", "append" and "weights"."""
+        dev, n = self.device, self.n
+        xn = self._test_ids(x_new)
+        b = int(xn.numel())
+        yn = None
+        if (y_new is None) != (self.y is None):
+            raise ValueError("ExactPosterior.condition_on: y_new is required exactly when the posterior has "
+                             "training targets")
+        if y_new is not None:
+            yn = torch.as_tensor(y_new, device=dev).detach().flatten().to(torch.float64)
+            if yn.numel() != b:
+                raise ValueError(f"ExactPosterior.condition_on: y_new has {yn.numel()} values for {b} new ids")
+        if b == 0:
+            return self
+        nb = n + b
+        with torch.cuda.device(dev):
+            self._mark("condition_start")
+            jn, cn, vn = self._gather(xn)
+            cols_n = torch.unique(cn)
+            fresh = cols_n[self.slot[cols_n] < 0]             # ascending
+            m0, m1 = self.m, self.m + int(fresh.numel())
+            ldc = (nb + 3) // 4 * 4
+            chunk = _condition_chunk(n, m1)
+            need = condition_bytes(n, b, m1, self.nnz_train)
+            budget = _free_bytes(dev) if self.mem_limit is None else int(self.mem_limit)
+            if need > budget:
+                raise MemoryError(f"exact posterior condition_on: C and L of {nb} training rows touching {m1} "
+                                  f"columns need {need} bytes, {budget} bytes of device memory are free")
+            slot = self.slot.clone()
+            slot[fresh] = torch.arange(m0, m1, dtype=torch.int32, device=dev)
+            sn = slot[cn].to(torch.int64)
+            gnt = torch.zeros((b, m1), dtype=torch.float64, device=dev)            # G_new^T
+            gnt[jn, sn] = vn.to(torch.float64)
+            k22 = gnt @ gnt.T
+            k21 = torch.zeros((b, n), dtype=torch.float64, device=dev)
+            if n:                       # K_21[:, j] = sum over the entries of old row j of val * G_new^T[:, slot]
+                jo, co, vo = self._gather(self.x)
+                so = slot[co].to(torch.int64)
+                hit = torch.zeros(m1, dtype=torch.bool, device=dev)
+                hit[sn] = True
+                keep = hit[so]
+                jo, so, vo = jo[keep], so[keep], vo[keep]
+                prod = gnt[:, so].T * vo.to(torch.float64)[:, None]             # exact products, [entries, b]
+                k21 = torch.segment_reduce(prod, "sum", lengths=torch.bincount(jo, minlength=n), axis=0).T
+                del jo, co, vo, so, keep, hit, prod
+            self._mark("cross")
+            l21t = torch.linalg.solve_triangular(self.L, k21.T, upper=False) if n else k21.T   # L_21^T, [n, b]
+            s22 = k22 - l21t.T @ l21t
+            s22.diagonal().add_(self.noise)
+            l22, info = torch.linalg.cholesky_ex(s22)
+            if int(info.item()) > 0:
+                raise ValueError(f"exact posterior: G^T G + sigma^2 I is not positive definite in float64 "
+                                 f"(sigma^2 = {self.noise}, n = {nb}, leading minor {n + int(info.item())})")
+            del k21, k22, s22
+            self._mark("factor")
+            C = torch.zeros((m1, ldc), dtype=torch.float32, device=dev)
+            C[:m0, :n] = self.C[:, :n]
+            for r0 in range(0, m1, chunk):                   # C_new = (G_new - C_old L_21^T) L_22^-T, by rows
+                r1 = min(m1, r0 + chunk)
+                t = gnt[:, r0:r1].T.contiguous()
+                if n and r0 < m0:
+                    t[:min(r1, m0) - r0] -= self.C[r0:min(r1, m0), :n].to(torch.float64) @ l21t
+                C[r0:r1, n:nb] = torch.linalg.solve_triangular(l22.T, t, upper=True, left=False).to(torch.float32)
+                del t
+            L = torch.zeros((nb, nb), dtype=torch.float64, device=dev)
+            L[:n, :n] = self.L
+            L[n:, :n] = l21t.T
+            L[n:, n:] = l22
+            del l21t, l22
+            self._mark("append")
+            x_all = torch.cat([self.x, xn])
+            a = None
+            if yn is not None:                               # a = G K^-1 y, float64 sums over slot-sorted entries
+                y = torch.cat([self.y, yn])
+                alpha = torch.cholesky_solve(y[:, None], L)[:, 0]
+                ja, ca, va = self._gather(x_all)
+                sa = slot[ca].to(torch.int64)
+                order = torch.argsort(sa * nb + ja)
+                contrib = (va.to(torch.float64) * alpha[ja])[order]
+                a = torch.segment_reduce(contrib, "sum", lengths=torch.bincount(sa, minlength=m1), axis=0)
+                a = a.to(torch.float32)[:, None]
+                del alpha, ja, ca, va, sa, order, contrib
+            # nothing above changed the posterior (a failed factor leaves it as it was); now it takes the new state
+            self.slot, self.m, self.C, self.L, self.ldc = slot, m1, C, L, ldc
+            self.x, self.n = x_all, nb
+            self.nnz_train += int(jn.numel())
+            if yn is not None:
+                self.y, self.a = y, a
+            self.version += 1
+            self._mark("weights")
+        return self
+
+    def marginals(self, x_cand) -> "PosteriorMarginals":
+        """The mean and variance at a fixed candidate set, kept current across ``condition_on`` calls at the cost
+        of one pass over the candidate rows per refresh (see PosteriorMarginals).  IndexError for ids outside Phi."""
+        return PosteriorMarginals(self, x_cand)
+
+
+class PosteriorMarginals:
+    """Mean and variance of an ExactPosterior at fixed candidate ids, brought up to date after the posterior is
+    conditioned on new rows without redoing the pass over all n columns of C.
+
+    It keeps d (float32) and q (float64) of var = max(d - q, 0).  After ``condition_on`` appended k = n - n_seen
+    columns to C, ``refresh`` adds the squares of the candidates' projections onto those columns to q and recomputes
+    the mean from the new a:
+      k + with_mean <= 64   one ``row_condition`` pass with B = [C[:, n_seen:n] | a] (a copied into the last
+                            column of an m x (k + 1) buffer)
+      k + with_mean > 64    ``row_quadform`` on C[:, n_seen:n] (q rounded to float32 once) plus one ``row_project``
+                            onto a
+    ``mean`` and ``variance`` refresh when the posterior has changed since the last refresh."""
+
+    def __init__(self, post: ExactPosterior, x_cand):
+        self.post = post
+        self.x = post._test_ids(x_cand)
+        dev = post.device
+        with torch.cuda.device(dev):
+            q, self.d = post.phi_f.row_quadform(torch.ones(1, device=dev), self.x, post.slot, post.C[:, :post.n])
+            self.q = q.to(torch.float64)
+            self._var = torch.clamp_min(self.d - q, 0.0)      # = post.variance(x_cand)
+            self._mean = post._project(self.x, post.a)[:, 0].contiguous() if post.y is not None else None
+        self.version, self.n_seen = post.version, post.n
+
+    @property
+    def stale(self) -> bool:
+        return self.version != self.post.version
+
+    def refresh(self) -> "PosteriorMarginals":
+        """Bring q, the variance and the mean up to date with the posterior (a no-op when it is current)."""
+        post = self.post
+        if not self.stale:
+            return self
+        dev, n0, n = post.device, self.n_seen, post.n
+        k, wm = n - n0, post.y is not None
+        one = torch.ones(1, device=dev)
+        with torch.cuda.device(dev):
+            post._mark("refresh_start")
+            if k + wm <= 64:
+                B = torch.empty((post.m, k + wm), dtype=torch.float32, device=dev)
+                B[:, :k] = post.C[:, n0:n]
+                if wm:
+                    B[:, k] = post.a[:, 0]
+                post.phi_f.row_condition(one, self.x, post.slot, B, k, wm, self.q, self.d, self._var,
+                                         self._mean if wm else None)
+            else:
+                dq, _ = post.phi_f.row_quadform(one, self.x, post.slot, post.C[:, n0:n])
+                self.q += dq.to(torch.float64)
+                self._var = torch.clamp_min((self.d.to(torch.float64) - self.q).to(torch.float32), 0.0)
+                if wm:
+                    self._mean = post.phi_f.row_project(one, self.x, post.slot, post.a)[:, 0].contiguous()
+            post._mark("refresh")
+        self.version, self.n_seen = post.version, n
+        return self
+
+    @property
+    def mean(self) -> torch.Tensor:
+        """Posterior mean at the candidates (float32 [len(x_cand)]); ValueError without training targets."""
+        self.post._need_y("mean")
+        return self.refresh()._mean.clone()
+
+    def variance(self, include_noise: bool = False) -> torch.Tensor:
+        """Posterior variance at the candidates (float32 [len(x_cand)]); ``include_noise`` adds sigma^2."""
+        var = self.refresh()._var.clone()
+        if include_noise:
+            var = var + torch.tensor(self.post.noise, dtype=torch.float32, device=self.post.device)
+        return var

@@ -521,6 +521,24 @@ int grf_phi_row_quadform(const GrfPhi *phi, const float *f, const int32_t *x, in
 int grf_phi_row_project(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n, const int32_t *col_slot,
                         const float *B, int64_t ldb, int32_t r, float *out, int64_t ldo, void *stream);
 
+/* Rank-k update of the posterior variance (and mean) at fixed test rows after the training set grew
+ * (csrc/grf_posterior.cu; grf_b200/posterior.py, ExactPosterior.condition_on and PosteriorMarginals).  With
+ * w_e = f[length(e)] * e.val and p_c(i) = sum_{e in row x[i], col_slot[col(e)] >= 0} w_e * B[col_slot[col(e)] * ldb + c]:
+ *   q[i]   += sum_{c < r} p_c(i)^2        (the squares in float64, added to q[i] in the order c = 0, 1, ..)
+ *   var[i]  = (float)(d[i] - q[i]) with the updated q, clamped at +0 (NaN stays NaN, as torch.clamp_min)
+ *   mean[i] = p_r(i)                      (only with with_mean = 1; mean may be NULL when with_mean = 0)
+ * k = r + with_mean columns of B [m][ldb] float32 are read, 1 <= k <= 64 and ldb >= k; columns [k, ldb) never
+ * reach a result.  B = [C_new | a]: the columns C gained and the new a = G K^-1 y.  q double[n], d float[n] (the
+ * prior variance, from grf_phi_row_quadform), var and mean float[n].  col_slot, x and the row shard as for
+ * grf_phi_row_project: ids outside [row_lo, row_lo + n_rows) have p = 0, so q stays as it is, var is still written
+ * from d and q and mean is +0.  Only elements [0, n) are written; the summation order is fixed (no atomics), so
+ * repeated calls agree bit for bit.  k <= 4 runs row_condition_narrow_kernel, k <= 64 row_condition_mid_kernel (the
+ * warp shapes of the projection).  -1 for k outside [1, 64], ldb < k, a NULL required pointer, or x NULL with
+ * n != n_rows. */
+int grf_phi_row_condition(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n, const int32_t *col_slot,
+                          const float *B, int64_t ldb, int32_t r, int32_t with_mean, double *q, const float *d,
+                          float *var, float *mean, void *stream);
+
 /* Per-length Gram of the training rows, light part (csrc/grf_gram.cu; no reference counterpart: the reference
  * estimates the marginal likelihood by CG and probes).  With A[R, c] = M_l[x_i, c] for the E row R = l * n + i,
  * E = A A^T is float64 [n_rows][lde], n_rows = L * n.  The columns the training rows touch are numbered as slots

@@ -451,13 +451,19 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_project_kernel(
 // then adds the squares to q in column order, so repeated calls agree bit for bit.  Ids outside the shard have
 // p = 0: q is left as it is, var is still written.
 
-// lane 0: q += s_c^2 for the columns c .. c + 3 below r, and the mean from column r when it is one of them
+// lane 0: q += s_c^2 (DOWN: q -= s_c^2) for the columns c .. c + 3 below r, and the mean from column r when it is
+// one of them
+template <bool DOWN>
 __device__ __forceinline__ void rc_add(double &qv, float &mv, const float4 &s, int32_t c, int32_t r) {
     const float v[4] = {s.x, s.y, s.z, s.w};
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
-        if (c + u < r) qv += (double)v[u] * (double)v[u];
-        else if (c + u == r) mv = v[u];
+        if (c + u < r) {
+            if (DOWN) qv -= (double)v[u] * (double)v[u];
+            else qv += (double)v[u] * (double)v[u];
+        } else if (c + u == r) {
+            mv = v[u];
+        }
     }
 }
 
@@ -466,8 +472,8 @@ __device__ __forceinline__ float rc_var(float d, double q) {
     return v > 0.f || v != v ? v : 0.f;   // clamped at +0; NaN propagates as in torch.clamp_min
 }
 
-template <bool VEC>
-__global__ void __launch_bounds__(kQfWarps * 32) row_condition_narrow_kernel(
+template <bool VEC, bool DOWN>
+__device__ __forceinline__ void rc_narrow(
     const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
     const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows, const int32_t *__restrict__ col_slot,
     const float *__restrict__ B, int64_t ldb, int32_t k, int32_t r, double *__restrict__ q,
@@ -499,7 +505,7 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_condition_narrow_kernel(
             double qv = q[i];
             float mv = 0.f;
             if (inside) {
-                rc_add(qv, mv, s, 0, r);
+                rc_add<DOWN>(qv, mv, s, 0, r);
                 q[i] = qv;
             }
             var[i] = rc_var(__ldg(d + i), qv);
@@ -510,8 +516,8 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_condition_narrow_kernel(
 
 // 4 < k <= 64: the groups x quads of row_project_mid_kernel; after the group tree, lane 0 collects the quads of
 // group 0 in column order
-template <bool VEC>
-__global__ void __launch_bounds__(kQfWarps * 32) row_condition_mid_kernel(
+template <bool VEC, bool DOWN>
+__device__ __forceinline__ void rc_mid(
     const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,
     const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows, const int32_t *__restrict__ col_slot,
     const float *__restrict__ B, int64_t ldb, int32_t k, int32_t r, double *__restrict__ q,
@@ -552,7 +558,7 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_condition_mid_kernel(
             t.y = __shfl_sync(0xffffffffu, s.y, j);
             t.z = __shfl_sync(0xffffffffu, s.z, j);
             t.w = __shfl_sync(0xffffffffu, s.w, j);
-            if (inside) rc_add(qv, mv, t, 4 * j, r);
+            if (inside) rc_add<DOWN>(qv, mv, t, 4 * j, r);
         }
         if (lane == 0) {
             if (inside) q[i] = qv;
@@ -561,6 +567,38 @@ __global__ void __launch_bounds__(kQfWarps * 32) row_condition_mid_kernel(
         }
     }
 }
+
+// The kernels: DOWN = false adds the squares (grf_phi_row_condition), DOWN = true subtracts them
+// (grf_phi_row_downdate).  Same bodies, so a downdate sums p in exactly the order of the condition pass.
+#define GRF_RC_ARGS                                                                                          \
+    const int32_t *__restrict__ ptr, const GrfEntry *__restrict__ ent, const float *__restrict__ f, int32_t L,     \
+        const int32_t *__restrict__ x, int64_t n, int64_t row_lo, int64_t n_rows,                                  \
+        const int32_t *__restrict__ col_slot, const float *__restrict__ B, int64_t ldb, int32_t k, int32_t r,      \
+        double *__restrict__ q, const float *__restrict__ d, float *__restrict__ var, float *__restrict__ mean
+#define GRF_RC_PASS ptr, ent, f, L, x, n, row_lo, n_rows, col_slot, B, ldb, k, r, q, d, var, mean
+
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_condition_narrow_kernel(GRF_RC_ARGS) {
+    rc_narrow<VEC, false>(GRF_RC_PASS);
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_downdate_narrow_kernel(GRF_RC_ARGS) {
+    rc_narrow<VEC, true>(GRF_RC_PASS);
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_condition_mid_kernel(GRF_RC_ARGS, int32_t qlog) {
+    rc_mid<VEC, false>(GRF_RC_PASS, qlog);
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(kQfWarps * 32) row_downdate_mid_kernel(GRF_RC_ARGS, int32_t qlog) {
+    rc_mid<VEC, true>(GRF_RC_PASS, qlog);
+}
+
+#undef GRF_RC_PASS
+#undef GRF_RC_ARGS
 
 }  // namespace
 }  // namespace grf
@@ -640,20 +678,20 @@ extern "C" int grf_phi_row_project(const GrfPhi *phi, const float *f, const int3
     return check_cuda(cudaGetLastError(), "row_project_kernel launch");
 }
 
-extern "C" int grf_phi_row_condition(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n,
-                                     const int32_t *col_slot, const float *B, int64_t ldb, int32_t r,
-                                     int32_t with_mean, double *q, const float *d, float *var, float *mean,
-                                     void *stream) {
+// grf_phi_row_condition (DOWN = false) and grf_phi_row_downdate (DOWN = true): the same arguments and rules
+template <bool DOWN>
+static int row_update(const char *name, const GrfPhi *phi, const float *f, const int32_t *x, int64_t n,
+                      const int32_t *col_slot, const float *B, int64_t ldb, int32_t r, int32_t with_mean, double *q,
+                      const float *d, float *var, float *mean, void *stream) {
     GRF_ON_STREAM_DEVICE(stream, var);
-    GRF_REQUIRE(phi && f && col_slot && B && q && d && var && (mean || !with_mean),
-                "grf_phi_row_condition: null argument");
-    GRF_REQUIRE(with_mean == 0 || with_mean == 1, "grf_phi_row_condition: with_mean must be 0 or 1");
+    GRF_REQUIRE(phi && f && col_slot && B && q && d && var && (mean || !with_mean), "%s: null argument", name);
+    GRF_REQUIRE(with_mean == 0 || with_mean == 1, "%s: with_mean must be 0 or 1", name);
     const int64_t k = (int64_t)r + with_mean;
     GRF_REQUIRE(n >= 0 && r >= 0 && k >= 1 && k <= 64 && ldb >= k,
-                "grf_phi_row_condition: bad n / r / ldb (needs 1 <= r + with_mean <= 64 and ldb >= r + with_mean)");
-    GRF_REQUIRE(phi->n_steps >= 1 && phi->n_steps <= kMaxSteps, "grf_phi_row_condition: n_steps out of range");
-    GRF_REQUIRE(x || n == phi->n_rows, "grf_phi_row_condition: n must equal n_rows when x is NULL");
-    GRF_REQUIRE(phi->blk_ptr, "grf_phi_row_condition: Phi blocks missing");
+                "%s: bad n / r / ldb (needs 1 <= r + with_mean <= 64 and ldb >= r + with_mean)", name);
+    GRF_REQUIRE(phi->n_steps >= 1 && phi->n_steps <= kMaxSteps, "%s: n_steps out of range", name);
+    GRF_REQUIRE(x || n == phi->n_rows, "%s: n must equal n_rows when x is NULL", name);
+    GRF_REQUIRE(phi->blk_ptr, "%s: Phi blocks missing", name);
     if (n == 0) return GRF_OK;
     const bool vin = ldb % 4 == 0 && ((uintptr_t)B & 15u) == 0;
     int64_t g = (n + kQfWarps - 1) / kQfWarps;
@@ -665,22 +703,34 @@ extern "C" int grf_phi_row_condition(const GrfPhi *phi, const float *f, const in
     const int32_t L = phi->n_steps, kk = (int32_t)k;
     float *mo = with_mean ? mean : nullptr;
     if (k <= 4) {
-        if (vin)
-            row_condition_narrow_kernel<true><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
-                                                                      col_slot, B, ldb, kk, r, q, d, var, mo);
-        else
-            row_condition_narrow_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo,
-                                                                       phi->n_rows, col_slot, B, ldb, kk, r, q, d,
-                                                                       var, mo);
-        return check_cuda(cudaGetLastError(), "row_condition_narrow_kernel launch");
+        auto kern = DOWN ? (vin ? row_downdate_narrow_kernel<true> : row_downdate_narrow_kernel<false>)
+                         : (vin ? row_condition_narrow_kernel<true> : row_condition_narrow_kernel<false>);
+        kern<<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows, col_slot, B, ldb, kk, r, q, d,
+                                     var, mo);
+        return check_cuda(cudaGetLastError(),
+                          DOWN ? "row_downdate_narrow_kernel launch" : "row_condition_narrow_kernel launch");
     }
     int qlog = 1;                             // quads: the next power of two >= ceil(k / 4), 2 .. 16
     while ((4 << qlog) < k) ++qlog;
-    if (vin)
-        row_condition_mid_kernel<true><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
-                                                               col_slot, B, ldb, kk, r, q, d, var, mo, qlog);
-    else
-        row_condition_mid_kernel<false><<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows,
-                                                                col_slot, B, ldb, kk, r, q, d, var, mo, qlog);
-    return check_cuda(cudaGetLastError(), "row_condition_mid_kernel launch");
+    auto kern = DOWN ? (vin ? row_downdate_mid_kernel<true> : row_downdate_mid_kernel<false>)
+                     : (vin ? row_condition_mid_kernel<true> : row_condition_mid_kernel<false>);
+    kern<<<grid, block, 0, st>>>(ptr, ent, f, L, x, n, phi->row_lo, phi->n_rows, col_slot, B, ldb, kk, r, q, d, var,
+                                 mo, qlog);
+    return check_cuda(cudaGetLastError(), DOWN ? "row_downdate_mid_kernel launch" : "row_condition_mid_kernel launch");
+}
+
+extern "C" int grf_phi_row_condition(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n,
+                                     const int32_t *col_slot, const float *B, int64_t ldb, int32_t r,
+                                     int32_t with_mean, double *q, const float *d, float *var, float *mean,
+                                     void *stream) {
+    return row_update<false>("grf_phi_row_condition", phi, f, x, n, col_slot, B, ldb, r, with_mean, q, d, var, mean,
+                             stream);
+}
+
+extern "C" int grf_phi_row_downdate(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n,
+                                    const int32_t *col_slot, const float *B, int64_t ldb, int32_t r,
+                                    int32_t with_mean, double *q, const float *d, float *var, float *mean,
+                                    void *stream) {
+    return row_update<true>("grf_phi_row_downdate", phi, f, x, n, col_slot, B, ldb, r, with_mean, q, d, var, mean,
+                            stream);
 }

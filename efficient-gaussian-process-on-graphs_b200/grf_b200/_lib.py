@@ -35,7 +35,7 @@ EXPORTS = (
     "grf_kmat_phi_count", "grf_kmat_phi_fill", "grf_kmat_transpose_count", "grf_kmat_transpose_fill", "grf_kmat_row_sizes",
     "grf_kmat_bin", "grf_kmat_workspace_bytes", "grf_kmat_count", "grf_kmat_fill", "grf_phi_row_quadform",
     "grf_alias_records", "grf_walk_weighted", "grf_phi_row_project", "grf_gram_light", "grf_gram_mirror",
-    "grf_phi_row_condition",
+    "grf_phi_row_condition", "grf_phi_row_downdate",
 )
 
 
@@ -188,6 +188,8 @@ def lib():
     L.grf_phi_row_project.argtypes = [POINTER(GrfPhi), vp, vp, i64, vp, vp, i64, i32, vp, i64, vp]
     L.grf_phi_row_condition.restype = i32
     L.grf_phi_row_condition.argtypes = [POINTER(GrfPhi), vp, vp, i64, vp, vp, i64, i32, i32, vp, vp, vp, vp, vp]
+    L.grf_phi_row_downdate.restype = i32
+    L.grf_phi_row_downdate.argtypes = [POINTER(GrfPhi), vp, vp, i64, vp, vp, i64, i32, i32, vp, vp, vp, vp, vp]
     L.grf_gram_light.restype = i32
     L.grf_gram_light.argtypes = [vp, i64, vp, vp, vp, vp, i64, vp, i64, vp]
     L.grf_gram_mirror.restype = i32

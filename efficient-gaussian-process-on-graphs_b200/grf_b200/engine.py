@@ -1218,6 +1218,15 @@ class PhiBlocks:
         contiguous, on Phi's device.  B: float32 [m, >= r + with_mean] (a column slice of a wider buffer is read in
         place; any other layout is copied); ValueError when col_slot names a row past m, or for 1 <= r + with_mean
         <= 64 not holding.  x = None: every local row.  See grf_b200/posterior.py, PosteriorMarginals."""
+        self._row_update("row_condition", f, x, col_slot, B, r, with_mean, q, d, var, mean)
+
+    def row_downdate(self, f, x, col_slot, B, r: int, with_mean: bool, q, d, var, mean=None) -> None:
+        """``row_condition`` with the squares subtracted: q[i] -= sum_{c < r} p[i, c]^2 (float64), then var and mean
+        as there (``grf_phi_row_downdate``; the same operands and checks).  With B = [U | a] for the U of
+        ExactPosterior.forget this brings the variance at the rows x down to the remaining training rows."""
+        self._row_update("row_downdate", f, x, col_slot, B, r, with_mean, q, d, var, mean)
+
+    def _row_update(self, what, f, x, col_slot, B, r, with_mean, q, d, var, mean) -> None:
         dev = self.device
         f = self._f(f)
         xi = self._ids(x, dev)
@@ -1225,12 +1234,12 @@ class PhiBlocks:
         r, wm = int(r), int(bool(with_mean))
         k = r + wm
         if not 1 <= k <= 64 or r < 0:
-            raise ValueError(f"row_condition: r + with_mean must be in [1, 64], got r = {r}, with_mean = {wm}")
+            raise ValueError(f"{what}: r + with_mean must be in [1, 64], got r = {r}, with_mean = {wm}")
         col_slot = torch.as_tensor(col_slot, device=dev).to(torch.int32).contiguous()
         if col_slot.numel() != self.n_cols:
-            raise ValueError(f"row_condition: col_slot has {col_slot.numel()} entries, Phi has {self.n_cols} columns")
+            raise ValueError(f"{what}: col_slot has {col_slot.numel()} entries, Phi has {self.n_cols} columns")
         if B.dim() != 2 or B.dtype != torch.float32 or B.device != dev or B.shape[1] < k:
-            raise ValueError(f"row_condition: B must be a 2-D float32 tensor on Phi's device with at least {k} "
+            raise ValueError(f"{what}: B must be a 2-D float32 tensor on Phi's device with at least {k} "
                              "columns")
         if (k > 1 and B.stride(1) != 1) or (B.shape[0] > 1 and B.stride(0) < k):
             B = B[:, :k].contiguous()      # the kernel reads rows of k floats ldb apart
@@ -1239,17 +1248,17 @@ class PhiBlocks:
                 (("mean", mean, torch.float32),) * wm:
             if (t is None or t.dtype != dt or t.device != dev or t.numel() != n or t.dim() != 1
                     or (n > 1 and t.stride(0) != 1)):
-                raise ValueError(f"row_condition: {name} must be a contiguous {dt} [{n}] tensor on Phi's device")
+                raise ValueError(f"{what}: {name} must be a contiguous {dt} [{n}] tensor on Phi's device")
         if n == 0:
             return
         if col_slot.numel() and int(col_slot.max()) >= B.shape[0]:
-            raise ValueError(f"row_condition: col_slot names row {int(col_slot.max())} of B, which has "
+            raise ValueError(f"{what}: col_slot names row {int(col_slot.max())} of B, which has "
                              f"{B.shape[0]} rows")
         keep = B if B.numel() else torch.zeros(k, dtype=torch.float32, device=dev)   # no row of B is read then
         phi = self.c_struct()
-        check(_lib.lib().grf_phi_row_condition(ctypes.byref(phi), _ptr(f), _ptr(xi), n, _ptr(col_slot), _ptr(keep),
-                                               ldb, r, wm, _ptr(q), _ptr(d), _ptr(var),
-                                               _ptr(mean) if wm else None, _stream(dev)))
+        fn = getattr(_lib.lib(), "grf_phi_" + what)
+        check(fn(ctypes.byref(phi), _ptr(f), _ptr(xi), n, _ptr(col_slot), _ptr(keep), ldb, r, wm, _ptr(q), _ptr(d),
+                 _ptr(var), _ptr(mean) if wm else None, _stream(dev)))
 
     def training_gram(self, x, mem_limit: Optional[int] = None) -> torch.Tensor:
         """E[l, i, l', j] = <M_l[x_i], M_l'[x_j]>, float64 [L, n, L, n]: the per-length Gram of the training rows, so

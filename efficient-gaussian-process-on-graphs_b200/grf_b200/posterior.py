@@ -32,10 +32,25 @@ Between refits of f and sigma^2 a BO loop only appends observations: ``condition
 Cholesky (C keeps its old columns and gains b), and ``PosteriorMarginals`` keeps the mean and variance at a fixed
 candidate set current with one pass over the candidate rows per update (``grf_phi_row_condition``: q grows by the
 squares of the projections onto the new columns of C, the mean is the projection onto the new a).
+
+``forget`` removes training rows (the positions B in the current training order, R the kept ones, j0 = min B):
+
+    Z  = L^-1 E_B (n x b; its rows before j0 are zero),  Z^T Z = (K^-1)_BB = R_B^T R_B   (b x b Cholesky)
+    U  = C Z R_B^-1 (m x b):  C C^T - U U^T = G_R K_RR^-1 G_R^T,  so at every candidate  q' = q - |S* U|^2
+    L' = [[L[:j0, :j0], 0], [L[R2, :j0], chol(T T^T)]],  T = L[R2, j0:]  (R2: the kept rows after j0)
+    C' = [C[:, :j0] | C[:, j0:] T^T L'_22^-T]              (the right factor has orthonormal columns)
+
+(removing the trailing positions truncates L and C), a is recomputed from L' in float64, and the rows of C' of
+columns that only removed rows touched are set to exactly zero: those columns keep their slots (m never shrinks; a
+later append that touches one reuses it) and give candidates the contribution of a posterior built without them,
+none.  ``set_targets`` replaces y and recomputes a; L and C stay.  ``PosteriorMarginals`` replays any mix of these
+changes from the posterior's change log: the appended columns of C through ``grf_phi_row_condition``, U through
+``grf_phi_row_downdate`` (q shrinks by the same squares), and the mean once, onto the current a.
 """
 
 from __future__ import annotations
 
+import weakref
 from typing import Dict, Optional
 
 import torch
@@ -60,6 +75,23 @@ def condition_bytes(n: int, b: int, m: int, nnz_old: int) -> int:
     return 4 * m * ldc + 8 * nb * nb + 8 * b * m + 8 * chunk * (n + 2 * b) + 16 * nnz_old * b
 
 
+def downdate_bytes(n: int, b: int, j0: int, m: int, nnz: int, logged: bool = True) -> int:
+    """Device bytes ExactPosterior.forget allocates to remove b of n rows, the first at position j0, from a
+    posterior whose C has m rows and whose training rows hold nnz entries of Phi_f: the new C (float32, ldc =
+    round_up(n - b, 4)) and L (float64); T = L[R2, j0:], T T^T, L'_22 and the right factor M (float64); one float64 row
+    chunk of C[:, j0:] and its product; the gather of the kept rows' entries (int64 row, column and index, float32
+    value); and with ``logged`` (a PosteriorMarginals is alive) E_B, Z, Z^T Z, R_B, Z R_B^-1 and [M | Z R_B^-1]
+    (float64) and U (float32 [m, b])."""
+    nn, nt = n - b, n - j0
+    n2 = nn - j0
+    ldc = (nn + 3) // 4 * 4
+    chunk = _condition_chunk(nt, m)
+    need = 4 * m * ldc + 8 * nn * nn + 16 * n2 * nt + 16 * n2 * n2 + 8 * chunk * (nt + n2 + b) + 28 * nnz
+    if logged:
+        need += 24 * nt * b + 16 * b * b + 8 * nt * (n2 + b) + 4 * m * b
+    return need
+
+
 class ExactPosterior:
     """The training-side cache (slots, L, C and, with ``y_train``, a = G K^-1 y) of the exact posterior, built once
     per (Phi, f, x, sigma^2, y).
@@ -69,8 +101,9 @@ class ExactPosterior:
     events recorded at the stage boundaries ("start", "merge", "slots", "G", "gram", "cholesky", "solve";
     ``variance`` adds "quadform_start" and "quadform"; every projection, of ``mean``, ``covariance`` and ``sample``,
     "project_start" and "project"; ``sample`` also "sample_start", "prior", "triangular" and "gemm";
-    ``condition_on`` "condition_start", "cross", "factor", "append" and "weights"; a PosteriorMarginals refresh
-    "refresh_start" and "refresh")."""
+    ``condition_on`` "condition_start", "cross", "factor", "append" and "weights"; ``forget`` "downdate_start",
+    "downdate_factor", "downdate_columns" and "downdate_weights"; a PosteriorMarginals refresh "refresh_start" and
+    "refresh")."""
 
     def __init__(self, blocks: PhiBlocks, f, x_train, noise, mem_limit: Optional[int] = None,
                  events: Optional[Dict[str, torch.cuda.Event]] = None, *, y_train=None):
@@ -139,6 +172,10 @@ class ExactPosterior:
             del ct
             self._mark("solve")
         self.version = 0
+        # (version, "append" / "remove" / "targets", float32 block) of every change a live PosteriorMarginals has
+        # not seen yet: the appended columns of C, or U of a removal (see PosteriorMarginals.refresh)
+        self._log = []
+        self._watchers = weakref.WeakSet()
 
     def _gather(self, x):
         """(row index j, column, value) of every entry of the rows x of the merged Phi_f, row by row in entry
@@ -377,16 +414,9 @@ class ExactPosterior:
             self._mark("append")
             x_all = torch.cat([self.x, xn])
             a = None
-            if yn is not None:                               # a = G K^-1 y, float64 sums over slot-sorted entries
+            if yn is not None:
                 y = torch.cat([self.y, yn])
-                alpha = torch.cholesky_solve(y[:, None], L)[:, 0]
-                ja, ca, va = self._gather(x_all)
-                sa = slot[ca].to(torch.int64)
-                order = torch.argsort(sa * nb + ja)
-                contrib = (va.to(torch.float64) * alpha[ja])[order]
-                a = torch.segment_reduce(contrib, "sum", lengths=torch.bincount(sa, minlength=m1), axis=0)
-                a = a.to(torch.float32)[:, None]
-                del alpha, ja, ca, va, sa, order, contrib
+                a = self._weights(x_all, y, L, slot, m1)
             # nothing above changed the posterior (a failed factor leaves it as it was); now it takes the new state
             self.slot, self.m, self.C, self.L, self.ldc = slot, m1, C, L, ldc
             self.x, self.n = x_all, nb
@@ -394,26 +424,207 @@ class ExactPosterior:
             if yn is not None:
                 self.y, self.a = y, a
             self.version += 1
+            self._record("append", C[:, n:nb])
             self._mark("weights")
         return self
 
+    def _weights(self, x, y, L, slot, m: int) -> torch.Tensor:
+        """a = G K^-1 y (float32 [m, 1]) from the factor L of K over the training ids x: float64 sums over the
+        slot-sorted entries (slots no training row touches get exactly 0)."""
+        n = int(x.numel())
+        if n == 0:
+            return torch.zeros((m, 1), dtype=torch.float32, device=self.device)
+        alpha = torch.cholesky_solve(y[:, None], L)[:, 0]
+        ja, ca, va = self._gather(x)
+        sa = slot[ca].to(torch.int64)
+        order = torch.argsort(sa * n + ja)
+        contrib = (va.to(torch.float64) * alpha[ja])[order]
+        a = torch.segment_reduce(contrib, "sum", lengths=torch.bincount(sa, minlength=m), axis=0)
+        return a.to(torch.float32)[:, None]
+
+    def _record(self, kind: str, block: Optional[torch.Tensor]) -> None:
+        """Log a change (made as ``version``) for the live PosteriorMarginals; nothing is kept when there is none."""
+        self._trim()
+        if len(self._watchers):
+            self._log.append((self.version, kind, None if block is None else block.clone()))
+
+    def _trim(self) -> None:
+        """Drop the log entries every live PosteriorMarginals has already seen."""
+        seen = [w.version for w in self._watchers]
+        oldest = min(seen) if seen else self.version
+        self._log = [e for e in self._log if e[0] > oldest]
+
+    def _positions(self, positions, what: str) -> torch.Tensor:
+        """Positions into the current training order as an int64 host tensor (in the given order); IndexError
+        outside [0, n), ValueError for a repeated position."""
+        pos = torch.as_tensor(positions).detach().flatten()
+        if pos.numel() and (pos.dtype.is_floating_point or pos.dtype.is_complex or pos.dtype == torch.bool):
+            raise ValueError(f"ExactPosterior.{what}: positions must be integers, got {pos.dtype}")
+        pos = pos.cpu().to(torch.int64)
+        if pos.numel() and (int(pos.min()) < 0 or int(pos.max()) >= self.n):
+            bad = pos[(pos < 0) | (pos >= self.n)][0]
+            raise IndexError(f"ExactPosterior.{what}: position {int(bad)} is outside the {self.n} training rows")
+        if torch.unique(pos).numel() != pos.numel():
+            raise ValueError(f"ExactPosterior.{what}: positions repeat")
+        return pos
+
+    def forget(self, positions) -> "ExactPosterior":
+        """Remove the training rows at ``positions`` (indices into the current training order; ids may repeat in x,
+        so rows are named by position) in place: afterwards every method answers as a posterior constructed on the
+        kept rows, in their order, does, within float32 round-off.  Returns self.
+
+        With B the removed positions, R2 the kept positions after j0 = min B and T = L[R2, j0:]:
+            L' = [[L[:j0, :j0], 0], [L[R2, :j0], chol(T T^T)]],   C' = [C[:, :j0] | C[:, j0:] T^T L'_22^-T]
+        (the product in float64 row chunks, stored as float32; ldc = round_up(n - b, 4)), and, with y, a = G K^-1 y
+        from L' (float64).  Rows of C' whose column no kept row touches are set to exactly zero; the slots stay.
+        While a PosteriorMarginals is alive, the same chunks also form U = C Z R_B^-1 for its refresh (module
+        docstring).  C and L are reallocated at their new size.
+
+        An empty call is a no-op; removing every row leaves the prior (n = 0); each call that removes rows
+        increments ``version``.  IndexError for a position outside [0, n); ValueError for a repeated position, or
+        when chol(T T^T) fails in float64 (the posterior is then left as it was); MemoryError (naming the bytes)
+        before anything is allocated.  Events: "downdate_start", "downdate_factor", "downdate_columns" and
+        "downdate_weights"."""
+        pos = torch.sort(self._positions(positions, "forget")).values
+        b = int(pos.numel())
+        if b == 0:
+            return self
+        dev, n, m = self.device, self.n, self.m
+        j0 = int(pos[0])
+        keep = torch.ones(n, dtype=torch.bool)
+        keep[pos] = False
+        kept = torch.nonzero(keep).flatten()
+        nn, nt = n - b, n - j0
+        n2 = nn - j0
+        logged = len(self._watchers) > 0
+        need = downdate_bytes(n, b, j0, m, self.nnz_train, logged)
+        budget = _free_bytes(dev) if self.mem_limit is None else int(self.mem_limit)
+        if need > budget:
+            raise MemoryError(f"exact posterior forget: C and L of {nn} training rows touching {m} columns need "
+                              f"{need} bytes, {budget} bytes of device memory are free")
+        with torch.cuda.device(dev):
+            self._mark("downdate_start")
+            r2 = (kept[j0:] - j0).to(dev)                      # the kept rows after j0, in the trailing block
+            L22 = self.L[j0:, j0:]
+            T = L22[r2]                                        # [n2, nt]
+            l22 = torch.zeros((0, 0), dtype=torch.float64, device=dev)
+            if n2:
+                l22, info = torch.linalg.cholesky_ex(T @ T.T)
+                if int(info.item()) > 0:
+                    raise ValueError(f"exact posterior forget: the trailing factor T T^T of the {n2} kept rows after "
+                                     f"position {j0} is not positive definite in float64 (leading minor "
+                                     f"{int(info.item())})")
+            L = torch.zeros((nn, nn), dtype=torch.float64, device=dev)
+            L[:j0, :j0] = self.L[:j0, :j0]
+            L[j0:, :j0] = self.L[j0:, :j0][r2]
+            L[j0:, j0:] = l22
+            self._mark("downdate_factor")
+            rhs = torch.linalg.solve_triangular(l22, T, upper=False).T if n2 else T.T    # M = T^T L'_22^-T
+            del T
+            if logged:                                         # Z R_B^-1, Z = L^-1 E_B (rows >= j0)
+                eb = torch.zeros((nt, b), dtype=torch.float64, device=dev)
+                eb[(pos - j0).to(dev), torch.arange(b, device=dev)] = 1.0
+                z = torch.linalg.solve_triangular(L22, eb, upper=False)
+                del eb
+                rb, info = torch.linalg.cholesky_ex(z.T @ z)
+                if int(info.item()) > 0:
+                    raise ValueError(f"exact posterior forget: (K^-1)_BB of the {b} removed rows is not positive "
+                                     f"definite in float64 (leading minor {int(info.item())})")
+                w = torch.linalg.solve_triangular(rb.T, z, upper=True, left=False)
+                rhs = torch.cat([rhs, w], 1)
+                del z, rb, w
+            ldc = (nn + 3) // 4 * 4
+            C = torch.zeros((m, ldc), dtype=torch.float32, device=dev)
+            C[:, :j0] = self.C[:, :j0]
+            U = torch.empty((m, b), dtype=torch.float32, device=dev) if logged else None
+            chunk = _condition_chunk(nt, m)
+            for r0 in range(0, m, chunk):                     # C[:, j0:] [M | Z R_B^-1], by rows
+                r1 = min(m, r0 + chunk)
+                prod = self.C[r0:r1, j0:n].to(torch.float64) @ rhs
+                C[r0:r1, j0:nn] = prod[:, :n2].to(torch.float32)
+                if logged:
+                    U[r0:r1] = prod[:, n2:].to(torch.float32)
+                del prod
+            del rhs
+            x_kept = self.x[kept.to(dev)]
+            jk, ck, _ = self._gather(x_kept)
+            live = torch.zeros(m, dtype=torch.bool, device=dev)
+            live[self.slot[ck].to(torch.int64)] = True
+            C[~live] = 0.0                                     # columns only the removed rows touched
+            nnz = int(jk.numel())
+            del jk, ck, live
+            self._mark("downdate_columns")
+            y, a = None, None
+            if self.y is not None:
+                y = self.y[kept.to(dev)]
+                a = self._weights(x_kept, y, L, self.slot, m)
+            # nothing above changed the posterior; now it takes the new state
+            self.C, self.L, self.ldc = C, L, ldc
+            self.nnz_train = nnz
+            self.x, self.n = x_kept, nn
+            if y is not None:
+                self.y, self.a = y, a
+            self.version += 1
+            self._record("remove", U)
+            self._mark("downdate_weights")
+        return self
+
+    def set_targets(self, y, positions=None) -> "ExactPosterior":
+        """Replace the training targets: all of them (``positions`` None; y has n values), or those at
+        ``positions`` (indices into the current training order; y has one value per position).  a = G K^-1 y is
+        recomputed from L in float64; L and C stay.  Each call that changes targets increments ``version``; an empty
+        ``positions`` is a no-op.  With ``condition_on(x, mean(x))`` for a batch of hallucinated observations, this
+        swaps in the real targets once they arrive.  Returns self.  ValueError on a posterior built without y, for
+        a y of the wrong length or with non-finite values, or for a repeated position; IndexError for a position
+        outside [0, n)."""
+        self._need_y("set_targets")
+        dev = self.device
+        yv = torch.as_tensor(y, device=dev).detach().flatten().to(torch.float64)
+        if positions is None:
+            if yv.numel() != self.n:
+                raise ValueError(f"ExactPosterior.set_targets: y has {yv.numel()} values for {self.n} training rows")
+            pos = None
+        else:
+            pos = self._positions(positions, "set_targets")
+            if yv.numel() != pos.numel():
+                raise ValueError(f"ExactPosterior.set_targets: y has {yv.numel()} values for {pos.numel()} "
+                                 "positions")
+        if not bool(torch.isfinite(yv).all()):
+            raise ValueError("ExactPosterior.set_targets: y must be finite")
+        if pos is not None and pos.numel() == 0:
+            return self
+        with torch.cuda.device(dev):
+            if pos is None:
+                y_all = yv.clone()
+            else:
+                y_all = self.y.clone()
+                y_all[pos.to(dev)] = yv
+            self.a = self._weights(self.x, y_all, self.L, self.slot, self.m)
+            self.y = y_all
+            self.version += 1
+            self._record("targets", None)
+        return self
+
     def marginals(self, x_cand) -> "PosteriorMarginals":
-        """The mean and variance at a fixed candidate set, kept current across ``condition_on`` calls at the cost
-        of one pass over the candidate rows per refresh (see PosteriorMarginals).  IndexError for ids outside Phi."""
+        """The mean and variance at a fixed candidate set, kept current across ``condition_on``, ``forget`` and
+        ``set_targets`` calls at the cost of one pass over the candidate rows per kind of change (see
+        PosteriorMarginals).  IndexError for ids outside Phi."""
         return PosteriorMarginals(self, x_cand)
 
 
 class PosteriorMarginals:
-    """Mean and variance of an ExactPosterior at fixed candidate ids, brought up to date after the posterior is
-    conditioned on new rows without redoing the pass over all n columns of C.
+    """Mean and variance of an ExactPosterior at fixed candidate ids, brought up to date after the posterior gained
+    or lost training rows, or changed targets, without redoing the pass over all n columns of C.
 
-    It keeps d (float32) and q (float64) of var = max(d - q, 0).  After ``condition_on`` appended k = n - n_seen
-    columns to C, ``refresh`` adds the squares of the candidates' projections onto those columns to q and recomputes
-    the mean from the new a:
-      k + with_mean <= 64   one ``row_condition`` pass with B = [C[:, n_seen:n] | a] (a copied into the last
-                            column of an m x (k + 1) buffer)
-      k + with_mean > 64    ``row_quadform`` on C[:, n_seen:n] (q rounded to float32 once) plus one ``row_project``
-                            onto a
+    It keeps d (float32) and q (float64) of var = max(d - q, 0).  ``refresh`` replays the posterior's change log
+    since the last refresh, consecutive changes of one kind together: appends add the squares of the candidates'
+    projections onto the appended columns of C to q, removals subtract those onto U (module docstring), and the mean
+    is recomputed once from the current a.  For k columns of one kind, with_mean = 1 on the last of them:
+      k + with_mean <= 64   one ``row_condition`` (appends) or ``row_downdate`` (removals) pass with B = [blocks | a]
+                            (the blocks, and a in the last column, copied into an m x (k + with_mean) buffer)
+      k + with_mean > 64    ``row_quadform`` on the blocks (q rounded to float32 once) plus one ``row_project`` onto a
+    A history of appends alone is one block of the columns C gained, so it refreshes exactly as the posterior's
+    columns would.  The posterior keeps the blocks only while a PosteriorMarginals that has not seen them is alive.
     ``mean`` and ``variance`` refresh when the posterior has changed since the last refresh."""
 
     def __init__(self, post: ExactPosterior, x_cand):
@@ -426,6 +637,7 @@ class PosteriorMarginals:
             self._var = torch.clamp_min(self.d - q, 0.0)      # = post.variance(x_cand)
             self._mean = post._project(self.x, post.a)[:, 0].contiguous() if post.y is not None else None
         self.version, self.n_seen = post.version, post.n
+        post._watchers.add(self)
 
     @property
     def stale(self) -> bool:
@@ -436,26 +648,48 @@ class PosteriorMarginals:
         post = self.post
         if not self.stale:
             return self
-        dev, n0, n = post.device, self.n_seen, post.n
-        k, wm = n - n0, post.y is not None
+        dev, wm, m = post.device, post.y is not None, post.m
+        runs = []                                     # [kind, [blocks]]: consecutive changes of one kind
+        for v, kind, block in post._log:
+            if v <= self.version or kind == "targets":
+                continue
+            if runs and runs[-1][0] == kind:
+                runs[-1][1].append(block)
+            else:
+                runs.append([kind, [block]])
+        if not runs:                                  # only the targets changed
+            runs.append(["append", []])
         one = torch.ones(1, device=dev)
         with torch.cuda.device(dev):
             post._mark("refresh_start")
-            if k + wm <= 64:
-                B = torch.empty((post.m, k + wm), dtype=torch.float32, device=dev)
-                B[:, :k] = post.C[:, n0:n]
-                if wm:
-                    B[:, k] = post.a[:, 0]
-                post.phi_f.row_condition(one, self.x, post.slot, B, k, wm, self.q, self.d, self._var,
-                                         self._mean if wm else None)
-            else:
-                dq, _ = post.phi_f.row_quadform(one, self.x, post.slot, post.C[:, n0:n])
-                self.q += dq.to(torch.float64)
-                self._var = torch.clamp_min((self.d.to(torch.float64) - self.q).to(torch.float32), 0.0)
-                if wm:
-                    self._mean = post.phi_f.row_project(one, self.x, post.slot, post.a)[:, 0].contiguous()
+            for i, (kind, blocks) in enumerate(runs):
+                mean_here = int(wm and i == len(runs) - 1)
+                k = sum(int(blk.shape[1]) for blk in blocks)
+                B = torch.empty((m, k + mean_here), dtype=torch.float32, device=dev)
+                c = 0
+                for blk in blocks:                    # blocks logged before C gained slots: zero in the new rows
+                    B[:blk.shape[0], c:c + blk.shape[1]] = blk
+                    B[blk.shape[0]:, c:c + blk.shape[1]] = 0.0
+                    c += blk.shape[1]
+                if k + mean_here <= 64:
+                    if mean_here:
+                        B[:, k] = post.a[:, 0]
+                    update = post.phi_f.row_condition if kind == "append" else post.phi_f.row_downdate
+                    update(one, self.x, post.slot, B, k, mean_here, self.q, self.d, self._var,
+                           self._mean if mean_here else None)
+                else:
+                    dq, _ = post.phi_f.row_quadform(one, self.x, post.slot, B[:, :k])
+                    if kind == "append":
+                        self.q += dq.to(torch.float64)
+                    else:
+                        self.q -= dq.to(torch.float64)
+                    self._var = torch.clamp_min((self.d.to(torch.float64) - self.q).to(torch.float32), 0.0)
+                    if mean_here:
+                        self._mean = post.phi_f.row_project(one, self.x, post.slot, post.a)[:, 0].contiguous()
+                del B
             post._mark("refresh")
-        self.version, self.n_seen = post.version, n
+        self.version, self.n_seen = post.version, post.n
+        post._trim()
         return self
 
     @property

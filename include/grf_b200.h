@@ -539,6 +539,19 @@ int grf_phi_row_condition(const GrfPhi *phi, const float *f, const int32_t *x, i
                           const float *B, int64_t ldb, int32_t r, int32_t with_mean, double *q, const float *d,
                           float *var, float *mean, void *stream);
 
+/* Rank-k downdate of the posterior variance (and the mean) at fixed test rows after training rows were removed
+ * (csrc/grf_posterior.cu; grf_b200/posterior.py, ExactPosterior.forget and PosteriorMarginals).  The arguments and
+ * rules of grf_phi_row_condition, with the squares subtracted:
+ *   q[i]   -= sum_{c < r} p_c(i)^2        (the squares in float64, subtracted from q[i] in the order c = 0, 1, ..)
+ *   var[i]  = (float)(d[i] - q[i]) with the updated q, clamped at +0 (NaN stays NaN)
+ *   mean[i] = p_r(i)                      (only with with_mean = 1)
+ * B = [U | a]: U = C Z R^-1 with Z = L^-1 E_B and Z^T Z = R^T R for the removed positions B, so that C C^T - U U^T is
+ * the C C^T of the remaining rows, and the new a.  p is summed in exactly the order of grf_phi_row_condition.  k <= 4
+ * runs row_downdate_narrow_kernel, k <= 64 row_downdate_mid_kernel.  -1 in the cases of grf_phi_row_condition. */
+int grf_phi_row_downdate(const GrfPhi *phi, const float *f, const int32_t *x, int64_t n, const int32_t *col_slot,
+                         const float *B, int64_t ldb, int32_t r, int32_t with_mean, double *q, const float *d,
+                         float *var, float *mean, void *stream);
+
 /* Per-length Gram of the training rows, light part (csrc/grf_gram.cu; no reference counterpart: the reference
  * estimates the marginal likelihood by CG and probes).  With A[R, c] = M_l[x_i, c] for the E row R = l * n + i,
  * E = A A^T is float64 [n_rows][lde], n_rows = L * n.  The columns the training rows touch are numbered as slots
